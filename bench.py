@@ -20,6 +20,8 @@ timed per rank, with the imbalance of the partition; `cross_shard_read` gathers 
 all ranks through the library's own NCCL exchange (ii2_read_gather) and checks it.
 `--impl reference` times the CPU oracle with all host threads (InvertedIndex.Merge's worker
 pool over shards, inverted_index.go:83-103) on bounded samples of the SAME workload.
+`--dump-outputs DIR` writes the merged segment of the last timed step (rank 0) as .npy files;
+the inputs depend only on the arguments, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -33,6 +35,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the (possibly read-only) tree
 
 import numpy as np  # noqa: E402
 
@@ -65,7 +68,16 @@ def parse():
                     help="postings one rank holds at most in the strong leg (host RAM / time)")
     ap.add_argument("--verify", action="store_true",
                     help="check the full-size result against an independent numpy union")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the merged segment of the last timed step to DIR/<name>.npy "
+                         f"(float32 / float64; an array of more than {DUMP_CAP} values as a "
+                         "seeded sample of them)")
+    a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs dumps the GPU merge (--impl ours)")
+    return a
 
 
 def workload_name(a):
@@ -455,6 +467,33 @@ def pin(arr: np.ndarray):
     return t.numpy(), t
 
 
+# values kept per dumped array: the default workload's merged segment is ~300 MB; sampled, its
+# dump (values + sample positions) is ~30 MB and stays below 64 MB for any workload
+DUMP_CAP = 1 << 19
+
+
+def dump_outputs(out_dir: str, m) -> None:
+    """Writes the merged segment `m` (what ii2_result_download_merge hands a caller) as .npy
+    files that two builds can compare value for value.  Integer arrays are stored exactly as
+    float64 (bytes as float32); an array longer than DUMP_CAP is replaced by the values at
+    DUMP_CAP positions drawn with a fixed seed from its length, and `<name>_idx.npy` holds those
+    positions, so equal lengths give equal positions."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"term_bytes": m.term_bytes, "term_off": m.term_off, "val_off": m.val_off,
+              "val_bytes": m.val_bytes,
+              "min_term": np.frombuffer(m.min_term or b"", dtype=np.uint8),
+              "max_term": np.frombuffer(m.max_term or b"", dtype=np.uint8),
+              "counts": np.array([m.terms_count, m.terms_merged, m.postings_in, m.postings_out,
+                                  m.val_size], dtype=np.uint64)}
+    for seed, (name, arr) in enumerate(arrays.items()):
+        if len(arr) > DUMP_CAP:
+            idx = np.sort(np.random.default_rng(seed).choice(len(arr), DUMP_CAP, replace=False))
+            np.save(os.path.join(out_dir, f"{name}_idx.npy"), idx.astype(np.float64))
+            arr = arr[idx]
+        np.save(os.path.join(out_dir, f"{name}.npy"),
+                arr.astype(np.float32 if arr.dtype == np.uint8 else np.float64))
+
+
 def run_ours(a):
     import torch
     import torch.distributed as dist
@@ -477,17 +516,19 @@ def run_ours(a):
     drem = eng.upload_removed(w.removed)
     eng.sync()
 
-    def step():
+    def step(keep=False):
+        """One compaction; the result stays on the device (returned) only when `keep`."""
         res = eng.merge_dev(dsegs, drem, encode=True)
         info = res.info()
         out = (int(info.postings_in), int(info.postings_out), int(info.terms_count),
                int(info.term_bytes), int(info.val_size))
+        if keep:
+            return out, res
         res.release()
-        return out
+        return out, None
 
     for _ in range(a.warmup):
-        stats = step()
-    n_in, n_out, t_out, t_out_bytes, val_size = stats
+        step()
 
     def barrier():
         if world > 1:
@@ -501,8 +542,8 @@ def run_ours(a):
     l0 = eng.kernel_launches()
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record(stream)
-    for _ in range(a.steps):
-        step()
+    for i in range(a.steps):
+        stats, last = step(keep=bool(a.dump_outputs) and i == a.steps - 1)
     ev1.record(stream)
     barrier()
     launches = eng.kernel_launches() - l0
@@ -510,6 +551,11 @@ def run_ours(a):
     prof = eng.prof_read()
     eng.prof_enable(False)
     ms = ev0.elapsed_time(ev1)
+    n_in, n_out, t_out, t_out_bytes, val_size = stats
+    if last is not None:
+        if rank == 0:
+            dump_outputs(a.dump_outputs, last.download_merge(decoded=False))
+        last.release()
     if world > 1:
         t = torch.tensor([ms], device="cuda", dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
