@@ -4,6 +4,9 @@
   C3  term-range read union across 256 segments with 5 % removed_list filtering (µs per call)
   C4  file/bitmask + intcomp encode/decode sweep, posting-list lengths 16 .. 16M
   prefix  PrefixSearch batches over 64 resident segments (µs per call)
+  multidev  one process over every visible GPU (Engine(devices=...)): weak-scaling compaction from
+        one host thread per device, a 1 % read partitioned over the devices + ii2_read_gather_devices,
+        and ii2_prefix_gather_devices of the prefix batch; each checked against one device
 bench.py stays the headline (C2 compaction); these lines are evidence for SURVEY §8 rows."""
 from __future__ import annotations
 
@@ -250,6 +253,157 @@ def c4(eng, a):
     print(json.dumps({"config": "C4 codec sweep, list lengths 16..16M", "results": rows}))
 
 
+def _card():
+    """Card name and power limit, read in the same run as the numbers (read-only query)."""
+    import subprocess
+    try:
+        q = subprocess.run(["nvidia-smi", "--query-gpu=index,name,power.limit", "--format=csv,noheader"],
+                           capture_output=True, text=True, timeout=60).stdout.strip().splitlines()
+    except Exception as e:  # noqa: BLE001
+        q = [f"nvidia-smi unavailable: {e}"]
+    return q
+
+
+_POOL = None  # one long-lived host thread per device (no thread start inside a timed call)
+
+
+def _in_threads(fns):
+    """Runs fns[i] on worker thread i of the pool, all at once; their results in order."""
+    global _POOL
+    import queue
+    import threading
+    if _POOL is None or len(_POOL) < len(fns):
+        _POOL = []
+        for _ in range(max(len(fns), 16)):
+            q_in, q_out = queue.Queue(), queue.Queue()
+
+            def loop(q_in=q_in, q_out=q_out):
+                while True:
+                    f = q_in.get()
+                    try:
+                        q_out.put((True, f()))
+                    except BaseException as e:  # noqa: BLE001
+                        q_out.put((False, repr(e)))
+            threading.Thread(target=loop, daemon=True).start()
+            _POOL.append((q_in, q_out))
+    for (q_in, _), f in zip(_POOL, fns):
+        q_in.put(f)
+    got = [q_out.get() for (_, q_out), _f in zip(_POOL, fns)]
+    errs = [v for ok, v in got if not ok]
+    if errs:
+        raise RuntimeError("; ".join(errs))
+    return [v for _, v in got]
+
+
+def _partition(w, k):
+    from inverted_index_2_b200 import sharded
+    from inverted_index_2_b200.flat import FlatSegment
+    keys = sharded.shard_keys_of_sorted(w.term_bytes, w.term_off)
+    bounds = sharded.partition_shard_keys(np.bincount(keys, minlength=1024).astype(float), k)
+    parts = []
+    for r in range(k):
+        lo, hi = np.searchsorted(keys, [bounds[r], bounds[r + 1]])
+        out = []
+        for seg, ids in zip(w.segments, w.seg_term_ids):
+            a, b = np.searchsorted(ids, [lo, hi])
+            toff, poff = seg.term_off[a:b + 1], seg.post_off[a:b + 1]
+            out.append(FlatSegment(seg.term_bytes[int(toff[0]):int(toff[-1])].copy(),
+                                   (toff - toff[0]).astype(np.uint32), seg.mode,
+                                   post=seg.post[int(poff[0]):int(poff[-1])].copy(),
+                                   post_off=(poff - poff[0]).astype(np.uint64)))
+        parts.append(out)
+    return parts
+
+
+def multidev(a):
+    import torch
+    from inverted_index_2_b200.engine import Engine
+    n = torch.cuda.device_count()
+    devs = list(range(min(n, 16)))
+    eng = Engine(devices=devs)
+    N = len(devs)
+    card = _card()
+    # ---- weak scaling: every device compacts its own copy of the C2 workload (bench.py's shape)
+    w = synth.make_workload(a.terms, 64, a.postings, seed=0xC2, removed_frac=0.05)
+    res = {}
+
+    def setup(d):
+        eng.set_device(d)
+        return [eng.upload(s) for s in w.segments], eng.upload_removed(w.removed)
+    held = _in_threads([lambda d=d: setup(d) for d in devs])
+
+    def compact(i):
+        segs, rem = held[i]
+        r = eng.merge_dev(segs, rem, encode=True, decoded=False)
+        r.release()
+
+    def rate(idx, reps=5):
+        _in_threads([lambda i=i: compact(i) for i in idx])  # warm-up
+        t0 = time.perf_counter()
+        for _ in range(reps):
+            _in_threads([lambda i=i: compact(i) for i in idx])
+        return len(idx) * reps * w.postings_in / (time.perf_counter() - t0) / 1e9
+    single = rate([0])
+    agg = rate(list(range(N)))
+    # (an efficiency is a scaling figure: it means nothing with one device)
+    res["weak_scaling"] = {"devices": N, "single_device_gpostings_s": single, "aggregate_gpostings_s": agg,
+                           "efficiency": agg / (N * single) if N > 1 else None}
+    for segs, rem in held:
+        [s.release() for s in segs]
+        rem.release()
+    # ---- 1 % read of one index partitioned over the devices, gathered to device 0
+    parts = _partition(w, N)
+    eng.set_device(devs[0])
+    whole = [eng.upload(s) for s in w.segments]
+    dparts = _in_threads([lambda r=r: (eng.set_device(devs[r]), [eng.upload(s) for s in parts[r]])[1]
+                          for r in range(N)])
+    eng.set_device(devs[0])
+    nt = len(w.term_off) - 1
+    rng = np.random.default_rng(5)
+    lat, checked = [], 0
+    for _ in range(8):
+        span = max(1, nt // 100)
+        lo = int(rng.integers(0, nt - span + 1))
+        tlo = synth.term_at(w.term_bytes, w.term_off, lo)
+        thi = synth.term_at(w.term_bytes, w.term_off, lo + span - 1)
+        ts = []
+        for rep in range(4):
+            torch.cuda.synchronize()
+            t0 = time.perf_counter()
+            reads = _in_threads([lambda r=r: eng.read_range_dev(dparts[r], tlo, thi) for r in range(N)])
+            g = eng.read_gather_devices(reads, devs[0])
+            ts.append(time.perf_counter() - t0)
+            if rep == 3:
+                got = g.download_read()
+                ref = eng.read_range_dev(whole, tlo, thi).download_read()
+                for f in ("term_bytes", "term_off", "post", "post_off"):
+                    assert np.array_equal(getattr(got, f), getattr(ref, f)), f
+                checked += 1
+            [x.release() for x in reads]
+            g.release()
+        lat.append(float(np.median(ts[1:])))
+    res["read_1pct_gather_us"] = {"median_us": 1e6 * float(np.median(lat)), "max_us": 1e6 * float(np.max(lat)),
+                                  "positions_verified": checked,
+                                  "what": "per-device ii2_read_range_dev from one long-lived host thread per "
+                                          "device + ii2_read_gather_devices to device 0, wall clock"}
+    # ---- prefix search over the devices, gathered on device 0
+    prow = []
+    for plen, count in ((3, 16), (2, 16), (1, 16), (0, 1)):
+        picks = sorted({synth.term_at(w.term_bytes, w.term_off, int(i))[:plen]
+                        for i in rng.integers(0, nt, size=count)})
+        ref = eng.prefix_search_dev(whole, picks)
+
+        def call():
+            return eng.prefix_gather_devices(dparts, picks, devs[0])
+        got = call()
+        assert sorted(got) == sorted(ref) and all(np.array_equal(got[k], ref[k]) for k in ref)
+        med, worst = timed(call, 3)
+        prow.append({"prefix_len": plen, "prefixes": len(picks), "median_us": 1e6 * med, "max_us": 1e6 * worst})
+    res["prefix_gather"] = prow
+    print(json.dumps({"config": f"multidev: one process over {N} device(s)", "cards": card,
+                      "terms": a.terms, "postings": w.postings_in, "results": res}))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--which", default="c3,c4")
@@ -257,6 +411,9 @@ def main():
     ap.add_argument("--terms", type=int, default=1_000_000)
     ap.add_argument("--postings", type=int, default=100_000_000)
     a = ap.parse_args()
+    if "multidev" in a.which:  # binds every visible device: a process of its own
+        multidev(a)
+        return
     from inverted_index_2_b200.engine import Engine
     eng = Engine(0)
     if "c1" in a.which:

@@ -15,7 +15,8 @@
  *     (pinned host memory) and released with the matching *_free().
  *   - re-entrant: any number of host threads may call concurrently (the
  *     reference calls this path from many goroutines: inverted_index.go:83-103,
- *     :239-285).  Each call borrows a stream + scratch arena from a pool.
+ *     :239-285).  Each call uses its host thread's stream + scratch arena on
+ *     the call's device (see ii2_init for processes that drive several GPUs).
  *     ii2_bitmask objects are NOT thread-safe, like file/bitmask.go:10.
  *   - there is no CPU fallback: without a usable CUDA device every compute
  *     entry point returns II2_ERR_NO_DEVICE.
@@ -83,18 +84,40 @@ typedef struct ii2_seg_view {
 } ii2_seg_view;
 
 /* ---- lifecycle ---------------------------------------------------------- */
-/* Bind the calling process to CUDA device devices[0] (one process per GPU;
- * ndev > 1 is reserved and rejected).  devices == NULL picks device 0.
- * Called from NewInvertedIndex (inverted_index.go:342).  Idempotent. */
+/* Bind the calling process to the CUDA devices devices[0 .. ndev), 1 <= ndev <= 16
+ * distinct ordinals, every one an sm_100 device.  devices == NULL (or ndev == 0)
+ * picks device 0.  Peer access is enabled in this process for every ordered pair of
+ * the set the hardware allows.  Called from NewInvertedIndex (inverted_index.go:342).
+ * Idempotent for the same set (in any order); any other set, a duplicate or an
+ * out-of-range ordinal is II2_ERR_INVALID.
+ *
+ * Devices of a bound set
+ *   - host-buffer calls (ii2_merge, ii2_read_range, ii2_ingest, ii2_prefix_search,
+ *     the codecs, ii2_bitmask_new) and uploads (ii2_seg_upload, ii2_removed_upload)
+ *     run on the device the calling host thread selected with ii2_set_device
+ *     (devices[0] until it does);
+ *   - every handle (ii2_seg, ii2_removed, ii2_result, ii2_bitmask) lives on the
+ *     device that created it, and calls that take handles (the _dev calls, downloads,
+ *     ii2_result_to_seg, releases, bitmask operations) run there, whatever the thread
+ *     selected.  Handles of different devices in one call are II2_ERR_INVALID.
+ *     Segments never move between devices;
+ *   - streams, scratch memory and ii2_set_stream bindings belong to a (host thread,
+ *     device) pair; pinned host outputs are process-wide and usable from every device.
+ *   - a call leaves its device current on the calling thread. */
 int ii2_init(const int* devices, int ndev);
 int ii2_shutdown(void);
 int ii2_abi_version(void);
 const char* ii2_strerror(int code);
 /* Thread-local detail string of the last failing call on this thread. */
 const char* ii2_last_error(void);
+/* Select the device of this host thread's host-buffer calls and uploads: a CUDA
+ * ordinal of the bound set, else II2_ERR_INVALID.  Go moves goroutines between OS
+ * threads: wrap the selection and the calls it governs in runtime.LockOSThread. */
+int ii2_set_device(int device);
 /* Launch on a caller-owned CUDA stream (cudaStream_t as void*) instead of a
- * pooled one, for this host thread; NULL restores the pool.  Lets a host
- * framework time the kernels with its own events. */
+ * pooled one, for this host thread and the device it selected (the stream must
+ * belong to that device); NULL restores the pool.  Lets a host framework time the
+ * kernels with its own events. */
 int ii2_set_stream(void* cuda_stream);
 /* Number of kernels this library launched since ii2_init (all threads). */
 uint64_t ii2_kernel_launches(void);
@@ -236,8 +259,10 @@ int ii2_result_download_read(const ii2_result* res, ii2_read_out* out);
 /* Adopt a decoded result as a resident segment (for multi-pass compaction). */
 int ii2_result_to_seg(ii2_result* res, ii2_seg** seg);
 void ii2_result_release(ii2_result* res);
-/* Block until everything queued by this thread's stream is done. */
+/* Block until everything queued by this thread's streams is done. */
 int ii2_sync(void);
+/* The CUDA device a result lives on (routes follow-up calls; where a gather put it). */
+int ii2_result_device(const ii2_result* res, int* device);
 
 /* ---- PrefixSearch: replaces the per-shard scan of InvertedIndex.PrefixSearch
  *      (inverted_index.go:239-292) ------------------------------------------ */
@@ -291,6 +316,32 @@ int ii2_read_gather(const ii2_result* local, int root, ii2_result** gathered);
  * every rank's values, matched = OR of the ranks' flags (the final sort + compact
  * runs on the root GPU).  Free with ii2_prefix_out_free. */
 int ii2_prefix_gather(const ii2_prefix_out* local, int root, ii2_prefix_out* merged);
+/* (ii2_comm_init is II2_ERR_INVALID in a process that bound more than one device:
+ * NCCL is for one process per GPU; the calls below serve one process over many.) */
+
+/* ---- in-process cross-device gathers: one process, several bound devices ------
+ * The caller fans out (one host thread / goroutine per device, as the reference
+ * fans out over shards), then gathers on a root device of the set. */
+/* parts[0 .. nparts) are decoded read results (ii2_read_range_dev; an encoded-only
+ * merge result is II2_ERR_INVALID) in shard-key order, on any bound devices.
+ * `gathered` lives on root_device: the concatenation in part order, offsets
+ * rebased — what InvertedIndex.Read's sequential concatenation yields
+ * (inverted_index.go:330-338) and what ii2_read_gather gives its root.  ONE kernel
+ * on the root reads every part straight from its device's HBM (peer access) and
+ * writes it to its final place.  The call waits for the streams that produced the
+ * parts (they must still exist) and returns when the result is complete.  Limits:
+ * < 4 GiB of term bytes, < 2^32-1 terms, at most 64 parts (II2_ERR_UNSUPPORTED);
+ * a part on a device the root cannot read by peer access is II2_ERR_UNSUPPORTED.
+ * nparts == 0 gives an empty result on the root. */
+int ii2_read_gather_devices(const ii2_result* const* parts, int nparts, int root_device,
+                            ii2_result** gathered);
+/* parts are ii2_prefix_search(_dev) outputs for the SAME prefix list (one per
+ * device or shard group; II2_ERR_INVALID if n_prefixes differ).  `merged`: per
+ * prefix the sorted-unique union of the parts' values, matched = OR of the parts'
+ * flags (inverted_index.go:274-292); the union runs on root_device.  Free with
+ * ii2_prefix_out_free. */
+int ii2_prefix_gather_devices(const ii2_prefix_out* parts, int nparts, int root_device,
+                              ii2_prefix_out* merged);
 
 /* ---- posting codec: replaces intcomp.CompressUint32 (file/writer.go:49) and
  *      intcomp.UncompressUint32 (file/reader.go:100), batched ---------------- */

@@ -150,6 +150,7 @@ PROTOTYPES = {
     "ii2_strerror": (C.c_char_p, [C.c_int]),
     "ii2_last_error": (C.c_char_p, []),
     "ii2_set_stream": (C.c_int, [C.c_void_p]),
+    "ii2_set_device": (C.c_int, [C.c_int]),
     "ii2_kernel_launches": (C.c_uint64, []),
     "ii2_prof_enable": (C.c_int, [C.c_int]),
     "ii2_prof_read": (C.c_int, [C.POINTER(ProfEntry), C.c_int]),
@@ -176,6 +177,7 @@ PROTOTYPES = {
     "ii2_result_to_seg": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p)]),
     "ii2_result_release": (None, [C.c_void_p]),
     "ii2_sync": (C.c_int, []),
+    "ii2_result_device": (C.c_int, [C.c_void_p, C.POINTER(C.c_int)]),
     "ii2_prefix_search_dev": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, u8p, u32p, C.c_uint32,
                                         C.POINTER(PrefixOut)]),
     "ii2_prefix_search": (C.c_int, [C.POINTER(SegView), C.c_int, u8p, u32p, C.c_uint32,
@@ -187,6 +189,10 @@ PROTOTYPES = {
     "ii2_comm_shutdown": (None, []),
     "ii2_read_gather": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p)]),
     "ii2_prefix_gather": (C.c_int, [C.POINTER(PrefixOut), C.c_int, C.POINTER(PrefixOut)]),
+    "ii2_read_gather_devices": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.c_int,
+                                          C.POINTER(C.c_void_p)]),
+    "ii2_prefix_gather_devices": (C.c_int, [C.POINTER(PrefixOut), C.c_int, C.c_int,
+                                            C.POINTER(PrefixOut)]),
     "ii2_intcomp_encode_u32": (C.c_int, [u32p, u64p, C.c_uint64, C.POINTER(u32p),
                                          C.POINTER(u64p)]),
     "ii2_intcomp_decode_u32": (C.c_int, [u32p, u64p, C.c_uint64, C.POINTER(u32p),

@@ -311,6 +311,7 @@ int run_pipeline_impl(ii2_seg* const* segs, int nseg, const uint8_t* min, size_t
                       bool keep_empty, ii2_result** res_out, cudaStream_t s, bool allow_spec = true) {
   ProfScope pipe_scope("pipeline_total", s);
   std::unique_ptr<ii2_result> res(new ii2_result());
+  res->stream = s;
   res->has_dec = want_dec;
   res->has_enc = want_enc;
   if (nseg < 0 || (nseg > 0 && !segs)) return II2_ERR_INVALID;
@@ -713,7 +714,11 @@ int ii2_seg_upload(const ii2_seg_view* v, ii2_seg** seg_out) {
   return rc;
 }
 
-void ii2_seg_release(ii2_seg* seg) { delete seg; }
+void ii2_seg_release(ii2_seg* seg) {
+  if (!seg) return;
+  DeviceScope on(seg->device);
+  delete seg;
+}
 
 int ii2_removed_upload(const uint32_t* removed_sorted, uint64_t nrem, ii2_removed** out) {
   if (!out || (nrem && !removed_sorted)) return II2_ERR_INVALID;
@@ -755,13 +760,19 @@ int ii2_removed_upload(const uint32_t* removed_sorted, uint64_t nrem, ii2_remove
   return II2_OK;
 }
 
-void ii2_removed_release(ii2_removed* rem) { delete rem; }
+void ii2_removed_release(ii2_removed* rem) {
+  if (!rem) return;
+  DeviceScope on(rem->device);
+  delete rem;
+}
 
 int ii2_merge_dev(ii2_seg* const* segs, int nseg, const ii2_removed* rem, uint32_t flags,
                   ii2_result** res) {
   if (!res) return II2_ERR_INVALID;
   *res = nullptr;
-  II2_TRY(ctx_require());
+  int dev = -1;
+  II2_TRY(handles_device(segs, nseg, rem, &dev));
+  II2_TRY(ctx_require_device(dev));
   if (flags == 0) flags = II2_RESULT_DECODED;
   // merge: full windows, min/max recorded, emptied terms dropped
   return run_pipeline(segs, nseg, nullptr, 0, false, nullptr, 0, false, rem,
@@ -774,7 +785,9 @@ int ii2_read_range_dev(ii2_seg* const* segs, int nseg, const uint8_t* min, size_
                        ii2_result** res) {
   if (!res) return II2_ERR_INVALID;
   *res = nullptr;
-  II2_TRY(ctx_require());
+  int dev = -1;
+  II2_TRY(handles_device(segs, nseg, rem, &dev));
+  II2_TRY(ctx_require_device(dev));
   // plain reads keep empty lists (file/writer_test.go:15 round trip); with a removed list the
   // merge-style filter drops emptied terms
   return run_pipeline(segs, nseg, min, minlen, min != nullptr, max, maxlen, max != nullptr, rem,
@@ -801,7 +814,7 @@ int ii2_result_info_get(const ii2_result* r, ii2_result_info* info) {
 int ii2_result_download_merge(const ii2_result* r, uint32_t flags, ii2_merge_out* o) {
   if (!r || !o) return II2_ERR_INVALID;
   memset(o, 0, sizeof(*o));
-  II2_TRY(ctx_require());
+  II2_TRY(ctx_require_device(r->device));
   if (!r->has_enc) {
     set_last_error("result was produced without the encoder");
     return II2_ERR_INVALID;
@@ -841,7 +854,7 @@ int ii2_result_download_merge(const ii2_result* r, uint32_t flags, ii2_merge_out
 int ii2_result_download_read(const ii2_result* r, ii2_read_out* o) {
   if (!r || !o) return II2_ERR_INVALID;
   memset(o, 0, sizeof(*o));
-  II2_TRY(ctx_require());
+  II2_TRY(ctx_require_device(r->device));
   if (!r->has_dec) return II2_ERR_INVALID;
   cudaStream_t s = cur_stream();
   std::unique_ptr<HostOwner> own(new HostOwner());
@@ -861,6 +874,7 @@ int ii2_result_to_seg(ii2_result* r, ii2_seg** seg_out) {
   if (!r->has_dec || !r->out.post_off.p) return II2_ERR_INVALID;
   if (r->T >= 0xFFFFFFFFull) return II2_ERR_UNSUPPORTED;
   std::unique_ptr<ii2_seg> g(new ii2_seg());
+  g->device = r->device;
   g->n_terms = (uint32_t)r->T;
   g->n_post = r->P;
   g->term_bytes_len = r->TB;
@@ -874,7 +888,21 @@ int ii2_result_to_seg(ii2_result* r, ii2_seg** seg_out) {
   return II2_OK;
 }
 
-void ii2_result_release(ii2_result* r) { delete r; }
+void ii2_result_release(ii2_result* r) {
+  if (!r) return;
+  DeviceScope on(r->device);
+  delete r;
+}
+
+int ii2_result_device(const ii2_result* r, int* device) {
+  if (!ctx_ready()) {
+    set_last_error("ii2_init has not succeeded: no CUDA device bound (there is no CPU fallback)");
+    return II2_ERR_NO_DEVICE;
+  }
+  if (!r || !device) return II2_ERR_INVALID;
+  *device = r->device;
+  return II2_OK;
+}
 
 // ------------------------------------------------------------------ PrefixSearch
 static int prefix_search_impl(ii2_seg* const* segs, int nseg, const uint8_t* prefix_bytes,
@@ -945,7 +973,9 @@ int ii2_prefix_search_dev(ii2_seg* const* segs, int nseg, const uint8_t* prefix_
                           const uint32_t* prefix_off, uint32_t nprefix, ii2_prefix_out* out) {
   if (!out || nseg < 0 || (nseg && !segs) || (nprefix && !prefix_off)) return II2_ERR_INVALID;
   memset(out, 0, sizeof(*out));
-  II2_TRY(ctx_require());
+  int dev = -1;
+  II2_TRY(handles_device(segs, nseg, nullptr, &dev));
+  II2_TRY(ctx_require_device(dev));
   cudaStream_t s = cur_stream();
   const int rc = prefix_search_impl(segs, nseg, prefix_bytes, prefix_off, nprefix, out, s);
   if (rc != II2_OK) {

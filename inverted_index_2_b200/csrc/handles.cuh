@@ -1,5 +1,6 @@
 // handles.cuh — the opaque handle types of include/ii2.h (resident segment, removed set, result),
-// shared by the translation units that implement the C-ABI (api.cu, comm.cu).
+// shared by the translation units that implement the C-ABI (api.cu, comm.cu).  Every handle
+// records the CUDA device its memory lives on: calls that take handles run there.
 #pragma once
 #include <string>
 #include <vector>
@@ -10,6 +11,7 @@
 using namespace ii2;
 
 struct ii2_seg {
+  int device = ctx_current_device();
   uint32_t n_terms = 0;
   uint64_t n_post = 0;
   uint64_t term_bytes_len = 0;
@@ -20,6 +22,7 @@ struct ii2_seg {
 };
 
 struct ii2_removed {
+  int device = ctx_current_device();
   uint64_t n = 0;
   DevBuf<uint32_t> sorted;
   DevBuf<uint32_t> bitmap;
@@ -35,6 +38,8 @@ struct ii2_removed {
 };
 
 struct ii2_result {
+  int device = ctx_current_device();
+  cudaStream_t stream = nullptr;  // the stream that produced it (in-process gathers wait for it)
   EmitOut out;
   uint64_t T = 0, TB = 0, P = 0, E = 0;
   uint64_t postings_in = 0, terms_merged = 0;
@@ -44,6 +49,22 @@ struct ii2_result {
   std::string min_term, max_term;
 };
 
+// The device of one call's handles (segments and removed set; NULL entries are left to the
+// call's own checks): -1 when there is none (the call runs on the selected device),
+// II2_ERR_INVALID when they live on different devices.
+inline int handles_device(ii2_seg* const* segs, int nseg, const ii2_removed* rem, int* device) {
+  int d = rem ? rem->device : -1;
+  for (int i = 0; segs && i < nseg; i++) {
+    if (!segs[i]) continue;
+    if (d >= 0 && segs[i]->device != d) {
+      set_last_error("handles of one call live on different devices (%d and %d)", d, segs[i]->device);
+      return II2_ERR_INVALID;
+    }
+    d = segs[i]->device;
+  }
+  *device = d;
+  return II2_OK;
+}
 
 // Host-side outputs of the C-ABI (ii2_merge_out, ii2_read_out, ii2_prefix_out ...): pinned
 // buffers owned by one object behind the struct's `_owner` field.

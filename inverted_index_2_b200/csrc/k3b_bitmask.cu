@@ -25,6 +25,7 @@
 using namespace ii2;
 
 struct ii2_bitmask {
+  int device = ctx_current_device();  // where its arrays live: every operation runs there
   uint64_t n = 0;  // dictionary length
   DevBuf<uint32_t> values;
   uint64_t values_cap = 0;
@@ -580,13 +581,17 @@ int ii2_bitmask_new(const uint32_t* init, uint64_t n, ii2_bitmask** out) {
   return II2_OK;
 }
 
-void ii2_bitmask_free(ii2_bitmask* bm) { delete bm; }
+void ii2_bitmask_free(ii2_bitmask* bm) {
+  if (!bm) return;
+  DeviceScope on(bm->device);
+  delete bm;
+}
 
 int ii2_bitmask_all_values(const ii2_bitmask* bm, uint32_t** vals, uint64_t* n) {
   if (!bm || !vals || !n) return II2_ERR_INVALID;
   *vals = nullptr;
   *n = 0;
-  II2_TRY(ctx_require());
+  II2_TRY(ctx_require_device(bm->device));
   cudaStream_t s = cur_stream();
   uint32_t* h = static_cast<uint32_t*>(pinned_alloc(bm->n * 4 + 4));
   if (!h) return II2_ERR_NOMEM;
@@ -609,7 +614,7 @@ int ii2_bitmask_put(ii2_bitmask* bm, const uint32_t* vals, uint64_t n, uint8_t**
   if (!bm || !bytes || !nbytes || (n && !vals)) return II2_ERR_INVALID;
   *bytes = nullptr;
   *nbytes = 0;
-  II2_TRY(ctx_require());
+  II2_TRY(ctx_require_device(bm->device));
   if (bm->n + n >= 0xFFFFFFFEull) {
     set_last_error("bitmask dictionary would exceed uint32 indexes");
     return II2_ERR_UNSUPPORTED;
@@ -723,7 +728,7 @@ int ii2_bitmask_get(const ii2_bitmask* bm, const uint8_t* enc, uint64_t nenc, ui
   if (!bm || !vals || !n || (nenc && !enc)) return II2_ERR_INVALID;
   *vals = nullptr;
   *n = 0;
-  II2_TRY(ctx_require());
+  II2_TRY(ctx_require_device(bm->device));
   cudaStream_t s = cur_stream();
   ProfScope scope("k3b_get", s);
   const uint32_t meta_cap = (uint32_t)std::min<uint64_t>(65536, nenc / 4 + 1);

@@ -3,6 +3,7 @@
 
 #include <cstdarg>
 #include <map>
+#include <memory>
 #include <mutex>
 
 #include "runtime.cuh"
@@ -26,27 +27,81 @@ void set_last_error(const char* fmt, ...) {
 }
 
 // ------------------------------------------------------------------ context
+// The bound device set.  Per-thread state is keyed by CUDA ordinal (so it stays right across
+// ii2_shutdown + ii2_init of another set): t_sel is the device ii2_set_device chose (-1: the
+// first of the set), t_dev the device of the running call (set at call entry, so finding the
+// per-device state costs no CUDA runtime query).
 struct Ctx {
   std::mutex m;
   bool ready = false;
-  int device = -1;
+  int ndev = 0;
+  int devices[kMaxDevices] = {};
+  bool peer[kMaxDevices][kMaxDevices] = {};  // [a][b]: kernels on devices[a] read devices[b]
 };
 static Ctx g_ctx;
+static thread_local int t_sel = -1;
+static thread_local int t_dev = 0;
+constexpr int kMaxOrdinal = 64;  // CUDA ordinals the per-thread tables cover
+
+static int slot_of(int device) {
+  for (int i = 0; i < g_ctx.ndev; i++)
+    if (g_ctx.devices[i] == device) return i;
+  return -1;
+}
 
 bool ctx_ready() { return g_ctx.ready; }
+int ctx_device_count() { return g_ctx.ready ? g_ctx.ndev : 0; }
+int ctx_current_device() { return t_dev; }
+bool ctx_bound(int device) { return g_ctx.ready && slot_of(device) >= 0; }
+bool ctx_peer(int dev, int peer) {
+  const int a = slot_of(dev), b = slot_of(peer);
+  return a >= 0 && b >= 0 && (a == b || g_ctx.peer[a][b]);
+}
 
-int ctx_require() {
-  if (!g_ctx.ready) {
-    set_last_error("ii2_init has not succeeded: no CUDA device bound (there is no CPU fallback)");
-    return II2_ERR_NO_DEVICE;
-  }
+// the device this thread selected, if it is still bound; else the first of the set
+static int selected_device() {
+  return (t_sel >= 0 && slot_of(t_sel) >= 0) ? t_sel : g_ctx.devices[0];
+}
+
+static int ctx_enter(int device) {
+  t_dev = device;
   // Each host thread needs the device current.
-  cudaError_t e = cudaSetDevice(g_ctx.device);
+  cudaError_t e = cudaSetDevice(device);
   if (e != cudaSuccess) {
-    set_last_error("cudaSetDevice(%d): %s", g_ctx.device, cudaGetErrorString(e));
+    set_last_error("cudaSetDevice(%d): %s", device, cudaGetErrorString(e));
     return II2_ERR_CUDA;
   }
   return II2_OK;
+}
+
+static int no_device() {
+  set_last_error("ii2_init has not succeeded: no CUDA device bound (there is no CPU fallback)");
+  return II2_ERR_NO_DEVICE;
+}
+
+int ctx_require() {
+  if (!g_ctx.ready) return no_device();
+  return ctx_enter(selected_device());
+}
+
+int ctx_require_device(int device) {
+  if (device < 0 || !g_ctx.ready) return ctx_require();
+  if (slot_of(device) < 0) {
+    set_last_error("device %d is not in the set bound by ii2_init", device);
+    return II2_ERR_INVALID;
+  }
+  return ctx_enter(device);
+}
+
+DeviceScope::DeviceScope(int device) {
+  if (device < 0 || cudaGetDevice(&prev) != cudaSuccess) {
+    prev = -1;
+    return;
+  }
+  if (prev == device || cudaSetDevice(device) != cudaSuccess) prev = -1;
+}
+DeviceScope::~DeviceScope() {
+  if (prev >= 0) cudaSetDevice(prev);
 }
 
 struct ThreadStream {
@@ -54,6 +109,7 @@ struct ThreadStream {
   cudaStream_t aux = nullptr;
   cudaStream_t copy[4] = {};
   cudaEvent_t ev[16] = {};
+  cudaEvent_t wait_ev = nullptr;  // stream_wait
   cudaStream_t user = nullptr;
   bool use_user = false;
   ~ThreadStream() {
@@ -61,27 +117,57 @@ struct ThreadStream {
     // already be torn down when thread-local destructors run at process exit.
   }
 };
-static thread_local ThreadStream t_stream;
+static thread_local std::unique_ptr<ThreadStream> t_streams[kMaxOrdinal];  // by CUDA ordinal
+
+static ThreadStream& thread_stream(int device) {
+  std::unique_ptr<ThreadStream>& p = t_streams[device];
+  if (!p) p.reset(new ThreadStream());
+  return *p;
+}
 
 cudaStream_t cur_stream() {
-  if (t_stream.use_user) return t_stream.user;
-  if (!t_stream.own) cudaStreamCreateWithFlags(&t_stream.own, cudaStreamNonBlocking);
-  return t_stream.own;
+  ThreadStream& t = thread_stream(t_dev);
+  if (t.use_user) return t.user;
+  if (!t.own) cudaStreamCreateWithFlags(&t.own, cudaStreamNonBlocking);
+  return t.own;
 }
 
 cudaStream_t aux_stream() {
-  if (!t_stream.aux) cudaStreamCreateWithFlags(&t_stream.aux, cudaStreamNonBlocking);
-  return t_stream.aux;
+  ThreadStream& t = thread_stream(t_dev);
+  if (!t.aux) cudaStreamCreateWithFlags(&t.aux, cudaStreamNonBlocking);
+  return t.aux;
 }
 
 cudaStream_t copy_stream(int i) {
-  if (!t_stream.copy[i]) cudaStreamCreateWithFlags(&t_stream.copy[i], cudaStreamNonBlocking);
-  return t_stream.copy[i];
+  ThreadStream& t = thread_stream(t_dev);
+  if (!t.copy[i]) cudaStreamCreateWithFlags(&t.copy[i], cudaStreamNonBlocking);
+  return t.copy[i];
 }
 
 cudaEvent_t aux_event(int i) {
-  if (!t_stream.ev[i]) cudaEventCreateWithFlags(&t_stream.ev[i], cudaEventDisableTiming);
-  return t_stream.ev[i];
+  ThreadStream& t = thread_stream(t_dev);
+  if (!t.ev[i]) cudaEventCreateWithFlags(&t.ev[i], cudaEventDisableTiming);
+  return t.ev[i];
+}
+
+int stream_wait(cudaStream_t waiter, cudaStream_t producer, int producer_device) {
+  if (slot_of(producer_device) < 0) {
+    set_last_error("device %d is not in the set bound by ii2_init", producer_device);
+    return II2_ERR_INVALID;
+  }
+  ThreadStream& t = thread_stream(producer_device);
+  const int here = t_dev;
+  if (producer_device != here) II2_CUDA_TRY(cudaSetDevice(producer_device));
+  cudaError_t e = cudaSuccess;
+  if (!t.wait_ev) e = cudaEventCreateWithFlags(&t.wait_ev, cudaEventDisableTiming);
+  if (e == cudaSuccess) e = cudaEventRecord(t.wait_ev, producer);
+  if (producer_device != here) II2_CUDA_TRY(cudaSetDevice(here));
+  if (e != cudaSuccess) {
+    set_last_error("event on the stream of device %d: %s", producer_device, cudaGetErrorString(e));
+    return II2_ERR_CUDA;
+  }
+  II2_CUDA_TRY(cudaStreamWaitEvent(waiter, t.wait_ev, 0));
+  return II2_OK;
 }
 
 // ------------------------------------------------------------------ pinned pool
@@ -206,21 +292,24 @@ static void pinned_drain() {
 
 // ------------------------------------------------------------------ scratch arena
 struct Arena {
+  int device = 0;
   uint8_t* base = nullptr;
   size_t cap = 0, used = 0, want = 0;
   std::vector<void*> spill;  // stream-ordered allocations made when the block was too small
 };
 static std::mutex g_arena_m;
 static std::vector<Arena*> g_arenas;
-static thread_local Arena* t_arena = nullptr;
+static thread_local Arena* t_arena[kMaxOrdinal] = {};  // by CUDA ordinal
 
 static Arena* my_arena() {
-  if (!t_arena) {
-    t_arena = new Arena();
+  Arena*& a = t_arena[t_dev];
+  if (!a) {
+    a = new Arena();
+    a->device = t_dev;
     std::lock_guard<std::mutex> lk(g_arena_m);
-    g_arenas.push_back(t_arena);
+    g_arenas.push_back(a);
   }
-  return t_arena;
+  return a;
 }
 
 void* arena_alloc(size_t bytes, cudaStream_t stream) {
@@ -268,6 +357,7 @@ void arena_reset(cudaStream_t stream) {
 void arena_release_all() {
   std::lock_guard<std::mutex> lk(g_arena_m);
   for (Arena* a : g_arenas) {
+    DeviceScope on(a->device);
     if (a->base) cudaFree(a->base);
     a->base = nullptr;
     a->cap = a->used = a->want = 0;
@@ -277,6 +367,7 @@ void arena_release_all() {
 // ------------------------------------------------------------------ instrumentation
 struct ProfRec {
   const char* name;
+  int device;  // CUDA ordinal of the events
   cudaEvent_t e0, e1;
   double host_t0, host_ms;
 };
@@ -289,7 +380,7 @@ struct Prof {
   std::mutex m;
   std::atomic<bool> on{false};
   std::vector<ProfRec> recs;
-  std::vector<cudaEvent_t> spare;
+  std::vector<cudaEvent_t> spare[kMaxOrdinal];  // by CUDA ordinal (an event belongs to one device)
 };
 static Prof g_prof;
 
@@ -298,10 +389,12 @@ ProfScope::ProfScope(const char* name, cudaStream_t stream) : s(stream), slot(-1
   std::lock_guard<std::mutex> lk(g_prof.m);
   ProfRec r;
   r.name = name;
+  r.device = t_dev;
+  std::vector<cudaEvent_t>& spare = g_prof.spare[t_dev];
   for (cudaEvent_t* e : {&r.e0, &r.e1}) {
-    if (!g_prof.spare.empty()) {
-      *e = g_prof.spare.back();
-      g_prof.spare.pop_back();
+    if (!spare.empty()) {
+      *e = spare.back();
+      spare.pop_back();
     } else if (cudaEventCreate(e) != cudaSuccess) {
       return;
     }
@@ -325,8 +418,8 @@ void ProfScope::end() {
 
 static void prof_reset_locked() {
   for (ProfRec& r : g_prof.recs) {
-    g_prof.spare.push_back(r.e0);
-    g_prof.spare.push_back(r.e1);
+    g_prof.spare[r.device].push_back(r.e0);
+    g_prof.spare[r.device].push_back(r.e1);
   }
   g_prof.recs.clear();
 }
@@ -529,40 +622,93 @@ const char* ii2_last_error(void) { return t_last_error; }
 
 int ii2_init(const int* devices, int ndev) {
   std::lock_guard<std::mutex> lk(g_ctx.m);
-  if (ndev > 1) {
-    set_last_error("one process drives one GPU: pass exactly one device (got %d)", ndev);
+  if (ndev < 0 || ndev > kMaxDevices || (!devices && ndev > 1)) {
+    set_last_error("ii2_init: %d devices (1 .. %d, or devices == NULL for device 0)", ndev, kMaxDevices);
     return II2_ERR_INVALID;
   }
-  int dev = (devices && ndev == 1) ? devices[0] : 0;
-  if (g_ctx.ready) {
-    if (g_ctx.device == dev) return II2_OK;
-    set_last_error("already initialised on device %d", g_ctx.device);
-    return II2_ERR_INVALID;
-  }
+  int want[kMaxDevices];
+  int n = (devices && ndev >= 1) ? ndev : 1;
+  for (int i = 0; i < n; i++) want[i] = (devices && ndev >= 1) ? devices[i] : 0;
+  for (int i = 0; i < n; i++)
+    for (int j = 0; j < i; j++)
+      if (want[i] == want[j]) {
+        set_last_error("ii2_init: device %d listed twice", want[i]);
+        return II2_ERR_INVALID;
+      }
   int count = 0;
   cudaError_t e = cudaGetDeviceCount(&count);
   if (e != cudaSuccess || count == 0) {
     set_last_error("no CUDA device: %s", e != cudaSuccess ? cudaGetErrorString(e) : "count=0");
     return II2_ERR_NO_DEVICE;
   }
-  if (dev < 0 || dev >= count) {
-    set_last_error("device %d out of range (have %d)", dev, count);
+  for (int i = 0; i < n; i++) {
+    const int dev = want[i];
+    if (dev < 0 || dev >= count || dev >= kMaxOrdinal) {
+      set_last_error("device %d out of range (have %d)", dev, count);
+      return II2_ERR_INVALID;
+    }
+  }
+  if (g_ctx.ready) {  // idempotent for the same set (any order); any other set is refused
+    bool same = n == g_ctx.ndev;
+    for (int i = 0; i < n && same; i++) same = slot_of(want[i]) >= 0;
+    if (same) return II2_OK;
+    set_last_error("already initialised on %d device(s), the first being %d", g_ctx.ndev, g_ctx.devices[0]);
     return II2_ERR_INVALID;
   }
-  II2_CUDA_TRY(cudaSetDevice(dev));
-  cudaDeviceProp prop;
-  II2_CUDA_TRY(cudaGetDeviceProperties(&prop, dev));
-  if (prop.major < 10) {
-    set_last_error("device %d is sm_%d%d; this library is built for sm_100a only", dev, prop.major,
-                   prop.minor);
-    return II2_ERR_NO_DEVICE;
+  for (int i = 0; i < n; i++) {
+    const int dev = want[i];
+    II2_CUDA_TRY(cudaSetDevice(dev));
+    cudaDeviceProp prop;
+    II2_CUDA_TRY(cudaGetDeviceProperties(&prop, dev));
+    if (prop.major < 10) {
+      set_last_error("device %d is sm_%d%d; this library is built for sm_100a only", dev, prop.major,
+                     prop.minor);
+      return II2_ERR_NO_DEVICE;
+    }
+    // Keep freed stream-ordered memory in the pool instead of returning it to the driver.
+    cudaMemPool_t pool;
+    II2_CUDA_TRY(cudaDeviceGetDefaultMemPool(&pool, dev));
+    uint64_t thresh = UINT64_MAX;
+    II2_CUDA_TRY(cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &thresh));
   }
-  // Keep freed stream-ordered memory in the pool instead of returning it to the driver.
-  cudaMemPool_t pool;
-  II2_CUDA_TRY(cudaDeviceGetDefaultMemPool(&pool, dev));
-  uint64_t thresh = UINT64_MAX;
-  II2_CUDA_TRY(cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &thresh));
-  g_ctx.device = dev;
+  // Peer access of this process's contexts wherever the hardware allows it (the in-process
+  // gathers read other devices' HBM directly).  Peer access covers cudaMalloc memory only: the
+  // stream-ordered allocations (every result array) come from the device's default pool, which
+  // another device may read only once the pool grants it access (cudaMemPoolSetAccess).
+  bool peer[kMaxDevices][kMaxDevices] = {};
+  for (int i = 0; i < n; i++) {
+    for (int j = 0; j < n; j++) {
+      if (i == j) continue;
+      int can = 0;
+      II2_CUDA_TRY(cudaDeviceCanAccessPeer(&can, want[i], want[j]));
+      if (!can) continue;
+      II2_CUDA_TRY(cudaSetDevice(want[i]));
+      e = cudaDeviceEnablePeerAccess(want[j], 0);
+      if (e == cudaErrorPeerAccessAlreadyEnabled) {
+        cudaGetLastError();
+        e = cudaSuccess;
+      }
+      II2_CUDA_TRY(e);
+      cudaMemPool_t pool;
+      II2_CUDA_TRY(cudaDeviceGetDefaultMemPool(&pool, want[j]));
+      cudaMemAccessDesc acc = {};
+      acc.location.type = cudaMemLocationTypeDevice;
+      acc.location.id = want[i];
+      acc.flags = cudaMemAccessFlagsProtReadWrite;
+      e = cudaMemPoolSetAccess(pool, &acc, 1);
+      if (e != cudaSuccess) {  // that pair stays unreadable: the gathers refuse it
+        cudaGetLastError();
+        continue;
+      }
+      peer[i][j] = true;
+    }
+  }
+  II2_CUDA_TRY(cudaSetDevice(want[0]));
+  g_ctx.ndev = n;
+  for (int i = 0; i < n; i++) {
+    g_ctx.devices[i] = want[i];
+    for (int j = 0; j < n; j++) g_ctx.peer[i][j] = peer[i][j];
+  }
   g_ctx.ready = true;
   return II2_OK;
 }
@@ -570,16 +716,30 @@ int ii2_init(const int* devices, int ndev) {
 int ii2_shutdown(void) {
   std::lock_guard<std::mutex> lk(g_ctx.m);
   if (!g_ctx.ready) return II2_OK;
-  cudaDeviceSynchronize();
+  for (int i = 0; i < g_ctx.ndev; i++) {
+    DeviceScope on(g_ctx.devices[i]);
+    cudaDeviceSynchronize();
+  }
   arena_release_all();
   pinned_drain();
   g_ctx.ready = false;
   return II2_OK;
 }
 
+int ii2_set_device(int device) {
+  if (!g_ctx.ready) return no_device();
+  if (slot_of(device) < 0) {
+    set_last_error("device %d is not in the set bound by ii2_init", device);
+    return II2_ERR_INVALID;
+  }
+  t_sel = device;
+  return II2_OK;
+}
+
 int ii2_set_stream(void* cuda_stream) {
-  t_stream.user = static_cast<cudaStream_t>(cuda_stream);
-  t_stream.use_user = cuda_stream != nullptr;
+  ThreadStream& t = thread_stream(g_ctx.ready ? selected_device() : 0);
+  t.user = static_cast<cudaStream_t>(cuda_stream);
+  t.use_user = cuda_stream != nullptr;
   return II2_OK;
 }
 
@@ -624,6 +784,13 @@ void ii2_free(void* p) { pinned_free(p); }
 int ii2_sync(void) {
   II2_TRY(ctx_require());
   II2_CUDA_TRY(cudaStreamSynchronize(cur_stream()));
+  for (int i = 0; i < g_ctx.ndev; i++) {  // this thread's streams on the other bound devices
+    const int d = g_ctx.devices[i];
+    if (d == t_dev || !t_streams[d]) continue;
+    const ThreadStream& t = *t_streams[d];
+    if (t.use_user) II2_CUDA_TRY(cudaStreamSynchronize(t.user));
+    if (t.own) II2_CUDA_TRY(cudaStreamSynchronize(t.own));
+  }
   return II2_OK;
 }
 

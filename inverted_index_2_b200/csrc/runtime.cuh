@@ -1,5 +1,6 @@
-// runtime.cuh — process context, per-thread streams, stream-ordered device buffers,
-// pinned host pool.  One process drives one GPU (torch.distributed-style launch).
+// runtime.cuh — process context, per-(thread, device) streams and scratch, stream-ordered
+// device buffers, pinned host pool.  One process drives one GPU or a bound set of up to
+// kMaxDevices GPUs (ii2_init); every call runs on one device of the set.
 #pragma once
 #include <vector>
 
@@ -7,14 +8,39 @@
 
 namespace ii2 {
 
+constexpr int kMaxDevices = 16;  // GPUs one process can bind (ii2_init)
+
 bool ctx_ready();
-int ctx_require();            // II2_OK or II2_ERR_NO_DEVICE (sets last error)
+// Enter a call on the device the calling thread selected (ii2_set_device; devices[0] by
+// default) and make it current: II2_OK or II2_ERR_NO_DEVICE (sets last error).
+int ctx_require();
+// Enter a call on CUDA device `device` (the device of the call's handles); device < 0 means the
+// selected one.  II2_ERR_INVALID if the device is not in the bound set.
+int ctx_require_device(int device);
+int ctx_current_device();      // CUDA ordinal of the running call (devices[0] outside calls)
+int ctx_device_count();        // devices bound by ii2_init (0 before)
+bool ctx_bound(int device);    // device is in the bound set
+// kernels on `dev` can read all of `peer`'s memory: peer access is on and `peer`'s default
+// memory pool (every stream-ordered allocation) grants `dev` access
+bool ctx_peer(int dev, int peer);
+// Make `waiter` (a stream of the running call's device) wait for the work queued so far on
+// `producer`, a stream of bound device `producer_device` (one reusable event per host thread
+// and device; the wait is taken at once, so the event can be recorded again).
+int stream_wait(cudaStream_t waiter, cudaStream_t producer, int producer_device);
+// Makes `device` current for a scope and restores the previous device (handle releases from
+// any thread).
+struct DeviceScope {
+  int prev = -1;
+  explicit DeviceScope(int device);
+  ~DeviceScope();
+};
+// The streams and events below belong to the calling thread AND the running call's device.
 cudaStream_t cur_stream();    // this thread's stream (caller-provided or library-owned)
 cudaStream_t aux_stream();    // a second library-owned stream of this thread (kernel overlap)
 cudaStream_t copy_stream(int i);  // copy-engine streams of this thread (staging of host slices), i < 4
 cudaEvent_t aux_event(int i);  // this thread's reusable timing-free events, i < 16
 
-// Per-thread scratch arena: one grow-only device block, bump-allocated during a pipeline call
+// Per-(thread, device) scratch arena: one grow-only device block, bump-allocated during a pipeline call
 // and reset when the call is over.  GB-sized cudaMallocAsync requests were measured at tens of
 // milliseconds per call on B200 (the pool re-maps physical memory); the arena makes every
 // intermediate buffer free of charge after the first call.

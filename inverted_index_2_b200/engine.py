@@ -55,10 +55,10 @@ def _bytes_arg(b: bytes | None):
 
 
 class DeviceSegment:
-    """A segment resident in HBM (ii2_seg)."""
+    """A segment resident in HBM (ii2_seg) of CUDA device `device`."""
 
-    def __init__(self, eng: "Engine", handle: int, n_terms: int):
-        self.eng, self.h, self.n_terms = eng, handle, n_terms
+    def __init__(self, eng: "Engine", handle: int, n_terms: int, device: int):
+        self.eng, self.h, self.n_terms, self.device = eng, handle, n_terms, device
 
     def release(self):
         if self.h:
@@ -73,8 +73,8 @@ class DeviceSegment:
 
 
 class DeviceRemoved:
-    def __init__(self, eng: "Engine", handle: int):
-        self.eng, self.h = eng, handle
+    def __init__(self, eng: "Engine", handle: int, device: int):
+        self.eng, self.h, self.device = eng, handle, device
 
     def release(self):
         if self.h:
@@ -89,10 +89,10 @@ class DeviceRemoved:
 
 
 class DeviceResult:
-    """Merge / read result resident in HBM (ii2_result)."""
+    """Merge / read result resident in HBM (ii2_result) of CUDA device `device`."""
 
-    def __init__(self, eng: "Engine", handle: int):
-        self.eng, self.h = eng, handle
+    def __init__(self, eng: "Engine", handle: int, device: int):
+        self.eng, self.h, self.device = eng, handle, device
 
     def info(self) -> A.ResultInfo:
         info = A.ResultInfo()
@@ -144,7 +144,7 @@ class DeviceResult:
         h = C.c_void_p()
         n = int(self.info().terms_count)
         self.eng._check(self.eng.lib.ii2_result_to_seg(self.h, C.byref(h)), "result_to_seg")
-        return DeviceSegment(self.eng, h.value, n)
+        return DeviceSegment(self.eng, h.value, n, self.device)
 
     def release(self):
         if self.h:
@@ -206,19 +206,35 @@ class Bitmask:
 
 
 class Engine:
-    """One process drives one GPU (ii2_init binds it)."""
+    """The process's GPUs (ii2_init binds them): one device, or with `devices` a set of them.
+
+    With a set, host-buffer calls and uploads of a thread run on the device it selected with
+    set_device (devices[0] by default); calls on resident handles run on the handles' device."""
 
     _default = None
     _lock = threading.Lock()
 
-    def __init__(self, device: int = 0):
+    def __init__(self, device: int = 0, devices: list[int] | None = None):
         self.lib = load_library()
-        dev = (C.c_int * 1)(device)
-        rc = self.lib.ii2_init(dev, 1)
+        devs = [int(d) for d in devices] if devices is not None else [device]
+        if not devs:
+            raise ValueError("Engine(devices=...) needs at least one device")
+        arr = (C.c_int * max(1, len(devs)))(*devs)
+        rc = self.lib.ii2_init(arr, len(devs))
         if rc != A.II2_OK:
             raise EngineError(rc, "ii2_init failed — no CPU fallback exists",
                               self.lib.ii2_last_error().decode())
-        self.device = device
+        self.device = devs[0]
+        self.devices = devs
+        self._tls = threading.local()
+
+    def set_device(self, device: int) -> None:
+        """Device of this thread's host-buffer calls and uploads (one of `devices`)."""
+        self._check(self.lib.ii2_set_device(int(device)), "set_device")
+        self._tls.device = int(device)
+
+    def selected_device(self) -> int:
+        return getattr(self._tls, "device", self.device)
 
     @classmethod
     def default(cls) -> "Engine":
@@ -273,7 +289,7 @@ class Engine:
         v = seg.view()
         h = C.c_void_p()
         self._check(self.lib.ii2_seg_upload(C.byref(v), C.byref(h)), "seg_upload")
-        return DeviceSegment(self, h.value, seg.n_terms)
+        return DeviceSegment(self, h.value, seg.n_terms, self.selected_device())
 
     def upload_removed(self, removed) -> DeviceRemoved:
         r = np.ascontiguousarray(removed, dtype=np.uint32)
@@ -281,7 +297,18 @@ class Engine:
         self._check(self.lib.ii2_removed_upload(
             A.np_ptr(r, A.u32p) if len(r) else C.cast(None, A.u32p), len(r), C.byref(h)),
             "removed_upload")
-        return DeviceRemoved(self, h.value)
+        return DeviceRemoved(self, h.value, self.selected_device())
+
+    def _call_device(self, segs, removed) -> int:
+        """Where a call on these handles runs (and its result lives)."""
+        if segs:
+            return segs[0].device
+        return removed.device if removed is not None else self.selected_device()
+
+    def result_device(self, res: DeviceResult) -> int:
+        d = C.c_int(-1)
+        self._check(self.lib.ii2_result_device(res.h, C.byref(d)), "result_device")
+        return d.value
 
     @staticmethod
     def _handles(segs: list[DeviceSegment]):
@@ -297,7 +324,7 @@ class Engine:
         self._check(self.lib.ii2_merge_dev(self._handles(segs), len(segs),
                                            removed.h if removed else None, flags, C.byref(h)),
                     "merge_dev")
-        return DeviceResult(self, h.value)
+        return DeviceResult(self, h.value, self._call_device(segs, removed))
 
     def read_range_dev(self, segs: list[DeviceSegment], min_term: bytes | None = None,
                        max_term: bytes | None = None, removed: DeviceRemoved | None = None
@@ -308,7 +335,7 @@ class Engine:
         self._check(self.lib.ii2_read_range_dev(self._handles(segs), len(segs), pmin, nmin, pmax,
                                                 nmax, removed.h if removed else None, C.byref(h)),
                     "read_range_dev")
-        return DeviceResult(self, h.value)
+        return DeviceResult(self, h.value, self._call_device(segs, removed))
 
     # ---- ingest batching (Shard.Put x D + Shard.Merge as one call) ----------------------------
     def ingest(self, docs: list[tuple[list[bytes], int]], removed=None, decoded: bool = False
@@ -439,7 +466,7 @@ class Engine:
         results on `root` (every rank if root < 0) — InvertedIndex.Read over all shards."""
         h = C.c_void_p()
         self._check(self.lib.ii2_read_gather(local.h, root, C.byref(h)), "read_gather")
-        return DeviceResult(self, h.value)
+        return DeviceResult(self, h.value, local.device)
 
     def prefix_search_gather(self, segs: list[DeviceSegment], prefixes: list[bytes], root: int = 0
                              ) -> dict[bytes, np.ndarray]:
@@ -454,6 +481,54 @@ class Engine:
             self._check(self.lib.ii2_prefix_gather(C.byref(local), root, C.byref(merged)), "prefix_gather")
         finally:
             self.lib.ii2_prefix_out_free(C.byref(local))
+        return self._prefix_result(prefixes, merged)
+
+    # ---- in-process gathers over the devices of this process -----------------------------
+    def read_gather_devices(self, parts: list[DeviceResult], root_device: int) -> DeviceResult:
+        """The part-ordered concatenation of decoded read results that live on any of this
+        process's devices, on `root_device` (one peer-reading kernel there)."""
+        arr = (C.c_void_p * max(1, len(parts)))()
+        for i, p in enumerate(parts):
+            arr[i] = p.h
+        h = C.c_void_p()
+        self._check(self.lib.ii2_read_gather_devices(arr, len(parts), int(root_device), C.byref(h)),
+                    "read_gather_devices")
+        return DeviceResult(self, h.value, int(root_device))
+
+    def prefix_search_dev_out(self, segs: list[DeviceSegment], prefixes: list[bytes]) -> A.PrefixOut:
+        """ii2_prefix_search_dev's raw output (input of prefix_gather_devices); free it with
+        prefix_out_free."""
+        blob, off = self._prefix_args(prefixes)
+        out = A.PrefixOut()
+        self._check(self.lib.ii2_prefix_search_dev(self._handles(segs), len(segs),
+                                                   A.np_ptr(blob, A.u8p), A.np_ptr(off, A.u32p),
+                                                   len(prefixes), C.byref(out)), "prefix_search_dev")
+        return out
+
+    def prefix_out_free(self, out: A.PrefixOut) -> None:
+        self.lib.ii2_prefix_out_free(C.byref(out))
+
+    def prefix_gather_devices(self, parts: list, prefixes: list[bytes], root_device: int
+                              ) -> dict[bytes, np.ndarray]:
+        """found[prefix] over several devices: `parts` are raw prefix outputs of `prefixes`
+        (prefix_search_dev_out; the caller keeps and frees them) or groups of resident segments
+        (searched here, each group on its own device); the union runs on `root_device`."""
+        outs, owned = [], []
+        try:
+            for p in parts:
+                if isinstance(p, A.PrefixOut):
+                    outs.append(p)
+                else:
+                    o = self.prefix_search_dev_out(list(p), prefixes)
+                    owned.append(o)
+                    outs.append(o)
+            arr = (A.PrefixOut * max(1, len(outs)))(*outs)
+            merged = A.PrefixOut()
+            self._check(self.lib.ii2_prefix_gather_devices(arr, len(outs), int(root_device),
+                                                           C.byref(merged)), "prefix_gather_devices")
+        finally:
+            for o in owned:
+                self.prefix_out_free(o)
         return self._prefix_result(prefixes, merged)
 
     # ---- misc --------------------------------------------------------------------------
