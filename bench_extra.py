@@ -4,6 +4,8 @@
   C3  term-range read union across 256 segments with 5 % removed_list filtering (µs per call)
   C4  file/bitmask + intcomp encode/decode sweep, posting-list lengths 16 .. 16M
   prefix  PrefixSearch batches over 64 resident segments (µs per call)
+  lookup  batched exact-term reads (ii2_lookup_dev) on the C3 and C2 workloads, Q = 1 .. 65 536
+        keys per call, against a loop of point reads for Q <= 256
   multidev  one process over every visible GPU (Engine(devices=...)): weak-scaling compaction from
         one host thread per device, a 1 % read partitioned over the devices + ii2_read_gather_devices,
         and ii2_prefix_gather_devices of the prefix batch; each checked against one device
@@ -111,6 +113,62 @@ def prefix(eng, a):
     print(json.dumps({"config": "PrefixSearch over 64 resident segments (one C-ABI call per batch, "
                                 "results downloaded)", "terms": a.terms, "postings": w.postings_in,
                       "results": out}))
+
+
+def lookup(eng, a):
+    """Read(t, t) for Q keys as ONE ii2_lookup_dev call (results downloaded) on the C3 workload
+    (256 segments, 5 % removed: read + merge-style filter) and the 64-segment C2 workload, random
+    keys of which ~10 % are absent (a term with a byte appended).  For Q <= 256 the same keys are
+    also read one by one (read_range_dev(t, t) + download), and every batch must equal that loop."""
+    card = _card()
+    rows = []
+    for name, nseg, pres, seed, with_rem in (("C3", 256, 0.125, 0xC3, True), ("C2", 64, 0.5, 0xC2, False)):
+        w = synth.make_workload(a.terms, nseg, a.postings, seed=seed, presence=pres)
+        dsegs = [eng.upload(s) for s in w.segments]
+        drem = eng.upload_removed(w.removed) if with_rem else None
+        n = len(w.term_off) - 1
+        rng = np.random.default_rng(8)
+        for q in (1, 16, 256, 4096, 65536):
+            ids = rng.integers(0, n, size=q)
+            absent = rng.random(q) < 0.1
+            keys = [synth.term_at(w.term_bytes, w.term_off, int(i)) + (b"\x01" if x else b"")
+                    for i, x in zip(ids, absent)]
+            res = None
+
+            def call():
+                nonlocal res
+                res = eng.lookup_dev(dsegs, keys, drem)
+            med, p99 = timed(call, 50 if q <= 4096 else 10)
+            out = int(sum(len(v) for v in res if v is not None))
+            row = {"workload": name, "segments": nseg, "removed": with_rem, "keys": q,
+                   "found": int(sum(v is not None for v in res)), "postings_out": out,
+                   "median_us": 1e6 * med, "p99_us": 1e6 * p99, "us_per_key": 1e6 * med / q,
+                   "postings_out_per_s": out / med}
+            if q <= 256:
+                loop = None
+
+                def point_loop():
+                    nonlocal loop
+                    loop = []
+                    for k in keys:
+                        r = eng.read_range_dev(dsegs, k, k, drem)
+                        d = r.download_read()
+                        r.release()
+                        loop.append(d.post if d.n_terms else None)
+                lmed, lp99 = timed(point_loop, 10 if q <= 16 else 3)
+                same = all((x is None and y is None) or (x is not None and y is not None and np.array_equal(x, y))
+                           for x, y in zip(res, loop))
+                row.update({"point_loop_median_us": 1e6 * lmed, "point_loop_us_per_key": 1e6 * lmed / q,
+                            "speedup_vs_point_loop": lmed / med, "same_as_point_loop": bool(same)})
+                if not same:
+                    raise SystemExit(f"lookup: batch of {q} keys on {name} differs from the point reads")
+            rows.append(row)
+        for s in dsegs:
+            s.release()
+        if drem is not None:
+            drem.release()
+    print(json.dumps({"config": "batched term lookup (ii2_lookup_dev, results downloaded)", "cards": card,
+                      "terms": a.terms, "postings": a.postings, "results": rows}))
 
 
 def c1(eng, a):
@@ -424,6 +482,8 @@ def main():
         c4(eng, a)
     if "prefix" in a.which:
         prefix(eng, a)
+    if "lookup" in a.which:
+        lookup(eng, a)
 
 
 if __name__ == "__main__":

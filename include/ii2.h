@@ -291,6 +291,39 @@ int ii2_prefix_search(const ii2_seg_view* segs, int nseg, const uint8_t* prefix_
                       const uint32_t* prefix_off, uint32_t nprefix, ii2_prefix_out* out);
 void ii2_prefix_out_free(ii2_prefix_out* out);
 
+/* ---- batched term lookup: InvertedIndex.Read(t, t) for many keys t in one call */
+typedef struct ii2_lookup_out {
+  uint64_t n_keys;
+  uint8_t* found;       /* n_keys: != 0 <=> Read(key, key) yields the term          */
+  uint32_t* post;       /* key i's list = post[post_off[i] .. post_off[i+1])        */
+  uint64_t* post_off;   /* n_keys + 1                                               */
+  uint64_t postings_in; /* Σ lengths of the source lists that were unioned          */
+  void* _owner;
+} ii2_lookup_out;
+
+/* Key i = key_bytes[key_off[i] .. key_off[i+1]); any order, duplicates and the
+ * empty key allowed.  For every key, found[i] and list i are exactly the term and
+ * list ii2_read_range_dev(segs, nseg, key, key, rem) returns:
+ *   - no segment holds the key: found = 0, empty list;
+ *   - one segment holds it: that list as stored (possibly unsorted, duplicates kept);
+ *   - two or more hold it: the sorted-unique union, even when some lists are empty;
+ *   - without rem a key held only with empty lists is found with an empty list;
+ *   - with rem the removed values are dropped after the union, and a key whose list
+ *     ends empty is not found.
+ * ii2_lookup_dev runs on the device of its handles (handles of two devices:
+ * II2_ERR_INVALID); ii2_lookup uploads the views to the device the thread selected.
+ * nkeys == 0 or nseg == 0 gives empty results.  Outputs are pinned host memory;
+ * free them with ii2_lookup_out_free.  II2_ERR_INVALID: NULL out, NULL data
+ * pointers, key_off not monotone.  II2_ERR_UNSUPPORTED: more than 1024 segments,
+ * a key longer than 65 535 bytes, one key's union of 2^32 postings or more. */
+int ii2_lookup_dev(ii2_seg* const* segs, int nseg, const uint8_t* key_bytes,
+                   const uint32_t* key_off, uint32_t nkeys, const ii2_removed* rem,
+                   ii2_lookup_out* out);
+int ii2_lookup(const ii2_seg_view* segs, int nseg, const uint8_t* key_bytes,
+               const uint32_t* key_off, uint32_t nkeys, const uint32_t* removed_sorted,
+               uint64_t nrem, ii2_lookup_out* out);
+void ii2_lookup_out_free(ii2_lookup_out* out);
+
 /* ---- cross-shard exchange: one process per GPU, contiguous shard-key ranges per
  *      rank (shardKey, shard.go:362-378), NCCL over NVLink --------------------
  * Compaction needs no exchange (shards never interact, shard.go:19-20).  Reads

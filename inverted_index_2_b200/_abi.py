@@ -99,6 +99,17 @@ class PrefixOut(C.Structure):
     ]
 
 
+class LookupOut(C.Structure):
+    _fields_ = [
+        ("n_keys", C.c_uint64),
+        ("found", u8p),
+        ("post", u32p),
+        ("post_off", u64p),
+        ("postings_in", C.c_uint64),
+        ("_owner", C.c_void_p),
+    ]
+
+
 class FstTerms(C.Structure):
     _fields_ = [
         ("n_terms", C.c_uint64),
@@ -183,6 +194,11 @@ PROTOTYPES = {
     "ii2_prefix_search": (C.c_int, [C.POINTER(SegView), C.c_int, u8p, u32p, C.c_uint32,
                                     C.POINTER(PrefixOut)]),
     "ii2_prefix_out_free": (None, [C.POINTER(PrefixOut)]),
+    "ii2_lookup_dev": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, u8p, u32p, C.c_uint32, C.c_void_p,
+                                 C.POINTER(LookupOut)]),
+    "ii2_lookup": (C.c_int, [C.POINTER(SegView), C.c_int, u8p, u32p, C.c_uint32, u32p, C.c_uint64,
+                             C.POINTER(LookupOut)]),
+    "ii2_lookup_out_free": (None, [C.POINTER(LookupOut)]),
     "ii2_comm_unique_id": (C.c_int, [u8p]),
     "ii2_comm_init": (C.c_int, [u8p, C.c_int, C.c_int]),
     "ii2_comm_info": (C.c_int, [C.POINTER(C.c_int), C.POINTER(C.c_int)]),

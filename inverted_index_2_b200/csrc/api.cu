@@ -9,6 +9,7 @@
 
 #include "codec.cuh"
 #include "ingest.cuh"
+#include "lookup.cuh"
 #include "prefix.cuh"
 #include "handles.cuh"
 #include "union.cuh"
@@ -992,6 +993,122 @@ void ii2_prefix_out_free(ii2_prefix_out* o) {
   memset(o, 0, sizeof(*o));
 }
 
+// ------------------------------------------------------------------ batched term lookup
+constexpr uint32_t kLookupMaxKey = 65535;  // bytes of one key
+
+static int lookup_impl(ii2_seg* const* segs, int nseg, const uint8_t* key_bytes,
+                       const uint32_t* key_off, uint32_t nkeys, const ii2_removed* rem,
+                       ii2_lookup_out* o, cudaStream_t s) {
+  ProfScope pipe_scope("lookup_total", s);
+  if (nseg > kMaxSegs) {
+    set_last_error("%d segments in one call (max %d per pass)", nseg, kMaxSegs);
+    return II2_ERR_UNSUPPORTED;
+  }
+  for (uint32_t i = 0; i < nkeys; i++) {
+    if (key_off[i + 1] < key_off[i]) return II2_ERR_INVALID;
+    if (key_off[i + 1] - key_off[i] > kLookupMaxKey) {
+      set_last_error("lookup: key %u is %u bytes long (max %u)", i, key_off[i + 1] - key_off[i],
+                     kLookupMaxKey);
+      return II2_ERR_UNSUPPORTED;
+    }
+  }
+  const size_t kbytes = nkeys ? key_off[nkeys] : 0;
+  if (kbytes && !key_bytes) return II2_ERR_INVALID;
+  uint64_t n_post = 0;
+  for (int i = 0; i < nseg; i++) {
+    if (!segs[i]) return II2_ERR_INVALID;
+    n_post += segs[i]->n_post;
+  }
+  std::unique_ptr<HostOwner> own(new HostOwner());
+  o->n_keys = nkeys;
+  if (nkeys == 0 || nseg == 0) {  // nothing to find
+    o->found = own->alloc<uint8_t>(nkeys);
+    o->post_off = own->alloc<uint64_t>((size_t)nkeys + 1);
+    o->post = own->alloc<uint32_t>(0);
+    if (!o->found || !o->post_off || !o->post) return II2_ERR_NOMEM;
+    memset(o->found, 0, nkeys);
+    memset(o->post_off, 0, ((size_t)nkeys + 1) * 8);
+    o->postings_in = 0;
+    o->_owner = own.release();
+    return II2_OK;
+  }
+  // segment table + key offsets + key bytes through one pinned block and one copy
+  const size_t off_bytes = ((size_t)nkeys + 1) * 4;
+  const size_t stage_bytes = sizeof(SegDesc) * nseg + off_bytes + kbytes + 64;
+  struct PinnedBlock {
+    void* p = nullptr;
+    ~PinnedBlock() { pinned_free(p); }
+  } stage;
+  stage.p = pinned_alloc(stage_bytes);
+  if (!stage.p) return II2_ERR_NOMEM;
+  SegDesc* h = static_cast<SegDesc*>(stage.p);
+  uint32_t* h_off = reinterpret_cast<uint32_t*>(h + nseg);
+  uint8_t* h_kb = reinterpret_cast<uint8_t*>(h_off + nkeys + 1);
+  for (int i = 0; i < nseg; i++) {
+    const ii2_seg* g = segs[i];
+    h[i].tb = g->tb.p;
+    h[i].toff = g->toff.p;
+    h[i].post = g->post.p;
+    h[i].poff = g->poff.p;
+    h[i].n = g->n_terms;
+    h[i].lo = 0;
+    h[i].hi = g->n_terms;
+    h[i].base = 0;
+  }
+  memcpy(h_off, key_off, off_bytes);
+  if (kbytes) memcpy(h_kb, key_bytes, kbytes);
+  DevBuf<uint8_t> d_stage;
+  II2_TRY(d_stage.alloc_scratch(stage_bytes, s, 32));
+  II2_CUDA_TRY(cudaMemcpyAsync(d_stage.p, stage.p, stage_bytes, cudaMemcpyHostToDevice, s));
+  const SegDesc* d_segs = reinterpret_cast<const SegDesc*>(d_stage.p);
+  const uint32_t* d_off = reinterpret_cast<const uint32_t*>(d_segs + nseg);
+  const uint8_t* d_kb = reinterpret_cast<const uint8_t*>(d_off + nkeys + 1);
+  RemovedSet rs;
+  if (rem) {
+    rs = rem->set();
+  } else {
+    rs.sorted = nullptr;
+    rs.n = 0;
+    rs.bitmap = nullptr;
+    rs.bitmap_bits = 0;
+  }
+  LookupOut lo;
+  // plain reads keep empty lists; with a removed set an emptied key is not found (as
+  // ii2_read_range_dev)
+  II2_TRY(k8_lookup(d_segs, nseg, n_post, d_kb, d_off, nkeys, rs, rem == nullptr, lo, s));
+  II2_TRY(d2h(&o->found, lo.found.p, nkeys, *own, s));
+  II2_TRY(d2h(&o->post_off, lo.post_off.p, (size_t)nkeys + 1, *own, s));
+  II2_TRY(d2h(&o->post, lo.post.p, (size_t)lo.total, *own, s));
+  II2_CUDA_TRY(cudaStreamSynchronize(s));
+  o->postings_in = lo.postings_in;
+  o->_owner = own.release();
+  return II2_OK;
+}
+
+int ii2_lookup_dev(ii2_seg* const* segs, int nseg, const uint8_t* key_bytes,
+                   const uint32_t* key_off, uint32_t nkeys, const ii2_removed* rem,
+                   ii2_lookup_out* out) {
+  if (!out || nseg < 0 || (nseg && !segs) || (nkeys && !key_off)) return II2_ERR_INVALID;
+  memset(out, 0, sizeof(*out));
+  int dev = -1;
+  II2_TRY(handles_device(segs, nseg, rem, &dev));
+  II2_TRY(ctx_require_device(dev));
+  cudaStream_t s = cur_stream();
+  const int rc = lookup_impl(segs, nseg, key_bytes, key_off, nkeys, rem, out, s);
+  if (rc != II2_OK) {
+    cudaStreamSynchronize(s);
+    memset(out, 0, sizeof(*out));
+  }
+  arena_reset(s);
+  return rc;
+}
+
+void ii2_lookup_out_free(ii2_lookup_out* o) {
+  if (!o) return;
+  delete static_cast<HostOwner*>(o->_owner);
+  memset(o, 0, sizeof(*o));
+}
+
 // ------------------------------------------------------------------ ingest batching
 static int ingest_impl(const ii2_doc_view* docs, int ndocs, const uint32_t* removed_sorted,
                        uint64_t nrem, uint32_t flags, ii2_merge_out* out, cudaStream_t s) {
@@ -1803,6 +1920,24 @@ int ii2_prefix_search(const ii2_seg_view* segs, int nseg, const uint8_t* prefix_
     list.v.push_back(g);
   }
   return ii2_prefix_search_dev(list.v.data(), nseg, prefix_bytes, prefix_off, nprefix, out);
+}
+
+int ii2_lookup(const ii2_seg_view* segs, int nseg, const uint8_t* key_bytes,
+               const uint32_t* key_off, uint32_t nkeys, const uint32_t* removed_sorted,
+               uint64_t nrem, ii2_lookup_out* out) {
+  if (!out || nseg < 0 || (nseg && !segs) || (nkeys && !key_off)) return II2_ERR_INVALID;
+  memset(out, 0, sizeof(*out));
+  II2_TRY(ctx_require());
+  SegList list;
+  for (int i = 0; i < nseg; i++) {
+    ii2_seg* g = nullptr;
+    II2_TRY(ii2_seg_upload(&segs[i], &g));
+    list.v.push_back(g);
+  }
+  ii2_removed* rem = nullptr;
+  if (removed_sorted) II2_TRY(ii2_removed_upload(removed_sorted, nrem, &rem));
+  std::unique_ptr<ii2_removed> rem_guard(rem);
+  return ii2_lookup_dev(list.v.data(), nseg, key_bytes, key_off, nkeys, rem, out);
 }
 
 }  // extern "C"

@@ -1101,197 +1101,7 @@ __global__ void __launch_bounds__(MW_WARPS * 32, MW_MIN_CTAS) k2_mwarp_kernel(co
 // whole-CTA intcomp encode, one write of the result.  The CTAs pull terms from the
 // list K2b filled (a device-side counter: no host synchronisation); output space comes from two
 // bump cursors over regions sized by the input postings.  Longer terms go on to the `huge`
-// list for the path below.
-constexpr int MED_V = 16;                 // values per lane of a warp-sorted run
-constexpr uint32_t MED_RUN = 32 * MED_V;  // 512
-// Word of s_o that holds gathered value e: runs of MED_RUN values, one pad word per 16.
-__device__ __forceinline__ uint32_t med_run_slot(uint32_t e) { return e + (e >> 4); }
-
-// The union of ONE term by a CTA of NW warps (k2_medium_kernel, api.cu's point read): c sources
-// (g_ptr[0 .. c), lengths as the prefix s_moff[0 .. c], L = s_moff[c] <= NW * 512 values) are
-// gathered into shared memory, sorted and deduped when c >= 2 (a single source passes through in
-// its own order, duplicates kept: survey Q4), filtered against the removed set and compacted.
-// Every thread of the CTA calls; returns the number of survivors, which end in s_v[0 .. outn).
-// s_v: NW * 512 words, s_o: NW * 512 * 17 / 16 words, s_cnt / s_last: NW words.
-template <int NW>
-__device__ __forceinline__ uint32_t cta_union_term(const uint64_t* __restrict__ g_ptr, uint32_t c,
-                                                   uint32_t L, const RemovedSet& rem, uint32_t* s_v,
-                                                   uint32_t* s_o, const uint32_t* s_moff,
-                                                   uint32_t* s_cnt, uint32_t* s_last) {
-  constexpr int MED_THREADS = NW * 32;
-  const uint32_t tid = threadIdx.x;
-  // ---- gather.  The term lands in s_o as runs of MED_RUN values (one per warp), every run
-  // padded (one word per 16) so that the blocked register load below is free of bank
-  // conflicts; the tail up to a power-of-two number of runs is the sentinel 0xFFFFFFFF.
-  const bool single = c == 1;  // passes through unsorted, duplicates kept (survey Q4)
-  const uint32_t w = warp_id(), lane = lane_id();
-  uint32_t nrun = 1;
-  while (nrun * MED_RUN < L) nrun <<= 1;
-  const uint32_t Lpad = nrun * MED_RUN;
-  // The source pointers wait in s_v (free until the first exchange) and every thread resolves
-  // eight elements before it stores any: eight value loads in flight instead of a chain of
-  // pointer load -> value load per element.
-  uint64_t* const s_ptr = reinterpret_cast<uint64_t*>(s_v);
-  const uint32_t* const src0 = reinterpret_cast<const uint32_t*>(g_ptr[0]);
-  if (!single) {
-    for (uint32_t i = tid; i < c; i += MED_THREADS) s_ptr[i] = g_ptr[i];
-    __syncthreads();
-  }
-  uint32_t top = 1;  // largest power of two below c
-  while (top * 2 < c) top <<= 1;
-  const bool by_source = !single && c * 8 <= L;  // sources of >= 8 values on average
-  if (by_source) {
-    // a warp per source, two sources (eight loads per lane) in flight; no search at all
-    for (uint32_t e = L + tid; e < Lpad; e += MED_THREADS) s_o[med_run_slot(e)] = 0xFFFFFFFFu;
-    for (uint32_t j0 = 2 * w; j0 < c; j0 += 2 * (MED_THREADS / 32)) {
-      uint32_t x[2][4], o2[2], n2[2];
-      const uint32_t* p2[2];
-#pragma unroll
-      for (int q = 0; q < 2; q++) {
-        const uint32_t j = j0 + q;
-        const bool in = j < c;
-        p2[q] = reinterpret_cast<const uint32_t*>(in ? s_ptr[j] : 0ull);
-        o2[q] = in ? s_moff[j] : 0u;
-        n2[q] = in ? s_moff[j + 1] - o2[q] : 0u;
-#pragma unroll
-        for (int t = 0; t < 4; t++) x[q][t] = t * 32 + lane < n2[q] ? __ldg(p2[q] + t * 32 + lane) : 0u;
-      }
-#pragma unroll
-      for (int q = 0; q < 2; q++) {
-#pragma unroll
-        for (int t = 0; t < 4; t++)
-          if (t * 32 + lane < n2[q]) s_o[med_run_slot(o2[q] + t * 32 + lane)] = x[q][t];
-        for (uint32_t i = 128 + lane; i < n2[q]; i += 32) s_o[med_run_slot(o2[q] + i)] = __ldg(p2[q] + i);
-      }
-    }
-  }
-  for (uint32_t e0 = tid; e0 < (by_source ? 0u : Lpad); e0 += 8 * MED_THREADS) {
-    uint32_t x[8];
-#pragma unroll
-    for (int q = 0; q < 8; q++) {
-      const uint32_t e = e0 + q * MED_THREADS;
-      x[q] = 0xFFFFFFFFu;
-      if (e < L) {
-        if (single) {
-          x[q] = __ldg(src0 + e);
-        } else {
-          uint32_t lo = 0;  // last source whose first element is <= e (empty sources skipped)
-          for (uint32_t st = top; st; st >>= 1) {
-            const uint32_t m = lo + st;
-            if (m < c && s_moff[m] <= e) lo = m;
-          }
-          x[q] = __ldg(reinterpret_cast<const uint32_t*>(s_ptr[lo]) + (e - s_moff[lo]));
-        }
-      }
-    }
-#pragma unroll
-    for (int q = 0; q < 8; q++) {
-      const uint32_t e = e0 + q * MED_THREADS;
-      if (e < Lpad) s_o[med_run_slot(e)] = x[q];
-    }
-  }
-  __syncthreads();
-  // ---- sort.  From here to the compaction the values live in registers: warp w holds run w,
-  // lane l its values 16 l .. 16 l + 15.  Each run is sorted by its warp (sort_warp_v<16>);
-  // then 1 / 2 / 3 bitonic merge levels double the sorted blocks up to Lpad.  A level starts
-  // with the stages whose partner sits in another warp — the flip (value e against the
-  // mirrored value of the partner run), then half-cleaners at warp distances — exchanged
-  // through shared memory in a transposed, conflict-free layout, alternating between the two
-  // buffers so that one barrier per stage is enough; the rest of the level is shuffles and
-  // register compare-exchanges (clean_warp_v).
-  const bool active = w < nrun;
-  uint32_t v[MED_V];
-#pragma unroll
-  for (int r = 0; r < MED_V; r++)
-    v[r] = active ? s_o[med_run_slot(w * MED_RUN + lane * MED_V + r)] : 0xFFFFFFFFu;
-  if (!single) {
-    {
-      const uint32_t at = w * MED_RUN, n = L > at ? min(L - at, MED_RUN) : 0u;
-      if (n > 1) sort_warp_v<MED_V>(v, lane, n);
-    }
-    uint32_t stage = 0;
-    for (uint32_t nw = 2; nw <= nrun; nw <<= 1) {  // warps per sorted block after this level
-      for (uint32_t dw = nw; dw >= 2; dw >>= 1) {  // dw == nw: the flip; below: half-cleaners
-        const bool flip = dw == nw;
-        uint32_t* const X = (stage++ & 1u) ? s_o : s_v;
-        if (active) {
-#pragma unroll
-          for (int r = 0; r < MED_V; r++) X[w * MED_RUN + r * 32 + lane] = v[r];
-        }
-        __syncthreads();
-        if (active) {
-          const uint32_t pw = flip ? (w ^ (nw - 1)) : (w ^ (dw >> 1));
-          const bool lower = (w & (dw >> 1)) == 0;
-          const uint32_t* const P = X + pw * MED_RUN;
-#pragma unroll
-          for (int r = 0; r < MED_V; r++) {
-            const uint32_t o = flip ? P[(MED_V - 1 - r) * 32 + (31 - lane)] : P[r * 32 + lane];
-            v[r] = ((v[r] < o) == lower) ? v[r] : o;
-          }
-        }
-      }
-      if (active) clean_warp_v<MED_V>(v, lane);
-    }
-  }
-  // ---- dedup + removed filter + compaction, still from the registers: sixteen membership
-  // probes per lane issued eight at a time, keep flags in a register, positions from one warp
-  // scan + the warps' totals; the survivors end in s_v.
-  uint32_t outn;
-  {
-    if (lane == 31) s_last[w] = v[MED_V - 1];
-    __syncthreads();  // (also: every partner has read the last exchange buffer)
-    const uint32_t e_l = w * MED_RUN + lane * MED_V;  // index of v[0]
-    uint32_t keep = 0;
-    if (rem.bitmap) {
-      const uint32_t nbits = (uint32_t)rem.bitmap_bits;
-#pragma unroll
-      for (int r0 = 0; r0 < MED_V; r0 += 8) {
-        uint32_t word[8];
-#pragma unroll
-        for (int r = 0; r < 8; r++) {
-          const bool probe = e_l + r0 + r < L && v[r0 + r] < nbits;
-          word[r] = probe ? __ldg(rem.bitmap + (v[r0 + r] >> 5)) : 0u;
-        }
-#pragma unroll
-        for (int r = 0; r < 8; r++)
-          keep |= (e_l + r0 + r < L && !((word[r] >> (v[r0 + r] & 31u)) & 1u)) ? 1u << (r0 + r) : 0u;
-      }
-    } else {
-#pragma unroll
-      for (int r = 0; r < MED_V; r++)
-        if (e_l + r < L && !(rem.n && is_removed_call(rem.sorted, rem.n, v[r]))) keep |= 1u << r;
-    }
-    uint32_t up = __shfl_up_sync(0xffffffffu, v[MED_V - 1], 1);  // the value before v[0]
-    if (lane == 0 && w > 0) up = s_last[w - 1];
-    if (!single) {
-      if (e_l > 0 && up == v[0]) keep &= ~1u;
-#pragma unroll
-      for (int r = 1; r < MED_V; r++)
-        if (v[r] == v[r - 1]) keep &= ~(1u << r);
-    }
-    const uint32_t cnt = __popc(keep);
-    const uint32_t inc = warp_inclusive_scan(cnt);
-    if (lane == 31) s_cnt[w] = inc;
-    __syncthreads();
-    uint32_t at = inc - cnt, tot = 0;
-#pragma unroll
-    for (int q = 0; q < MED_THREADS / 32; q++) {
-      const uint32_t cq = s_cnt[q];
-      at += (uint32_t)q < w ? cq : 0u;
-      tot += cq;
-    }
-    outn = tot;
-    uint32_t* dst = s_v + at;
-#pragma unroll
-    for (int r = 0; r < MED_V; r++) {
-      const bool k = (keep >> r) & 1u;
-      if (k) *dst = v[r];
-      dst += k ? 1 : 0;
-    }
-  }
-  __syncthreads();
-  return outn;
-}
+// list for the path below.  The union itself is cta_union_term (union_dev.cuh).
 
 struct MedArgs {
   const uint32_t* n_large;       // terms K2b deferred

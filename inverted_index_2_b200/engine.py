@@ -411,6 +411,47 @@ class Engine:
                     "prefix_search_dev")
         return self._prefix_result(prefixes, out)
 
+    # ---- batched term lookup: Read(t, t) for many keys at once --------------------------
+    def _lookup_result(self, out: A.LookupOut) -> list[np.ndarray | None]:
+        try:
+            n = int(out.n_keys)
+            found = A.from_ptr(out.found, n, np.uint8)
+            off = A.from_ptr(out.post_off, n + 1, np.uint64)
+            post = A.from_ptr(out.post, int(off[-1]) if n else 0, np.uint32)
+        finally:
+            self.lib.ii2_lookup_out_free(C.byref(out))
+        return [post[int(off[i]):int(off[i + 1])] if found[i] else None for i in range(n)]
+
+    def lookup(self, segs: list[FlatSegment], keys: list[bytes], removed=None
+               ) -> list[np.ndarray | None]:
+        """Read(key, key) for every key over host views: the key's list, or None if no term is
+        found (aligned with `keys`)."""
+        arr = views_array(segs)
+        blob, off = self._prefix_args(keys)
+        if removed is None:
+            rp, nr, keep = C.cast(None, A.u32p), 0, None
+        else:
+            keep = np.ascontiguousarray(removed, dtype=np.uint32)
+            nr = len(keep)
+            if nr == 0:
+                keep = np.zeros(1, dtype=np.uint32)
+            rp = A.np_ptr(keep, A.u32p)
+        out = A.LookupOut()
+        self._check(self.lib.ii2_lookup(arr, len(segs), A.np_ptr(blob, A.u8p), A.np_ptr(off, A.u32p),
+                                        len(keys), rp, nr, C.byref(out)), "lookup")
+        return self._lookup_result(out)
+
+    def lookup_dev(self, segs: list[DeviceSegment], keys: list[bytes],
+                   removed: DeviceRemoved | None = None) -> list[np.ndarray | None]:
+        """Read(key, key) for every key over resident segments, in one call on their device."""
+        blob, off = self._prefix_args(keys)
+        out = A.LookupOut()
+        self._check(self.lib.ii2_lookup_dev(self._handles(segs), len(segs), A.np_ptr(blob, A.u8p),
+                                            A.np_ptr(off, A.u32p), len(keys),
+                                            removed.h if removed else None, C.byref(out)),
+                    "lookup_dev")
+        return self._lookup_result(out)
+
     # ---- codec -----------------------------------------------------------------------
     def intcomp_encode_batch(self, post: np.ndarray, post_off: np.ndarray):
         post = np.ascontiguousarray(post, dtype=np.uint32)
