@@ -28,9 +28,6 @@ def _newer(srcs, target):
 
 def build(force: bool = False, verbose: bool = False) -> str:
     nvcc = os.environ.get("NVCC", "nvcc")
-    # tuning sweeps on the GPU box: II2_NVCC_EXTRA="-DK2B_MIN_CTAS=5" rebuilds with extra flags
-    extra = os.environ.get("II2_NVCC_EXTRA", "").split()
-    force = force or bool(extra)
     if not os.path.isdir(CSRC):
         if os.path.exists(OUT):
             return OUT
@@ -44,7 +41,7 @@ def build(force: bool = False, verbose: bool = False) -> str:
     def compile_one(src):
         obj = os.path.join(objdir, os.path.splitext(os.path.basename(src))[0] + ".o")
         if force or _newer([src] + hdrs, obj):
-            cmd = [nvcc] + NVCC_FLAGS + extra + ["-c", src, "-o", obj]
+            cmd = [nvcc] + NVCC_FLAGS + ["-c", src, "-o", obj]
             if verbose:
                 print(" ".join(cmd), file=sys.stderr)
             subprocess.check_call(cmd)

@@ -134,7 +134,7 @@ k_val_woff(const ValSlice* __restrict__ sl, uint32_t nslices, uint64_t* __restri
 // device address space by unified addressing) into device blocks with plain loads over the
 // bus.  One launch per term range replaces hundreds of copy-engine requests (measured ~7 us
 // of engine time each, more than the small slices take to transfer).
-// Reads over the bus are fastest as whole aligned lines (scratch/h2d_micro.cu on B200: 51.5 GB/s
+// Reads over the bus are fastest as whole aligned lines (scripts/h2d_micro.cu on B200: 51.5 GB/s
 // from a 512-byte aligned source, 46.9 .. 49.6 GB/s at other phases), and a slice starts anywhere
 // in its host array.  So a job is laid out over the 512-byte aligned ENVELOPE of its source
 // range: vector v of the job is the 16 bytes at (src rounded down to 512) + 16 v, a warp reads
@@ -1341,10 +1341,9 @@ static int merge_pipelined(const ii2_seg_view* segs, int nseg, const uint32_t* r
   // The ranges are equal except the last two: what follows the last upload (its merge and the
   // download of its result) is the only part of the call the bus does not cover, so the last
   // range is small; 0.65 and 0.4 of a full range keep every range's merge + download shorter
-  // than the next range's upload.  II2_MERGE_TAPER=0 turns it off (tuning).
+  // than the next range's upload (measured on B200, C2: 30.1 instead of 30.5 ms per call).
   std::vector<double> cum(P + 1, 0.0);
-  const char* env_taper = getenv("II2_MERGE_TAPER");
-  const bool taper = P >= 4 && segs[big].n_terms >= 64ull * P && !(env_taper && atoi(env_taper) == 0);
+  const bool taper = P >= 4 && segs[big].n_terms >= 64ull * P;
   for (int p = 0; p < P; p++)
     cum[p + 1] = cum[p] + (taper && p == P - 2 ? 0.65 : (taper && p == P - 1 ? 0.4 : 1.0));
   for (int p = 1; p < P; p++) {
@@ -1377,7 +1376,9 @@ static int merge_pipelined(const ii2_seg_view* segs, int nseg, const uint32_t* r
   std::vector<std::unique_ptr<SegList>> parts(P);
   std::vector<std::unique_ptr<ii2_result>> results(P);
   // Are the caller's arrays pinned and visible to the device (unified addressing)?  Then a
-  // kernel gathers them (k_gather_host); pageable arrays go through the copy engines.
+  // kernel gathers them (k_gather_host); pageable arrays go through the copy engine.  (A
+  // copy-engine request per slice was measured slower on pinned inputs too, on B200: 36.8 vs
+  // 31.1 ms per C2 call, on one to four streams — the fixed cost of a request does not overlap.)
   struct DevAlias {
     const uint8_t* tb;
     const uint8_t* toff;
@@ -1391,26 +1392,7 @@ static int merge_pipelined(const ii2_seg_view* segs, int nseg, const uint32_t* r
     return v.val_woff32 ? 4ull * v.val_woff32[t] : v.val_off[t];
   };
   std::vector<DevAlias> alias(nseg);
-  // II2_MERGE_UPLOAD picks how the slices cross the bus (tuning; results are the same):
-  //   gather  one kernel per range reads every slice from pinned host memory
-  //   dma<k>  every slice is a copy-engine request, round-robin over k streams (1..4) so the
-  //           fixed cost of a request overlaps the transfer of another
-  //   hybrid<k>  term bytes and postings (the large slices) by copy engine on k streams, the
-  //           offset arrays by the gather kernel, both at once
-  bool gather = getenv("II2_MERGE_NO_GATHER") == nullptr;
-  int dma_streams = 0;       // 0: copies (if any) go to sA itself
-  bool dma_large = false;    // hybrid: copy engines for term bytes and postings only
-  if (const char* m = getenv("II2_MERGE_UPLOAD")) {
-    if (!strncmp(m, "dma", 3)) {
-      gather = false;
-      dma_streams = m[3] ? atoi(m + 3) : 0;
-    } else if (!strncmp(m, "hybrid", 6)) {
-      dma_large = true;
-      dma_streams = m[6] ? atoi(m + 6) : 1;
-    }
-    if (dma_streams < 0 || dma_streams > 4) dma_streams = 4;
-    if (dma_large && dma_streams < 1) dma_streams = 1;
-  }
+  bool gather = true;
   auto dev_alias = [&](const void* hp, size_t align, const uint8_t** out_p) {
     *out_p = nullptr;
     if (!hp) return;  // empty array: nothing to read
@@ -1444,15 +1426,6 @@ static int merge_pipelined(const ii2_seg_view* segs, int nseg, const uint32_t* r
     }
   }
 
-  if (!gather) dma_large = false;  // hybrid needs the device aliases of the offset arrays
-  EventList fork_join;             // [0] = fork (allocations done), [1 + k] = join of copy stream k
-  if (dma_streams) {
-    for (int k = 0; k < 1 + dma_streams; k++) {
-      cudaEvent_t e;
-      II2_CUDA_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-      fork_join.v.push_back(e);
-    }
-  }
   // Stage the slices of range p: four allocations and one check launch for all segments (an
   // allocation + a kernel per slice would cost more host time than the copies take).  Offsets
   // stay absolute: the slice's base pointers are moved back by its first offset instead.  Every
@@ -1519,12 +1492,6 @@ static int merge_pipelined(const ii2_seg_view* segs, int nseg, const uint32_t* r
     size_t at_val = 0, at_voff = 0;
     uint64_t run_lists = 0, run_words = 0;
     if (gather) II2_TRY(L.blk_job.alloc(4 * nx, sA));
-    if (dma_streams) {  // the blocks are stream-ordered allocations of sA
-      II2_CUDA_TRY(cudaEventRecord(fork_join.v[0], sA));
-      for (int k = 0; k < dma_streams; k++)
-        II2_CUDA_TRY(cudaStreamWaitEvent(copy_stream(k), fork_join.v[0], 0));
-    }
-    int rr = 0;
     SliceRef* refs = reinterpret_cast<SliceRef*>(h_tab + (ref_bytes + job_bytes) * p);
     GatherJob* jobs = reinterpret_cast<GatherJob*>(h_tab + (ref_bytes + job_bytes) * p + ref_bytes);
     uint32_t njobs = 0;
@@ -1538,17 +1505,16 @@ static int merge_pipelined(const ii2_seg_view* segs, int nseg, const uint32_t* r
     // alignment of the caller's pointer (a Go sub-slice or an mmap offset may start anywhere;
     // the key loads need a 4-byte aligned term base).
     auto place = [&](uint8_t* blk, size_t& cursor, const void* hsrc, const uint8_t* dsrc,
-                     uint64_t bytes, uint64_t first, bool large, uint8_t** dst_out) -> int {
-      const bool by_kernel = gather && !(dma_large && large);
-      const uint8_t* src = by_kernel ? dsrc : static_cast<const uint8_t*>(hsrc);
+                     uint64_t bytes, uint64_t first, uint8_t** dst_out) -> int {
+      const uint8_t* src = gather ? dsrc : static_cast<const uint8_t*>(hsrc);
       cursor = ((cursor + kGatherAlign - 1) & ~(size_t)(kGatherAlign - 1)) +
-               (by_kernel ? (reinterpret_cast<uintptr_t>(src) & (kGatherAlign - 1))
-                          : (size_t)(first & (kGatherAlign - 1)));
+               (gather ? (reinterpret_cast<uintptr_t>(src) & (kGatherAlign - 1))
+                       : (size_t)(first & (kGatherAlign - 1)));
       uint8_t* dst = blk + cursor;
       *dst_out = dst;
       cursor += bytes;
       if (!bytes) return II2_OK;
-      if (by_kernel) {
+      if (gather) {
         GatherJob& g = jobs[njobs++];
         g.src = src;
         g.dst = dst;
@@ -1556,8 +1522,7 @@ static int merge_pipelined(const ii2_seg_view* segs, int nseg, const uint32_t* r
         g.vec0 = nvec;
         nvec += gather_job_vectors(src, bytes);
       } else {
-        cudaStream_t sc = dma_streams ? copy_stream(rr++ % dma_streams) : sA;
-        II2_CUDA_TRY(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, sc));
+        II2_CUDA_TRY(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, sA));
       }
       return II2_OK;
     };
@@ -1569,10 +1534,10 @@ static int merge_pipelined(const ii2_seg_view* segs, int nseg, const uint32_t* r
       if (tlen && !v.term_bytes) return II2_ERR_INVALID;
       uint8_t *d_tb, *d_toff, *d_post = nullptr, *d_poff = nullptr;
       II2_TRY(place(L.blk_tb.p, at_tb, v.term_bytes ? v.term_bytes + tfirst : nullptr,
-                    alias[i].tb ? alias[i].tb + tfirst : nullptr, tlen, tfirst, true, &d_tb));
+                    alias[i].tb ? alias[i].tb + tfirst : nullptr, tlen, tfirst, &d_tb));
       at_tb += 32;  // key loads read past the last term
       II2_TRY(place(reinterpret_cast<uint8_t*>(L.blk_toff.p), at_toff, v.term_off + lo[i],
-                    alias[i].toff + 4 * lo[i], (n + 1) * 4, 4 * lo[i], false, &d_toff));
+                    alias[i].toff + 4 * lo[i], (n + 1) * 4, 4 * lo[i], &d_toff));
       std::unique_ptr<ii2_seg> g(new ii2_seg());
       g->n_terms = (uint32_t)n;
       g->term_bytes_len = tlen;
@@ -1589,12 +1554,12 @@ static int merge_pipelined(const ii2_seg_view* segs, int nseg, const uint32_t* r
         const uint64_t b0 = val_at(v, lo[i]), b1 = val_at(v, hi[i]);
         uint8_t *d_val, *d_vo;
         II2_TRY(place(reinterpret_cast<uint8_t*>(L.blk_val.p), at_val, v.val_bytes + b0,
-                      alias[i].post ? alias[i].post + b0 : nullptr, b1 - b0, b0, true, &d_val));
+                      alias[i].post ? alias[i].post + b0 : nullptr, b1 - b0, b0, &d_val));
         const bool w32 = v.val_woff32 != nullptr;
         const size_t esz = w32 ? 4 : 8;
         II2_TRY(place(L.blk_voff.p, at_voff,
                       w32 ? static_cast<const void*>(v.val_woff32 + lo[i]) : static_cast<const void*>(v.val_off + lo[i]),
-                      alias[i].poff ? alias[i].poff + esz * lo[i] : nullptr, n * esz, esz * lo[i], false, &d_vo));
+                      alias[i].poff ? alias[i].poff + esz * lo[i] : nullptr, n * esz, esz * lo[i], &d_vo));
         ValSlice vs;
         vs.src = reinterpret_cast<const uint32_t*>(d_val);
         vs.off = d_vo;
@@ -1614,9 +1579,9 @@ static int merge_pipelined(const ii2_seg_view* segs, int nseg, const uint32_t* r
         const uint64_t pfirst = v.post_off[lo[i]], plen = v.post_off[hi[i]] - pfirst;
         if (plen && !v.post) return II2_ERR_INVALID;
         II2_TRY(place(reinterpret_cast<uint8_t*>(L.blk_post.p), at_post, v.post ? v.post + pfirst : nullptr,
-                      alias[i].post ? alias[i].post + 4 * pfirst : nullptr, plen * 4, 4 * pfirst, true, &d_post));
+                      alias[i].post ? alias[i].post + 4 * pfirst : nullptr, plen * 4, 4 * pfirst, &d_post));
         II2_TRY(place(reinterpret_cast<uint8_t*>(L.blk_poff.p), at_poff, v.post_off + lo[i],
-                      alias[i].poff + 8 * lo[i], (n + 1) * 8, 8 * lo[i], false, &d_poff));
+                      alias[i].poff + 8 * lo[i], (n + 1) * 8, 8 * lo[i], &d_poff));
         g->n_post = plen;
         g->post.p = reinterpret_cast<uint32_t*>(d_post) - pfirst;
         g->poff.p = reinterpret_cast<uint64_t*>(d_poff);
@@ -1631,17 +1596,12 @@ static int merge_pipelined(const ii2_seg_view* segs, int nseg, const uint32_t* r
     II2_TRY(small_copy(L.blk_ref.p, refs, sizeof(SliceRef) * nx, sA));
     if (gather && njobs) {
       II2_TRY(small_copy(L.blk_job.p, jobs, sizeof(GatherJob) * njobs, sA));
-      // II2_GATHER_GRID=<n>: CTAs of the staging kernel (tuning; it shares the SMs with the merge)
-      const char* env_grid = getenv("II2_GATHER_GRID");
-      const uint64_t max_grid = env_grid && atoi(env_grid) > 0 ? (uint64_t)atoi(env_grid) : 64;
+      // at most 64 CTAs: the staging kernel shares the SMs with the merge (32 and 128 were
+      // measured no faster)
       const unsigned grid = (unsigned)std::min<uint64_t>(
-          max_grid, std::max<uint64_t>(1, div_up(nvec, (uint64_t)kGatherThreads * kGatherUnroll)));
+          64, std::max<uint64_t>(1, div_up(nvec, (uint64_t)kGatherThreads * kGatherUnroll)));
       k_gather_host<<<grid, kGatherThreads, 0, sA>>>(L.blk_job.p, njobs, nvec);
       II2_LAUNCHED();
-    }
-    for (int k = 0; k < dma_streams; k++) {  // join: the check and the merge read every slice
-      II2_CUDA_TRY(cudaEventRecord(fork_join.v[1 + k], copy_stream(k)));
-      II2_CUDA_TRY(cudaStreamWaitEvent(sA, fork_join.v[1 + k], 0));
     }
     if (max_n) {
       const dim3 grid(std::min<unsigned>(div_up(max_n, 256), 64u), (unsigned)nseg);
@@ -1880,8 +1840,6 @@ int ii2_merge(const ii2_seg_view* segs, int nseg, const uint32_t* removed_sorted
   if (rc != II2_OK) {
     cudaStreamSynchronize(cur_stream());
     cudaStreamSynchronize(aux_stream());
-    if (getenv("II2_MERGE_UPLOAD"))
-      for (int k = 0; k < 4; k++) cudaStreamSynchronize(copy_stream(k));
     memset(out, 0, sizeof(*out));
   }
   return rc;

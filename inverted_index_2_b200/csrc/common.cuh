@@ -46,8 +46,7 @@ void set_last_error(const char* fmt, ...);
 // CTAs become resident while the previous kernel still runs, `griddepcontrol.wait` holds them
 // until that kernel has completed and its writes are visible, so only the gap disappears —
 // ordering and visibility are those of a plain stream.  A kernel WITHOUT pdl_enter() must never
-// be launched this way (it would run next to its producer).  II2_PDL=0 launches plainly.
-bool pdl_enabled();
+// be launched this way (it would run next to its producer).
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_chain(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem,
                                 cudaStream_t s, Args&&... args) {
@@ -60,7 +59,7 @@ inline cudaError_t launch_chain(void (*kern)(KArgs...), dim3 grid, dim3 block, s
   at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   at[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = at;
-  cfg.numAttrs = pdl_enabled() ? 1u : 0u;
+  cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
 }
 #define II2_LAUNCH_CHAIN(kern, grid, block, smem, s, ...)                                  \

@@ -29,18 +29,10 @@
 
 namespace ii2 {
 
-#ifndef K12F_THREADS_N
-#define K12F_THREADS_N 512
-#endif
-#ifndef K12F_MIN_CTAS
-#define K12F_MIN_CTAS 2
-#endif
-constexpr int F_THREADS = K12F_THREADS_N;
+constexpr int F_THREADS = 512;
+constexpr int F_MIN_CTAS = 2;
 constexpr int F_WARPS = F_THREADS / 32;
-#ifndef K12F_CAP_N
-#define K12F_CAP_N 1024
-#endif
-constexpr uint32_t F_CAP_I = K12F_CAP_N;         // instances of a bucket
+constexpr uint32_t F_CAP_I = 1024;               // instances of a bucket
 constexpr int F_PER = (F_CAP_I + F_THREADS - 1) / F_THREADS;  // instances per thread
 constexpr uint32_t F_HT = F_CAP_I > 512 ? 2048 : 1024;  // hash slots (a power of two >= 2 * F_CAP_I)
 constexpr uint32_t F_A_CH = F_CAP_I * 5 / 4;     // 16-byte chunks: staged term + posting offsets
@@ -108,7 +100,7 @@ __device__ __forceinline__ void smem_key16_at(const uint8_t* smem, uint32_t t0, 
   }
 }
 
-__global__ void __launch_bounds__(F_THREADS, K12F_MIN_CTAS) k12f_bucket_kernel(const K12fArgs a) {
+__global__ void __launch_bounds__(F_THREADS, F_MIN_CTAS) k12f_bucket_kernel(const K12fArgs a) {
   pdl_enter();
   extern __shared__ __align__(16) uint8_t smem[];
   __shared__ uint64_t s_p1[8], s_p2[8];

@@ -33,15 +33,10 @@
 
 namespace ii2 {
 
-#ifndef K1B_THREADS_N
-#define K1B_THREADS_N 256
-#endif
-constexpr int K1B_THREADS = K1B_THREADS_N;  // a tile holds CAP_I instances: CAP_I / K1B_THREADS per thread
+constexpr int K1B_THREADS = 256;  // a tile holds CAP_I instances: CAP_I / K1B_THREADS per thread
 constexpr int K1B_WARPS = K1B_THREADS / 32;
-#ifndef K1B_CAP_N
-#define K1B_CAP_N 1024  // 512 needs k <= 512 (a tile holds at least one instance of every segment)
-#endif
-constexpr uint32_t CAP_I = K1B_CAP_N;   // instances per sub-tile
+// instances per sub-tile (512 would need k <= 512: a tile holds at least one instance of every segment)
+constexpr uint32_t CAP_I = 1024;
 constexpr uint32_t K1B_HT = CAP_I > 512 ? 2048 : 1024;  // hash slots (a power of two >= 2 * CAP_I)
 static_assert(CAP_I % K1B_THREADS == 0 && CAP_I <= 1024 && CAP_I % 4 == 0,
               "tile = a whole number of instances per thread, 10-bit tile indexes");
@@ -99,30 +94,11 @@ __host__ __device__ inline size_t k1b_smem_bytes(int k) {
          + (size_t)CAP_I * 4 * 3                 // inst, count|length, pbase
          + (size_t)(4 * k) * 4 + (size_t)(2 * k + 2) * 4   // cur, mm, hi, endr; rstart (padded to 2^n + 1)
          + (size_t)CAP_I * 2 * 2                 // tlen, reps
-#ifndef K1B_SEG_GLOBAL
          + (size_t)k * 40 + 16                   // tb, toff, poff, post pointers; base - lo
-#endif
          + (size_t)K1B_HT * 4 + 64;
 }
 
-#ifndef K1B_MIN_CTAS
-#define K1B_MIN_CTAS 4
-#endif
-// -DK1B_TIMING: warp 0 of every CTA adds the clock ticks it spent in each phase of a tile to
-// g_k1b_clk (read back with ii2_debug_k1b_clocks); profiling builds only.
-#ifdef K1B_TIMING
-__device__ unsigned long long g_k1b_clk[10];
-#define K1B_TICK(slot)                                        \
-  do {                                                        \
-    if (tid == 0) {                                           \
-      const long long now_ = clock64();                       \
-      atomicAdd(&g_k1b_clk[slot], (unsigned long long)(now_ - tick_)); \
-      tick_ = now_;                                           \
-    }                                                         \
-  } while (0)
-#else
-#define K1B_TICK(slot) do { } while (0)
-#endif
+constexpr int K1B_MIN_CTAS = 4;
 // LIST: the CTA's bucket comes from a.list (the buckets the fused kernel deferred) — a separate
 // instantiation, because one more live pointer in the default one costs spills (64 registers).
 template <bool LIST>
@@ -154,7 +130,6 @@ __global__ void __launch_bounds__(K1B_THREADS, K1B_MIN_CTAS) k1b_group_kernel(co
   uint32_t* endr = reinterpret_cast<uint32_t*>(sp); sp += k * 4;
   // run starts inside the tile, padded with `size` up to kp2 = the power of two >= k
   uint32_t* rstart = reinterpret_cast<uint32_t*>(sp);
-#ifndef K1B_SEG_GLOBAL
   // the segment descriptors of the call, one field per array: phase (2) indexes them by run
   sp += (2 * k + 2) * 4;
   sp += (8 - (reinterpret_cast<uintptr_t>(sp) & 7)) & 7;
@@ -163,7 +138,6 @@ __global__ void __launch_bounds__(K1B_THREADS, K1B_MIN_CTAS) k1b_group_kernel(co
   const uint64_t** sg_poff = reinterpret_cast<const uint64_t**>(sp); sp += k * 8;
   const uint32_t** sg_post = reinterpret_cast<const uint32_t**>(sp); sp += k * 8;
   uint32_t* sg_bl = reinterpret_cast<uint32_t*>(sp);  // base - lo
-#endif
   // alias, valid once the hash table is done: first source slot by representative
   uint32_t* sbase = table;
   uint32_t kp2 = 1;
@@ -171,9 +145,6 @@ __global__ void __launch_bounds__(K1B_THREADS, K1B_MIN_CTAS) k1b_group_kernel(co
 
   const uint32_t tid = threadIdx.x;
   const unsigned lane = lane_id(), warp = warp_id();
-#ifdef K1B_TIMING
-  long long tick_ = clock64();
-#endif
   const uint32_t b = LIST ? a.list[blockIdx.x] : a.bucket0 + blockIdx.x;
   uint32_t W = (uint32_t)(a.bk_pos[b + 1] - a.bk_pos[b]);
   if (W == 0) {
@@ -185,37 +156,19 @@ __global__ void __launch_bounds__(K1B_THREADS, K1B_MIN_CTAS) k1b_group_kernel(co
     for (int s = tid; s < k; s += K1B_THREADS) {
       cur[s] = a.part[(uint64_t)r0 * k + s];
       endr[s] = a.part[(uint64_t)r1 * k + s];
-#ifndef K1B_SEG_GLOBAL
       const SegDesc sd = a.segs[s];
       sg_tb[s] = sd.tb;
       sg_toff[s] = sd.toff;
       sg_poff[s] = sd.poff;
       sg_post[s] = sd.post;
       sg_bl[s] = sd.base - sd.lo;
-#ifndef K1B_NO_PREFETCH_OFFS
       // the offsets of the run are read in phase (2), a few thousand clocks from here
       asm volatile("prefetch.global.L2 [%0];" ::"l"(sd.toff + cur[s]));
       asm volatile("prefetch.global.L2 [%0];" ::"l"(sd.poff + cur[s]));
       if (endr[s] - cur[s] > 12) asm volatile("prefetch.global.L2 [%0];" ::"l"(sd.poff + endr[s]));
-#endif
-#ifdef K1B_PREFETCH_RUNS
-      // With the plan's boundary tables the term bytes and postings of the run are known NOW, two
-      // dependent round trips before their addresses arrive through the offsets.  Measured
-      // (profiles/r02_experiments.md section 2): 1.30 ms instead of the per-instance prefetches
-      // below (1.23 ms), 1.45 ms with both - the extra live values cost spills at 64 registers.
-      if (endr[s] > cur[s]) {
-        const uint64_t r0s = (uint64_t)r0 * k + s, r1s = (uint64_t)r1 * k + s;
-        const uint32_t t0 = a.btb[r0s], t1 = a.btb[r1s];
-        const uint64_t p0 = a.bpo[r0s], p1 = a.bpo[r1s];
-        const char* tp = reinterpret_cast<const char*>(sd.tb) + t0;
-        const char* pp = reinterpret_cast<const char*>(sd.post + p0);
-        const uint32_t tbytes = min(t1 - t0, 512u);
-        const uint32_t pbytes = (uint32_t)min((p1 - p0) * 4, (uint64_t)512);
-        for (uint32_t o = 0; o < tbytes; o += 128) asm volatile("prefetch.global.L2 [%0];" ::"l"(tp + o));
-        for (uint32_t o = 0; o < pbytes; o += 128) asm volatile("prefetch.global.L2 [%0];" ::"l"(pp + o));
-      }
-#endif
-#endif
+      // (prefetching the run's term bytes and postings here, from the plan's boundary tables,
+      // was measured slower than the per-instance prefetches of phase (2): 1.30 vs 1.23 ms, and
+      // 1.45 ms with both - the extra live values cost spills at 64 registers)
     }
   }
   const uint64_t rec_base = a.bk_pos[b];
@@ -226,7 +179,6 @@ __global__ void __launch_bounds__(K1B_THREADS, K1B_MIN_CTAS) k1b_group_kernel(co
   uint32_t pcount = 0;   // postings of light terms so far
   uint32_t ecount = 0;   // staging words so far
   __syncthreads();
-  K1B_TICK(0);  // bucket header: part rows, prefix loads
 
   while (W > 0) {
     // ---------------- choose the sub-tile [cur, mmp) ----------------
@@ -274,14 +226,10 @@ __global__ void __launch_bounds__(K1B_THREADS, K1B_MIN_CTAS) k1b_group_kernel(co
       __syncthreads();
     }
 
-    K1B_TICK(1);  // tile choice (bisection of oversized buckets)
     // ---------------- (1) run starts; reset of the tile state ----------------
-#ifndef K1B_RSTART_ALL
     if (k <= 128 && warp != 0) {
       // warp 0 scans; the barrier after the resets below publishes the run starts
-    } else
-#endif
-    if (k <= 128) {  // every warp scans for itself (identical values): no warp waits for another
+    } else if (k <= 128) {
       uint32_t v[4], sum = 0;
 #pragma unroll
       for (int j = 0; j < 4; j++) {
@@ -316,7 +264,6 @@ __global__ void __launch_bounds__(K1B_THREADS, K1B_MIN_CTAS) k1b_group_kernel(co
     if (tid == 0) s_nreps = 0;
     __syncthreads();
 
-    K1B_TICK(2);  // run starts, resets
     // bytes past the 24-byte window, only needed for terms longer than cpl+24
     auto tail_compare = [&](uint32_t x, uint32_t y) -> int {
       const uint32_t skip = cpl + 24;
@@ -349,20 +296,9 @@ __global__ void __launch_bounds__(K1B_THREADS, K1B_MIN_CTAS) k1b_group_kernel(co
         const uint32_t i = tid + j * K1B_THREADS;
         sg[j] = -1;
         if (i < size) {
-#ifdef K1B_SEARCH_BRANCHY
-          uint32_t lo = 0, hi = k;  // first s with rstart[s+1] > i
-          while (lo < hi) {
-            const uint32_t mid = (lo + hi) >> 1;
-            if (rstart[mid + 1] <= i)
-              lo = mid + 1;
-            else
-              hi = mid;
-          }
-#else
           uint32_t lo = 0;  // last s with rstart[s] <= i: the run that holds instance i
           for (uint32_t step = kp2 >> 1; step > 0; step >>= 1)
             if (rstart[lo + step] <= i) lo += step;
-#endif
           sg[j] = (int)lo;
           ix[j] = cur[lo] + (i - rstart[lo]);
         }
@@ -370,25 +306,17 @@ __global__ void __launch_bounds__(K1B_THREADS, K1B_MIN_CTAS) k1b_group_kernel(co
 #pragma unroll
       for (int j = 0; j < PER; j++) {
         if (sg[j] >= 0) {
-#ifndef K1B_SEG_GLOBAL
           const uint32_t* const toff_s = sg_toff[sg[j]];
           const uint64_t* const poff_s = sg_poff[sg[j]];
-#else
-          const SegDesc& sd = a.segs[sg[j]];
-          const uint32_t* const toff_s = sd.toff;
-          const uint64_t* const poff_s = sd.poff;
-#endif
           to[j] = __ldg(toff_s + ix[j]);
           tn[j] = __ldg(toff_s + ix[j] + 1);
           pp[j] = __ldg(poff_s + ix[j]);
           p1[j] = __ldg(poff_s + ix[j] + 1);
         }
       }
-#if !defined(K1B_NO_PREFETCH_TB) && !defined(K1B_SEG_GLOBAL)
 #pragma unroll
       for (int j = 0; j < PER; j++)
         if (sg[j] >= 0) asm volatile("prefetch.global.L2 [%0];" ::"l"(sg_tb[sg[j]] + to[j] + cpl));
-#endif
       // (requesting the words of all four key windows before using any was measured slower,
       // 1.61 vs 1.43 ms, like batching the source copies below: the phase is bound by the
       // L1's handling of these 64-way scattered small reads, not by their latency)
@@ -398,16 +326,9 @@ __global__ void __launch_bounds__(K1B_THREADS, K1B_MIN_CTAS) k1b_group_kernel(co
           const uint32_t i = tid + j * K1B_THREADS;
           const uint32_t n = tn[j] - to[j];
           uint64_t kh, kl;
-#ifndef K1B_SEG_GLOBAL
           const uint8_t* const tb_s = sg_tb[sg[j]];
           const uint32_t* const post_s = sg_post[sg[j]];
           const uint32_t inst_s = sg_bl[sg[j]] + ix[j];
-#else
-          const SegDesc& sd = a.segs[sg[j]];
-          const uint8_t* const tb_s = sd.tb;
-          const uint32_t* const post_s = sd.post;
-          const uint32_t inst_s = sd.base + (ix[j] - sd.lo);
-#endif
           load_key16(tb_s, to[j], n, cpl, kh, kl);
           key_hi[i] = kh;
           key_lo[i] = kl;
@@ -416,17 +337,14 @@ __global__ void __launch_bounds__(K1B_THREADS, K1B_MIN_CTAS) k1b_group_kernel(co
           inst_a[i] = inst_s;
           pl[j] = (p1[j] - pp[j]) > 0xFFFFFFFEull ? 0xFFFFFFFFu : (uint32_t)(p1[j] - pp[j]);
           pp[j] = reinterpret_cast<uint64_t>(post_s + pp[j]);
-#ifndef K1B_NO_PREFETCH_POST
           // the copy of phase (5) is ~15 k clocks away: ask the L2 for the line now
           asm volatile("prefetch.global.L2 [%0];" ::"l"(pp[j]));
-#endif
         }
       }
     }
     // a thread's keys are visible to the block before it enters the hash table: whoever finds
     // its slot taken reads the owner's keys after the CAS
     __threadfence_block();
-    K1B_TICK(3);  // run search, offset loads, key windows (warp 0's own share)
 
     // ---------------- (3) group equal terms (hash table of representatives) ----------------
 #pragma unroll
@@ -434,21 +352,11 @@ __global__ void __launch_bounds__(K1B_THREADS, K1B_MIN_CTAS) k1b_group_kernel(co
       const uint32_t i = tid + j * K1B_THREADS;
       if (i >= size) break;
       const uint64_t kh = key_hi[i], kl = key_lo[i];
-#ifdef K1B_HASH64
-      uint64_t h = kh * 0x9E3779B97F4A7C15ull;
-      h ^= (kl + 0xD6E8FEB86659FD93ull + (h << 6) + (h >> 2));
-      h *= 0xFF51AFD7ED558CCDull;
-      h ^= h >> 33;
-      h += tlen[i] * 0xC2B2AE3D27D4EB4Full;
-      h ^= h >> 29;
-      uint32_t slot = (uint32_t)h & (K1B_HT - 1);
-#else
       // four 32-bit multiplies folded together; the top bits pick the slot
       uint32_t h = (uint32_t)kh * 0x9E3779B1u ^ (uint32_t)(kh >> 32) * 0x85EBCA77u ^
                    (uint32_t)kl * 0xC2B2AE3Du ^ (uint32_t)(kl >> 32) * 0x27D4EB2Fu;
       h = (h ^ (h >> 15)) * 0x2C1B3C6Du + tlen[i];
       uint32_t slot = (h ^ (h >> 13)) & (K1B_HT - 1);
-#endif
       uint32_t rep;
       for (;;) {
         const uint32_t prev = atomicCAS(&table[slot], K1B_EMPTY, i);
@@ -471,13 +379,10 @@ __global__ void __launch_bounds__(K1B_THREADS, K1B_MIN_CTAS) k1b_group_kernel(co
       og[j] = (rep << 20) |
               (atomicAdd(&cg[rep], (1u << 20) | (pl[j] > REG_CAP ? REG_CAP + 1 : pl[j])) & 0xFFFFFu);
     }
-    K1B_TICK(4);  // hash grouping (warp 0's own share)
     __syncthreads();
-    K1B_TICK(5);  // waiting for the other warps' keys + grouping
     const uint32_t D = s_nreps;
 
     // ---------------- (4) order the distinct terms; one record per term ----------------
-#ifndef K1B_RANK_WARP
     if (D <= K1B_SMALL_D) {  // rank by counting: EIGHT lanes per term, four terms per warp
       // (a warp per term leaves most lanes idle at ~24 distinct terms per bucket and takes
       // three rounds: 1.26 -> 1.23 ms; a thread per term issues a ninth of the instructions
@@ -533,50 +438,6 @@ __global__ void __launch_bounds__(K1B_THREADS, K1B_MIN_CTAS) k1b_group_kernel(co
           }
         }
       }
-    } else
-#endif
-    if (D <= K1B_SMALL_D) {  // rank by counting: one warp per term, lanes over the others
-#pragma unroll 1
-      for (uint32_t t = warp; t < D; t += K1B_WARPS) {
-        const uint32_t me = reps[t];
-        uint32_t rank = 0, ib = 0, pst = 0, est = 0;
-#pragma unroll 1
-        for (uint32_t j0 = 0; j0 < D; j0 += 32) {
-          const uint32_t j = j0 + lane;
-          uint32_t m_i = 0, m_p = 0, m_e = 0;
-          bool lt = false;
-          if (j < D) {
-            const uint32_t o = reps[j];
-            lt = o != me && less((uint16_t)o, (uint16_t)me);
-            if (lt) {
-              const uint32_t len = cg[o] & 0xFFFFFu;
-              m_i = cg[o] >> 20;
-              if (len <= REG_CAP) {
-                m_p = len;
-                m_e = enc_slot_words(len);
-              }
-            }
-          }
-          rank += __popc(__ballot_sync(0xffffffffu, lt));
-          ib += __reduce_add_sync(0xffffffffu, m_i);
-          pst += __reduce_add_sync(0xffffffffu, m_p);
-          est += __reduce_add_sync(0xffffffffu, m_e);
-        }
-        if (lane == 0) {
-          const uint32_t len = cg[me] & 0xFFFFFu;
-          const bool light = len <= REG_CAP;
-          const uint32_t src = (uint32_t)rec_base + icount + ib;
-          uint4* rec = reinterpret_cast<uint4*>(a.gin + rec_base + dcount + rank);
-          rec[0] = make_uint4(inst_a[me], tlen[me], src, cg[me] >> 20);
-          rec[1] = make_uint4(len, pcount + pst, ecount + est, 0u);
-          sbase[me] = src;
-          pbase[me] = light ? pcount + pst : K1B_HEAVY;
-          if (rank == D - 1) {
-            s_tot[0] = pst + (light ? len : 0u);
-            s_tot[1] = est + (light ? enc_slot_words(len) : 0u);
-          }
-        }
-      }
     } else {
       bitonic_sort_any(reps, D, tid, (uint32_t)K1B_THREADS, less, [] { __syncthreads(); });
       __syncthreads();
@@ -622,7 +483,6 @@ __global__ void __launch_bounds__(K1B_THREADS, K1B_MIN_CTAS) k1b_group_kernel(co
       }
     }
     __syncthreads();
-    K1B_TICK(6);  // ranking + records
 
     // ---------------- (5) sources of every term ---------------------------------------------
     // light terms: the postings themselves, copied into the term's slot (any order: the union
@@ -635,11 +495,7 @@ __global__ void __launch_bounds__(K1B_THREADS, K1B_MIN_CTAS) k1b_group_kernel(co
     // (requesting the first values of all four sources before storing any was measured
     // slower: 1.59 vs 1.44 ms)
     const uint32_t tile_p = s_tot[0];
-#ifdef K1B_NO_STAGE
-    const bool staged = false;
-#else
     const bool staged = tile_p <= K1B_STAGE_CAP;
-#endif
     uint32_t* const stage = reinterpret_cast<uint32_t*>(key_hi);  // key_hi | key_lo | key_x
     auto copy_source = [](const uint32_t* __restrict__ src, uint32_t* __restrict__ dst, uint32_t n) {
       uint32_t t = 0;
@@ -681,10 +537,8 @@ __global__ void __launch_bounds__(K1B_THREADS, K1B_MIN_CTAS) k1b_group_kernel(co
         }
       }
     }
-    K1B_TICK(7);  // source copies (warp 0's own share)
     if (staged) {
       __syncthreads();
-      K1B_TICK(8);  // waiting for the other warps' copies
       uint32_t* const out = gath + pcount;
       // head up to the first 16-byte boundary of the destination, then 128-bit stores
       const uint32_t head = min(tile_p, (uint32_t)((16u - ((uintptr_t)out & 15u)) & 15u) >> 2);
@@ -698,7 +552,6 @@ __global__ void __launch_bounds__(K1B_THREADS, K1B_MIN_CTAS) k1b_group_kernel(co
       const uint32_t tail0 = head + 4 * nvec;
       if (tail0 + tid < tile_p) out[tail0 + tid] = stage[tail0 + tid];
     }
-    K1B_TICK(9);  // coalesced write-out of the tile
     dcount += D;
     icount += size;
     pcount += s_tot[0];
@@ -714,10 +567,7 @@ __global__ void __launch_bounds__(K1B_THREADS, K1B_MIN_CTAS) k1b_group_kernel(co
 
 
 // ---------------------------------------------------------------- K2b: two terms per warp
-#ifndef K2B_THREADS_N
-#define K2B_THREADS_N 128
-#endif
-constexpr int K2B_THREADS = K2B_THREADS_N;
+constexpr int K2B_THREADS = 128;
 constexpr int K2B_WARPS = K2B_THREADS / 32;
 constexpr uint32_t K2B_HALF = 128;  // a 16-lane group handles terms of fewer values than this
 constexpr uint32_t K2B_ENC_WORDS = 3 + 2 * 129 + 1 + (5 * 127 + 3) / 4 + 1;  // enc_bound(255)
@@ -744,9 +594,7 @@ struct K2bArgs {
   const uint32_t* list;  // or: the buckets of this launch
 };
 
-#ifndef K2B_MIN_CTAS
-#define K2B_MIN_CTAS 8
-#endif
+constexpr int K2B_MIN_CTAS = 8;
 template <bool LIST>
 __global__ void __launch_bounds__(K2B_THREADS, K2B_MIN_CTAS) k2b_union_kernel(const K2bArgs a) {
   pdl_enter();
@@ -799,12 +647,6 @@ __global__ void __launch_bounds__(K2B_THREADS, K2B_MIN_CTAS) k2b_union_kernel(co
       uint32_t* const buf = s_buf[warp] + half * K2B_HALF;
       uint32_t* const ebuf = s_enc[warp] + half * (K2B_EBUF / 2);
       const uint32_t outn = union_blocked<16>(slot, buf, L, g.c > 1, a.rem);
-#ifdef K2B_PREFETCH_SLOT
-      // the record of the next round has arrived by now: its gathered values start moving
-      // towards the L2 while this round encodes and writes out
-      if (hl * 32 < g_next.L && hl < 8)
-        asm volatile("prefetch.global.L2 [%0];" ::"l"(gath + g_next.pst + hl * 32));
-#endif
       if (a.want_dec)
         for (uint32_t e = hl; e < outn; e += 16) slot[e] = buf[e];
       uint32_t enc = 0;
@@ -892,9 +734,7 @@ __global__ void __launch_bounds__(K2B_THREADS, K2B_MIN_CTAS) k2b_union_kernel(co
 constexpr uint32_t MW_CAP = 1024;
 constexpr int MW_V = 32;
 constexpr int MW_WARPS = 4;
-#ifndef MW_MIN_CTAS
-#define MW_MIN_CTAS 5  // 96 registers (6 = 80 registers measured no faster)
-#endif
+constexpr int MW_MIN_CTAS = 5;  // 96 registers (6 = 80 registers measured no faster)
 constexpr uint32_t MW_BUF = MW_CAP + MW_CAP / 32 + 8;   // one pad word per 32 values (bank-conflict-free blocked loads)
 constexpr uint32_t MW_EBUF = 3 + 8 * 129 + 1 + 1 + 6;   // enc_bound(1024) (also holds the source prefix: c + 1 <= 1025 entries)
 static_assert(MW_EBUF >= kMaxSegs + 1, "source prefix fits the stream buffer");
@@ -1764,18 +1604,6 @@ int k2_large_run(LargeArgs la, uint32_t h_nl, DevBuf<uint32_t>& large_tmp,
   return II2_OK;
 }
 
-#ifdef K1B_TIMING
-extern "C" int ii2_debug_k1b_clocks(unsigned long long* out, int reset) {
-  cudaDeviceSynchronize();
-  cudaMemcpyFromSymbol(out, g_k1b_clk, sizeof(g_k1b_clk));
-  if (reset) {
-    unsigned long long z[10] = {0};
-    cudaMemcpyToSymbol(g_k1b_clk, z, sizeof(z));
-  }
-  return 0;
-}
-#endif
-
 // ---------------------------------------------------------------- host driver
 bool k12_takes_fused(uint64_t N, int k) {
   const char* fused_env = getenv("II2_FUSED");
@@ -1872,12 +1700,7 @@ int k12_union(const MergePlan& plan, const RemovedSet& rem, bool want_dec, bool 
   a2.n_large = reinterpret_cast<uint32_t*>(u.totals.p + 6);
   a2.large_rec = large_u32.p;
   a2.large_bucket = large_u32.p + large_cap;
-  // II2_K1B_PAD=<bytes>: occupancy experiments (extra dynamic shared memory per CTA)
-  static const size_t pad = [] {
-    const char* e = getenv("II2_K1B_PAD");
-    return e ? (size_t)atol(e) : (size_t)0;
-  }();
-  const size_t smem = k1b_smem_bytes(k) + pad;
+  const size_t smem = k1b_smem_bytes(k);
   static size_t attr = 0;
   if (smem > attr) {
     const size_t want = std::max(k1b_smem_bytes(kMaxSegs), smem);
@@ -1933,7 +1756,7 @@ int k12_union(const MergePlan& plan, const RemovedSet& rem, bool want_dec, bool 
       w2.out_post = u.med_post.p;
       w2.out_enc = u.med_enc.p;
       w2.out_cursor = med_cursor.p;
-      II2_LAUNCH_CHAIN(k2_mwarp_kernel, kNumSMs * (MW_MIN_CTAS < 4 ? 4 : MW_MIN_CTAS), MW_WARPS * 32, 0, s, w2);
+      II2_LAUNCH_CHAIN(k2_mwarp_kernel, kNumSMs * MW_MIN_CTAS, MW_WARPS * 32, 0, s, w2);
       // one CTA per term: four warps up to 2048 values (eight CTAs per SM), eight warps up to
       // 4096 (five per SM); each passes the longer terms on through its own list
       uint32_t* const mid2_rec = large_u32.p + 6 * (size_t)large_cap;

@@ -126,10 +126,7 @@ k1_rank_samples(int k, const uint32_t* __restrict__ sbase, uint32_t S, SampleArr
   }
 }
 
-#ifndef K1_CHUNK_TERMS
-#define K1_CHUNK_TERMS 1024
-#endif
-constexpr uint32_t K1_CHUNK = K1_CHUNK_TERMS;
+constexpr uint32_t K1_CHUNK = 1024;
 
 // crank[c] = splitters <= the term just before chunk c (0 for the first chunk of a segment):
 // chunk c then owns the splitters [crank[c], crank[c+1]) (all the rest for a segment's last
@@ -484,27 +481,14 @@ int k1_build_plan(MergePlan& plan, const SegDesc* h_segs, uint32_t* sbase, cudaS
     return (v >= 32 && v <= 1024) ? (uint32_t)v : kInstancesPerBucket;
   }();
   uint64_t want = N / per_bucket;
-  // a small call (a narrow range read) is latency-bound: smaller buckets spread it over the SMs
-  // (II2_SMALL_BUCKET=<min instances per bucket>, 0 = off)
-  const uint32_t small_bucket = [] {  // (read per call: tuning runs sweep it inside one process)
-    const char* e = getenv("II2_SMALL_BUCKET");
-    const long v = e ? atol(e) : 128;
-    return (v >= 0 && v <= 1024) ? (uint32_t)v : 128u;
-  }();
-  const uint32_t small_want = [] {  // II2_SMALL_WANT=<buckets a small call is cut into>
-    const char* e = getenv("II2_SMALL_WANT");
-    const long v = e ? atol(e) : 592;
-    return (v >= 1 && v <= 65536) ? (uint32_t)v : 592u;
-  }();
-  if (small_bucket && want < small_want && N / small_bucket > want)
+  // a small call (a narrow range read) is latency-bound: smaller buckets spread it over the SMs,
+  // up to 592 buckets of at least 128 instances
+  constexpr uint32_t small_bucket = 128, small_want = 592;
+  if (want < small_want && N / small_bucket > want)
     want = std::min<uint64_t>(small_want, N / small_bucket);
   // ... and a window of a few hundred instances (a point read) is ONE bucket: planning it costs
-  // more launches than the bucket takes (k1_plan_single; II2_SINGLE_BUCKET=<max instances>, 0 = off)
-  const uint32_t single_max = [] {
-    const char* e = getenv("II2_SINGLE_BUCKET");
-    const long v = e ? atol(e) : 768;
-    return (v >= 0 && v <= 1024) ? (uint32_t)v : 768u;
-  }();
+  // more launches than the bucket takes (k1_plan_single)
+  constexpr uint32_t single_max = 768;
   if (N <= single_max || plan.speculative) want = 0;
   // II2_COALESCE=<fine> (default 1 = off): a partition `fine` times finer, coalesced afterwards.
   // Measured on B200 (C2, profiles/r02_experiments.md): fine = 4 takes the buckets above 1024

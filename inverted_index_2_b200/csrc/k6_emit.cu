@@ -55,9 +55,7 @@ constexpr uint32_t K6_MAX_GROUP = 32;  // buckets per CTA
 // bucket, form one flat sequence (buckets are in merged order and bk_out is the exclusive
 // prefix over buckets, so the running output positions simply continue across the buckets of
 // the group).  About 256 records per CTA: one set of block scans per 256 terms.
-#ifndef K6_MIN_CTAS
-#define K6_MIN_CTAS 6
-#endif
+constexpr int K6_MIN_CTAS = 6;
 __global__ void __launch_bounds__(K6_THREADS, K6_MIN_CTAS) k6_emit_kernel(const K6Args a, uint32_t group,
                                                              uint32_t n_buckets) {
   pdl_enter();
@@ -126,17 +124,6 @@ __global__ void __launch_bounds__(K6_THREADS, K6_MIN_CTAS) k6_emit_kernel(const 
       if (a.want_enc) a.o_val_off[t] = 4ull * w.enc_dst;
     }
     __syncthreads();
-#ifdef K6_SERIAL_COPY
-    for (uint32_t h = warp_id(); h < n_surv; h += K6_WARPS) {
-      const K6Work w = s_work[h];
-      const unsigned lane = lane_id();
-      for (uint32_t i = lane; i < w.tlen; i += 32) a.o_term_bytes[w.tdst + i] = w.tsrc[i];
-      if (a.want_dec)
-        for (uint32_t i = lane; i < w.cnt; i += 32) a.o_post[w.post_dst + i] = w.dsrc[i];
-      if (a.want_enc)
-        for (uint32_t i = lane; i < w.enc; i += 32) a.o_val_words[w.enc_dst + i] = w.esrc[i];
-    }
-#else
     // A term is ~15 bytes + ~100 words: with one load per lane in flight the warp pays a full
     // memory round trip per 32 words (source and destination may alias as far as the compiler
     // knows, so it keeps load -> store -> load in order).  The first 128 words of both streams
@@ -189,7 +176,6 @@ __global__ void __launch_bounds__(K6_THREADS, K6_MIN_CTAS) k6_emit_kernel(const 
             if (base + u * 32 + lane < w.cnt) a.o_post[w.post_dst + base + u * 32 + lane] = dv[u];
         }
     }
-#endif
     run_t += n_surv;
     run_tb += tot_a >> 32;
     run_p += tot_p;

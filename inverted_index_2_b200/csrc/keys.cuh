@@ -11,9 +11,9 @@
 namespace ii2 {
 
 // Bytes [c, c+16) of the term at tb+g0 (length len >= c) as two big-endian u64, zero padded
-// past the end.  Five aligned 32-bit loads + funnel shifts (KEYS_LOAD64: three 64-bit loads,
-// measured equal); tb must be 4-byte aligned (8 with KEYS_LOAD64) and readable 24 bytes past
-// the last term byte (segment term buffers are padded by 32).
+// past the end.  Five aligned 32-bit loads + funnel shifts (three aligned 64-bit loads were
+// measured equal and would need 8-byte alignment); tb must be 4-byte aligned and readable 24
+// bytes past the last term byte (segment term buffers are padded by 32).
 __device__ __forceinline__ void load_key16(const uint8_t* __restrict__ tb, uint32_t g0,
                                            uint32_t len, uint32_t c, uint64_t& hi, uint64_t& lo) {
   const uint32_t avail = len - c;
@@ -22,21 +22,10 @@ __device__ __forceinline__ void load_key16(const uint8_t* __restrict__ tb, uint3
     return;
   }
   const uint32_t a = g0 + c;
-#ifdef KEYS_LOAD64
-  // three aligned 8-byte loads cover any 16-byte window (fewer requests into the L1 than five
-  // 4-byte ones); word j of the little-endian 24 bytes, then the same funnel shifts
-  const uint2* wp = reinterpret_cast<const uint2*>(tb + (a & ~7u));
-  const uint2 q0 = __ldg(wp), q1 = __ldg(wp + 1), q2 = __ldg(wp + 2);
-  const bool up = (a & 4u) != 0;
-  const uint32_t sh = (a & 3u) * 8u;
-  const uint32_t w0 = up ? q0.y : q0.x, w1 = up ? q1.x : q0.y, w2 = up ? q1.y : q1.x,
-                 w3 = up ? q2.x : q1.y, w4 = up ? q2.y : q2.x;
-#else
   const uint32_t* wp = reinterpret_cast<const uint32_t*>(tb + (a & ~3u));
   const uint32_t sh = (a & 3u) * 8u;
   uint32_t w0 = __ldg(wp), w1 = __ldg(wp + 1), w2 = __ldg(wp + 2), w3 = __ldg(wp + 3),
            w4 = __ldg(wp + 4);
-#endif
   uint32_t x0 = __byte_perm(__funnelshift_r(w0, w1, sh), 0, 0x0123);
   uint32_t x1 = __byte_perm(__funnelshift_r(w1, w2, sh), 0, 0x0123);
   uint32_t x2 = __byte_perm(__funnelshift_r(w2, w3, sh), 0, 0x0123);

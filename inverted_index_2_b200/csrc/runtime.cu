@@ -12,11 +12,6 @@ namespace ii2 {
 
 std::atomic<uint64_t> g_kernel_launches{0};
 
-bool pdl_enabled() {  // read per launch (tuning runs flip it inside one process)
-  const char* e = getenv("II2_PDL");
-  return !(e && e[0] == '0');
-}
-
 static thread_local char t_last_error[512] = "";
 
 void set_last_error(const char* fmt, ...) {
@@ -107,7 +102,6 @@ DeviceScope::~DeviceScope() {
 struct ThreadStream {
   cudaStream_t own = nullptr;
   cudaStream_t aux = nullptr;
-  cudaStream_t copy[4] = {};
   cudaEvent_t ev[16] = {};
   cudaEvent_t wait_ev = nullptr;  // stream_wait
   cudaStream_t user = nullptr;
@@ -136,12 +130,6 @@ cudaStream_t aux_stream() {
   ThreadStream& t = thread_stream(t_dev);
   if (!t.aux) cudaStreamCreateWithFlags(&t.aux, cudaStreamNonBlocking);
   return t.aux;
-}
-
-cudaStream_t copy_stream(int i) {
-  ThreadStream& t = thread_stream(t_dev);
-  if (!t.copy[i]) cudaStreamCreateWithFlags(&t.copy[i], cudaStreamNonBlocking);
-  return t.copy[i];
 }
 
 cudaEvent_t aux_event(int i) {

@@ -37,7 +37,6 @@ struct DeviceScope {
 // The streams and events below belong to the calling thread AND the running call's device.
 cudaStream_t cur_stream();    // this thread's stream (caller-provided or library-owned)
 cudaStream_t aux_stream();    // a second library-owned stream of this thread (kernel overlap)
-cudaStream_t copy_stream(int i);  // copy-engine streams of this thread (staging of host slices), i < 4
 cudaEvent_t aux_event(int i);  // this thread's reusable timing-free events, i < 16
 
 // Per-(thread, device) scratch arena: one grow-only device block, bump-allocated during a pipeline call
