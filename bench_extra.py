@@ -6,6 +6,8 @@
   prefix  PrefixSearch batches over 64 resident segments (µs per call)
   lookup  batched exact-term reads (ii2_lookup_dev) on the C3 and C2 workloads, Q = 1 .. 65 536
         keys per call, against a loop of point reads for Q <= 256
+  query  boolean queries (ii2_query_dev) on the C2 and C3 workloads, Q = 1 .. 4096 per call, three
+        shapes, against lookup_dev + prefix_search_dev + host numpy set operations
   multidev  one process over every visible GPU (Engine(devices=...)): weak-scaling compaction from
         one host thread per device, a 1 % read partitioned over the devices + ii2_read_gather_devices,
         and ii2_prefix_gather_devices of the prefix batch; each checked against one device
@@ -168,6 +170,113 @@ def lookup(eng, a):
         if drem is not None:
             drem.release()
     print(json.dumps({"config": "batched term lookup (ii2_lookup_dev, results downloaded)", "cards": card,
+                      "terms": a.terms, "postings": a.postings, "results": rows}))
+
+
+def _compose(eng, dsegs, drem, removed, queries):
+    """The same answers as a caller composes them without ii2_query_dev: one lookup_dev call for
+    the batch's distinct terms, one prefix_search_dev call for its distinct prefixes, then numpy
+    set operations per query on the host (prefix search does not filter: the removed set is
+    subtracted here).  Returns (answers, values downloaded)."""
+    terms = sorted({t for q in queries for _, atoms in q for t, p in atoms if not p})
+    prefixes = sorted({t for q in queries for _, atoms in q for t, p in atoms if p})
+    look = dict(zip(terms, eng.lookup_dev(dsegs, terms, drem))) if terms else {}
+    pre = eng.prefix_search_dev(dsegs, prefixes) if prefixes else {}
+    empty = np.zeros(0, dtype=np.uint32)
+    lists = {(t, False): (np.unique(v) if v is not None else empty) for t, v in look.items()}
+    for t in prefixes:
+        v = pre.get(t, empty)
+        lists[(t, True)] = np.setdiff1d(v, removed, assume_unique=True) if removed is not None else v
+    out = []
+    for q in queries:
+        req, exc = [], []
+        for r, atoms in q:
+            u = lists[atoms[0]]
+            for at in atoms[1:]:
+                u = np.union1d(u, lists[at])
+            (req if r else exc).append(u)
+        req.sort(key=len)
+        e = req[0]
+        for x in req[1:]:
+            e = np.intersect1d(e, x, assume_unique=True)
+        for x in exc:
+            e = np.setdiff1d(e, x, assume_unique=True)
+        out.append(e)
+    downloaded = sum(len(v) for v in look.values() if v is not None) + sum(len(v) for v in pre.values())
+    return out, downloaded
+
+
+def query(eng, a):
+    """Boolean queries (ii2_query_dev, results downloaded) on the C2 workload (64 segments) and
+    the C3 workload (256 segments, 5 % removed), Q = 1 .. 4096 queries per call, in three shapes:
+    a term AND a 2-byte prefix; two 2-byte prefixes AND NOT a third; two 1-byte prefixes (clauses
+    of about 1.8 M values).  Each row also times the composition a caller writes without it
+    (_compose) and exits non-zero if the answers differ.  The host composition of two 1-byte
+    prefixes costs ~30 ms per query, so it runs up to Q = 256 there, and the first 256 answers of
+    the Q = 4096 batch are checked against it."""
+    card = _card()
+    rows = []
+    shapes = {
+        "term_and_prefix2": lambda a_, b_, c_: [(True, [(a_, False)]), (True, [(b_[:2], True)])],
+        "prefix2_and_prefix2_not_prefix2": lambda a_, b_, c_: [(True, [(a_[:2], True)]), (True, [(b_[:2], True)]),
+                                                               (False, [(c_[:2], True)])],
+        "prefix1_and_prefix1": lambda a_, b_, c_: [(True, [(a_[:1], True)]), (True, [(b_[:1], True)])],
+    }
+    for name, nseg, pres, seed, with_rem in (("C2", 64, 0.5, 0xC2, False), ("C3", 256, 0.125, 0xC3, True)):
+        w = synth.make_workload(a.terms, nseg, a.postings, seed=seed, presence=pres)
+        dsegs = [eng.upload(s) for s in w.segments]
+        drem = eng.upload_removed(w.removed) if with_rem else None
+        removed = w.removed if with_rem else None
+        n = len(w.term_off) - 1
+        rng = np.random.default_rng(9)
+        for shape, make in shapes.items():
+            picks = rng.integers(0, n, size=(4096, 3))
+            allq = [make(*(synth.term_at(w.term_bytes, w.term_off, int(i)) for i in row)) for row in picks]
+            ref256 = None
+            for q in (1, 16, 256, 4096):
+                queries = allq[:q]
+                res = None
+
+                def call():
+                    nonlocal res
+                    res = eng.query_dev(dsegs, queries, drem)
+                med, p99 = timed(call, 20 if q <= 256 else 5)
+                eng.prof_enable(True)
+                call()
+                phases = {p["name"]: round(1e3 * p["ms"] / max(1, p["count"]), 1) for p in eng.prof_read()}
+                eng.prof_enable(False)
+                row = {"workload": name, "segments": nseg, "removed": with_rem, "shape": shape, "queries": q,
+                       "median_us": 1e6 * med, "p99_us": 1e6 * p99, "values_downloaded": int(sum(len(v) for v in res)),
+                       "phase_us": phases}
+                if shape == "prefix1_and_prefix1" and q > 256:
+                    same = all(np.array_equal(x, y) for x, y in zip(res[:256], ref256))
+                    row.update({"compose": "not run (host intersections of ~1.8 M values per query); the "
+                                           "first 256 answers equal the Q = 256 composition",
+                                "same_as_compose": bool(same)})
+                else:
+                    comp = None
+
+                    def composed():
+                        nonlocal comp
+                        comp = _compose(eng, dsegs, drem, removed, queries)
+                    heavy = shape == "prefix1_and_prefix1" and q >= 16
+                    cmed, cp99 = timed(composed, 1 if heavy or q == 4096 else 5)
+                    same = all(np.array_equal(x, y) for x, y in zip(res, comp[0]))
+                    if q == 256:
+                        ref256 = comp[0]
+                    row.update({"compose_median_us": 1e6 * cmed, "compose_p99_us": 1e6 * cp99,
+                                "compose_values_downloaded": int(comp[1]), "speedup_vs_compose": cmed / med,
+                                "same_as_compose": bool(same)})
+                rows.append(row)
+                print(json.dumps(row), file=sys.stderr, flush=True)
+                if not row["same_as_compose"]:
+                    raise SystemExit(f"query: {shape} x {q} on {name} differs from the composed answers")
+        for s in dsegs:
+            s.release()
+        if drem is not None:
+            drem.release()
+    print(json.dumps({"config": "boolean queries (ii2_query_dev, results downloaded) vs lookup_dev + "
+                                "prefix_search_dev + host numpy set operations", "cards": card,
                       "terms": a.terms, "postings": a.postings, "results": rows}))
 
 
@@ -484,6 +593,8 @@ def main():
         prefix(eng, a)
     if "lookup" in a.which:
         lookup(eng, a)
+    if "query" in a.which:
+        query(eng, a)
 
 
 if __name__ == "__main__":

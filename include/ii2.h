@@ -324,6 +324,68 @@ int ii2_lookup(const ii2_seg_view* segs, int nseg, const uint8_t* key_bytes,
                uint64_t nrem, ii2_lookup_out* out);
 void ii2_lookup_out_free(ii2_lookup_out* out);
 
+/* ---- boolean term queries: AND / OR / NOT over exact terms and prefixes, many
+ *      queries per call (an extension beyond the reference's read surface) ---- */
+#define II2_ATOM_TERM 0
+#define II2_ATOM_PREFIX 1
+/* Q queries as three nested CSR levels: atom a = atom_bytes[atom_off[a] ..
+ * atom_off[a+1]) of kind atom_kind[a]; the atoms of clause c are
+ * [clause_atom_off[c], clause_atom_off[c+1]); the clauses of query q are
+ * [query_clause_off[q], query_clause_off[q+1]).  Every offset array starts at 0
+ * and is monotone; clause_atom_off[nclauses] == natoms and
+ * query_clause_off[nqueries] == nclauses. */
+typedef struct ii2_query_batch {
+  const uint8_t* atom_bytes;
+  const uint32_t* atom_off;         /* natoms + 1   */
+  const uint8_t* atom_kind;         /* natoms: II2_ATOM_* */
+  uint32_t natoms;
+  const uint32_t* clause_atom_off;  /* nclauses + 1 */
+  const uint8_t* clause_excluded;   /* nclauses: 0 = required, 1 = excluded */
+  uint32_t nclauses;
+  const uint32_t* query_clause_off; /* nqueries + 1 */
+  uint32_t nqueries;
+} ii2_query_batch;
+
+typedef struct ii2_query_out {
+  uint64_t n_queries;
+  uint32_t* values;        /* query i = values[value_off[i] .. value_off[i+1])  */
+  uint64_t* value_off;     /* n_queries + 1                                      */
+  uint64_t clause_values;  /* Σ sizes of the clause unions (work accounting)     */
+  void* _owner;
+} ii2_query_out;
+
+/* Semantics:
+ *   - values(TERM t)   = the sorted-unique set of t's values over all segments.
+ *     This is a set even when one segment holds t: unlike Read(t, t), which
+ *     passes a single-source list through as stored (quirk Q4).  An absent term
+ *     gives the empty set.
+ *   - values(PREFIX p) = found[p] of PrefixSearch, i.e. exactly the list
+ *     ii2_prefix_search_dev returns for p.  An unmatched prefix gives the empty
+ *     set; the empty prefix matches every term.
+ *   - values(clause)   = the union of its atoms; a clause with no atoms is the
+ *     empty set.
+ *   - result(query)    = the intersection of its required clauses, minus the
+ *     union of its excluded clauses, minus the removed set when rem != NULL
+ *     (reads never filter, quirk Q2, so rem is optional).  Ascending and unique.
+ *   - a query needs at least one required clause (there is no universe):
+ *     otherwise the call is II2_ERR_INVALID.  Duplicate atoms, clauses and
+ *     queries are allowed.
+ * ii2_query_dev runs on the device of its handles (handles of two devices:
+ * II2_ERR_INVALID); ii2_query uploads the views to the device the thread
+ * selected.  nqueries == 0 or nseg == 0 gives empty lists.  Outputs are pinned
+ * host memory; free them with ii2_query_out_free.  On error *out is zeroed.
+ * II2_ERR_INVALID (checked before any launch): NULL out or q, NULL arrays,
+ * non-monotone offsets, a first offset other than 0, a last offset that
+ * disagrees with the count of the next level, an unknown atom kind or clause
+ * flag, a query without a required clause.  II2_ERR_UNSUPPORTED: more than 1024
+ * segments, an atom longer than 65 535 bytes, a clause of more than 1024 atoms,
+ * a union of 2^32 values or more, natoms x nseg >= 2^32. */
+int ii2_query_dev(ii2_seg* const* segs, int nseg, const ii2_query_batch* q,
+                  const ii2_removed* rem, ii2_query_out* out);
+int ii2_query(const ii2_seg_view* segs, int nseg, const ii2_query_batch* q,
+              const uint32_t* removed_sorted, uint64_t nrem, ii2_query_out* out);
+void ii2_query_out_free(ii2_query_out* out);
+
 /* ---- cross-shard exchange: one process per GPU, contiguous shard-key ranges per
  *      rank (shardKey, shard.go:362-378), NCCL over NVLink --------------------
  * Compaction needs no exchange (shards never interact, shard.go:19-20).  Reads

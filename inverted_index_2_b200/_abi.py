@@ -27,6 +27,9 @@ II2_MERGE_WANT_DECODED = 1
 II2_RESULT_ENCODED = 1
 II2_RESULT_DECODED = 2
 
+II2_ATOM_TERM = 0
+II2_ATOM_PREFIX = 1
+
 u8p = C.POINTER(C.c_uint8)
 u32p = C.POINTER(C.c_uint32)
 u64p = C.POINTER(C.c_uint64)
@@ -106,6 +109,30 @@ class LookupOut(C.Structure):
         ("post", u32p),
         ("post_off", u64p),
         ("postings_in", C.c_uint64),
+        ("_owner", C.c_void_p),
+    ]
+
+
+class QueryBatch(C.Structure):
+    _fields_ = [
+        ("atom_bytes", u8p),
+        ("atom_off", u32p),
+        ("atom_kind", u8p),
+        ("natoms", C.c_uint32),
+        ("clause_atom_off", u32p),
+        ("clause_excluded", u8p),
+        ("nclauses", C.c_uint32),
+        ("query_clause_off", u32p),
+        ("nqueries", C.c_uint32),
+    ]
+
+
+class QueryOut(C.Structure):
+    _fields_ = [
+        ("n_queries", C.c_uint64),
+        ("values", u32p),
+        ("value_off", u64p),
+        ("clause_values", C.c_uint64),
         ("_owner", C.c_void_p),
     ]
 
@@ -199,6 +226,11 @@ PROTOTYPES = {
     "ii2_lookup": (C.c_int, [C.POINTER(SegView), C.c_int, u8p, u32p, C.c_uint32, u32p, C.c_uint64,
                              C.POINTER(LookupOut)]),
     "ii2_lookup_out_free": (None, [C.POINTER(LookupOut)]),
+    "ii2_query_dev": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.POINTER(QueryBatch), C.c_void_p,
+                                C.POINTER(QueryOut)]),
+    "ii2_query": (C.c_int, [C.POINTER(SegView), C.c_int, C.POINTER(QueryBatch), u32p, C.c_uint64,
+                            C.POINTER(QueryOut)]),
+    "ii2_query_out_free": (None, [C.POINTER(QueryOut)]),
     "ii2_comm_unique_id": (C.c_int, [u8p]),
     "ii2_comm_init": (C.c_int, [u8p, C.c_int, C.c_int]),
     "ii2_comm_info": (C.c_int, [C.POINTER(C.c_int), C.POINTER(C.c_int)]),

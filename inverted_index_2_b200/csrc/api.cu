@@ -5,12 +5,14 @@
 #include <cstdlib>
 #include <memory>
 #include <string>
+#include <unordered_map>
 #include <vector>
 
 #include "codec.cuh"
 #include "ingest.cuh"
 #include "lookup.cuh"
 #include "prefix.cuh"
+#include "query.cuh"
 #include "handles.cuh"
 #include "union.cuh"
 
@@ -1109,6 +1111,262 @@ void ii2_lookup_out_free(ii2_lookup_out* o) {
   memset(o, 0, sizeof(*o));
 }
 
+// ------------------------------------------------------------------ boolean term queries
+constexpr uint32_t kQueryMaxAtom = 65535;      // bytes of one atom (K5's term compare)
+constexpr uint32_t kQueryMaxClauseAtoms = 1024;  // sources of one clause union (k2_large_gather)
+
+// off[0 .. n]: starts at 0, monotone, and (last != ~0u) ends at `last`
+static bool query_csr_ok(const uint32_t* off, uint32_t n, uint32_t last) {
+  if (off[0] != 0) return false;
+  for (uint32_t i = 0; i < n; i++)
+    if (off[i + 1] < off[i]) return false;
+  return last == ~0u || off[n] == last;
+}
+
+// The batch's structure, on the host before anything is launched.
+static int query_validate(ii2_seg* const* segs, int nseg, const ii2_query_batch* qb) {
+  const uint32_t na = qb->natoms, nc = qb->nclauses, nq = qb->nqueries;
+  if (!qb->atom_off || !qb->clause_atom_off || !qb->query_clause_off ||
+      (na && !qb->atom_kind) || (nc && !qb->clause_excluded)) {
+    set_last_error("query: NULL batch array");
+    return II2_ERR_INVALID;
+  }
+  if (!query_csr_ok(qb->atom_off, na, ~0u) || !query_csr_ok(qb->clause_atom_off, nc, na) ||
+      !query_csr_ok(qb->query_clause_off, nq, nc)) {
+    set_last_error("query: offsets must start at 0, be monotone and end at the next level's count");
+    return II2_ERR_INVALID;
+  }
+  if (qb->atom_off[na] && !qb->atom_bytes) return II2_ERR_INVALID;
+  for (uint32_t a = 0; a < na; a++)
+    if (qb->atom_kind[a] > II2_ATOM_PREFIX) {
+      set_last_error("query: atom %u has unknown kind %u", a, qb->atom_kind[a]);
+      return II2_ERR_INVALID;
+    }
+  for (uint32_t c = 0; c < nc; c++)
+    if (qb->clause_excluded[c] > 1) {
+      set_last_error("query: clause %u has unknown flag %u", c, qb->clause_excluded[c]);
+      return II2_ERR_INVALID;
+    }
+  for (uint32_t q = 0; q < nq; q++) {
+    bool required = false;
+    for (uint32_t c = qb->query_clause_off[q]; c < qb->query_clause_off[q + 1] && !required; c++)
+      required = qb->clause_excluded[c] == 0;
+    if (!required) {
+      set_last_error("query %u has no required clause", q);
+      return II2_ERR_INVALID;
+    }
+  }
+  for (int i = 0; i < nseg; i++)
+    if (!segs[i]) return II2_ERR_INVALID;
+  if (nseg > kMaxSegs) {
+    set_last_error("%d segments in one call (max %d per pass)", nseg, kMaxSegs);
+    return II2_ERR_UNSUPPORTED;
+  }
+  for (uint32_t a = 0; a < na; a++)
+    if (qb->atom_off[a + 1] - qb->atom_off[a] > kQueryMaxAtom) {
+      set_last_error("query: atom %u is %u bytes long (max %u)", a,
+                     qb->atom_off[a + 1] - qb->atom_off[a], kQueryMaxAtom);
+      return II2_ERR_UNSUPPORTED;
+    }
+  for (uint32_t c = 0; c < nc; c++)
+    if (qb->clause_atom_off[c + 1] - qb->clause_atom_off[c] > kQueryMaxClauseAtoms) {
+      set_last_error("query: clause %u has %u atoms (max %u)", c,
+                     qb->clause_atom_off[c + 1] - qb->clause_atom_off[c], kQueryMaxClauseAtoms);
+      return II2_ERR_UNSUPPORTED;
+    }
+  if ((uint64_t)na * (uint64_t)nseg >= (1ull << 32) || na >= kClauseGroup) {
+    set_last_error("query: %u atoms x %d segments exceed 2^32 pairs", na, nseg);
+    return II2_ERR_UNSUPPORTED;
+  }
+  return II2_OK;
+}
+
+static int query_impl(ii2_seg* const* segs, int nseg, const ii2_query_batch* qb,
+                      const ii2_removed* rem, ii2_query_out* o, cudaStream_t s) {
+  ProfScope pipe_scope("query_total", s);
+  II2_TRY(query_validate(segs, nseg, qb));
+  const uint32_t na = qb->natoms, nc = qb->nclauses, nq = qb->nqueries;
+  std::unique_ptr<HostOwner> own(new HostOwner());
+  o->n_queries = nq;
+  if (nq == 0 || nseg == 0 || na == 0) {  // every clause is empty, so is every result
+    o->value_off = own->alloc<uint64_t>((size_t)nq + 1);
+    o->values = own->alloc<uint32_t>(0);
+    if (!o->value_off || !o->values) return II2_ERR_NOMEM;
+    memset(o->value_off, 0, ((size_t)nq + 1) * 8);
+    o->clause_values = 0;
+    o->_owner = own.release();
+    return II2_OK;
+  }
+  // distinct atoms (kind + bytes), in order of first appearance
+  std::vector<uint32_t> uid(na);
+  std::vector<uint32_t> u_first;  // an atom of every distinct atom
+  size_t ubytes = 0;
+  {
+    std::unordered_map<std::string, uint32_t> seen;
+    seen.reserve(na);
+    std::string key;
+    for (uint32_t a = 0; a < na; a++) {
+      const uint32_t o0 = qb->atom_off[a], n = qb->atom_off[a + 1] - o0;
+      key.assign(1, (char)qb->atom_kind[a]);
+      if (n) key.append(reinterpret_cast<const char*>(qb->atom_bytes + o0), n);
+      auto it = seen.emplace(key, (uint32_t)u_first.size());
+      if (it.second) {
+        u_first.push_back(a);
+        ubytes += n;
+      }
+      uid[a] = it.first->second;
+    }
+  }
+  const uint32_t nu = (uint32_t)u_first.size();
+  uint32_t ng = 0, nsrc = 0;
+  for (uint32_t c = 0; c < nc; c++) {
+    const uint32_t n = qb->clause_atom_off[c + 1] - qb->clause_atom_off[c];
+    if (n >= 2) {
+      ng++;
+      nsrc += n;
+    }
+  }
+  // segment table, distinct atoms, clauses, query offsets and clause-union sources through one
+  // pinned block and one copy; the atoms' list offsets come back into its tail
+  size_t cur = 0;
+  auto place = [&](size_t bytes) {
+    const size_t at = cur;
+    cur = (cur + bytes + 15) & ~(size_t)15;
+    return at;
+  };
+  const size_t o_segs = place(sizeof(SegDesc) * nseg);
+  const size_t o_gin = place(sizeof(GroupIn) * ng);
+  const size_t o_cl = place(sizeof(QueryClause) * nc);
+  const size_t o_aoff = place(4 * ((size_t)nu + 1));
+  const size_t o_qoff = place(4 * ((size_t)nq + 1));
+  const size_t o_grec = place(4 * (size_t)ng);
+  const size_t o_gatom = place(4 * (size_t)nsrc);
+  const size_t o_kind = place(nu);
+  const size_t o_bytes = place(ubytes);
+  const size_t stage_bytes = cur;
+  const size_t o_voff = place(8 * ((size_t)nu + 1));
+  struct PinnedBlock {
+    void* p = nullptr;
+    ~PinnedBlock() { pinned_free(p); }
+  } stage;
+  stage.p = pinned_alloc(cur);
+  if (!stage.p) return II2_ERR_NOMEM;
+  uint8_t* hb = static_cast<uint8_t*>(stage.p);
+  SegDesc* h = reinterpret_cast<SegDesc*>(hb + o_segs);
+  for (int i = 0; i < nseg; i++) {
+    const ii2_seg* g = segs[i];
+    h[i].tb = g->tb.p;
+    h[i].toff = g->toff.p;
+    h[i].post = g->post.p;
+    h[i].poff = g->poff.p;
+    h[i].n = g->n_terms;
+    h[i].lo = 0;
+    h[i].hi = g->n_terms;
+    h[i].base = 0;
+  }
+  uint32_t* h_aoff = reinterpret_cast<uint32_t*>(hb + o_aoff);
+  uint8_t* h_kind = hb + o_kind;
+  uint8_t* h_bytes = hb + o_bytes;
+  h_aoff[0] = 0;
+  for (uint32_t u = 0; u < nu; u++) {
+    const uint32_t a = u_first[u], o0 = qb->atom_off[a], n = qb->atom_off[a + 1] - o0;
+    if (n) memcpy(h_bytes + h_aoff[u], qb->atom_bytes + o0, n);
+    h_aoff[u + 1] = h_aoff[u] + n;
+    h_kind[u] = qb->atom_kind[a];
+  }
+  memcpy(hb + o_qoff, qb->query_clause_off, 4 * ((size_t)nq + 1));
+  GroupIn* h_gin = reinterpret_cast<GroupIn*>(hb + o_gin);
+  QueryClause* h_cl = reinterpret_cast<QueryClause*>(hb + o_cl);
+  uint32_t* h_grec = reinterpret_cast<uint32_t*>(hb + o_grec);
+  uint32_t* h_gatom = reinterpret_cast<uint32_t*>(hb + o_gatom);
+  for (uint32_t c = 0, g = 0, j = 0; c < nc; c++) {
+    const uint32_t a0 = qb->clause_atom_off[c], n = qb->clause_atom_off[c + 1] - a0;
+    h_cl[c].excluded = qb->clause_excluded[c];
+    if (n == 0) {
+      h_cl[c].src = kClauseEmpty;
+    } else if (n == 1) {
+      h_cl[c].src = uid[a0];
+    } else {
+      GroupIn gi;
+      memset(&gi, 0, sizeof(gi));
+      gi.src = j;
+      gi.c = n;
+      gi.L = 0xFFFFFFFFu;
+      h_gin[g] = gi;
+      h_grec[g] = g;
+      for (uint32_t i = 0; i < n; i++) h_gatom[j++] = uid[a0 + i];
+      h_cl[c].src = kClauseGroup | g++;
+    }
+  }
+  DevBuf<uint8_t> d_stage;
+  II2_TRY(d_stage.alloc_scratch(stage_bytes, s, 32));
+  II2_CUDA_TRY(cudaMemcpyAsync(d_stage.p, stage.p, stage_bytes, cudaMemcpyHostToDevice, s));
+  uint8_t* db = d_stage.p;
+  QueryDev d;
+  d.segs = reinterpret_cast<const SegDesc*>(db + o_segs);
+  d.k = nseg;
+  d.abytes = db + o_bytes;
+  d.aoff = reinterpret_cast<const uint32_t*>(db + o_aoff);
+  d.akind = db + o_kind;
+  d.nu = nu;
+  d.clauses = reinterpret_cast<const QueryClause*>(db + o_cl);
+  d.nclauses = nc;
+  d.qoff = reinterpret_cast<const uint32_t*>(db + o_qoff);
+  d.nq = nq;
+  d.gin = reinterpret_cast<const GroupIn*>(db + o_gin);
+  d.grec = reinterpret_cast<const uint32_t*>(db + o_grec);
+  d.gatom = reinterpret_cast<const uint32_t*>(db + o_gatom);
+  d.ngroups = ng;
+  d.nsrc = nsrc;
+  QueryHost hq;
+  hq.clauses = h_cl;
+  hq.qoff = qb->query_clause_off;
+  hq.gin = h_gin;
+  hq.gatom = h_gatom;
+  hq.value_off = reinterpret_cast<uint64_t*>(hb + o_voff);
+  RemovedSet rs;
+  if (rem) {
+    rs = rem->set();
+  } else {
+    rs.sorted = nullptr;
+    rs.n = 0;
+    rs.bitmap = nullptr;
+    rs.bitmap_bits = 0;
+  }
+  QueryOut qo;
+  II2_TRY(k9_query(d, hq, rs, qo, s));
+  II2_TRY(d2h(&o->values, qo.values.p, (size_t)qo.total, *own, s));
+  II2_TRY(d2h(&o->value_off, qo.value_off.p, (size_t)nq + 1, *own, s));
+  II2_CUDA_TRY(cudaStreamSynchronize(s));
+  o->clause_values = qo.clause_values;
+  o->_owner = own.release();
+  return II2_OK;
+}
+
+int ii2_query_dev(ii2_seg* const* segs, int nseg, const ii2_query_batch* q, const ii2_removed* rem,
+                  ii2_query_out* out) {
+  if (!out) return II2_ERR_INVALID;
+  memset(out, 0, sizeof(*out));
+  if (!q || nseg < 0 || (nseg && !segs)) return II2_ERR_INVALID;
+  int dev = -1;
+  II2_TRY(handles_device(segs, nseg, rem, &dev));
+  II2_TRY(ctx_require_device(dev));
+  cudaStream_t s = cur_stream();
+  const int rc = query_impl(segs, nseg, q, rem, out, s);
+  if (rc != II2_OK) {
+    cudaStreamSynchronize(s);
+    memset(out, 0, sizeof(*out));
+  }
+  arena_reset(s);
+  return rc;
+}
+
+void ii2_query_out_free(ii2_query_out* o) {
+  if (!o) return;
+  delete static_cast<HostOwner*>(o->_owner);
+  memset(o, 0, sizeof(*o));
+}
+
 // ------------------------------------------------------------------ ingest batching
 static int ingest_impl(const ii2_doc_view* docs, int ndocs, const uint32_t* removed_sorted,
                        uint64_t nrem, uint32_t flags, ii2_merge_out* out, cudaStream_t s) {
@@ -1896,6 +2154,24 @@ int ii2_lookup(const ii2_seg_view* segs, int nseg, const uint8_t* key_bytes,
   if (removed_sorted) II2_TRY(ii2_removed_upload(removed_sorted, nrem, &rem));
   std::unique_ptr<ii2_removed> rem_guard(rem);
   return ii2_lookup_dev(list.v.data(), nseg, key_bytes, key_off, nkeys, rem, out);
+}
+
+int ii2_query(const ii2_seg_view* segs, int nseg, const ii2_query_batch* q,
+              const uint32_t* removed_sorted, uint64_t nrem, ii2_query_out* out) {
+  if (!out) return II2_ERR_INVALID;
+  memset(out, 0, sizeof(*out));
+  if (!q || nseg < 0 || (nseg && !segs)) return II2_ERR_INVALID;
+  II2_TRY(ctx_require());
+  SegList list;
+  for (int i = 0; i < nseg; i++) {
+    ii2_seg* g = nullptr;
+    II2_TRY(ii2_seg_upload(&segs[i], &g));
+    list.v.push_back(g);
+  }
+  ii2_removed* rem = nullptr;
+  if (removed_sorted) II2_TRY(ii2_removed_upload(removed_sorted, nrem, &rem));
+  std::unique_ptr<ii2_removed> rem_guard(rem);
+  return ii2_query_dev(list.v.data(), nseg, q, rem, out);
 }
 
 }  // extern "C"

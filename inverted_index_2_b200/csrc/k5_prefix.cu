@@ -38,6 +38,7 @@ struct K5Args {
   int k;
   const uint8_t* pbytes;
   const uint32_t* poff;  // [np + 1]
+  const uint8_t* kind;   // [np] II2_ATOM_*, or null: every item is a prefix
   uint32_t np;
   uint64_t* src_ptr;   // [np * k]
   uint32_t* src_len;   // [np * k]
@@ -49,7 +50,8 @@ struct K5Args {
 
 // One WARP per (prefix, segment): lo = first term >= p (every term with prefix p is >= p),
 // hi = first term at or after lo that does not start with p (terms with a common prefix are
-// contiguous in bytes.Compare order); both are 32-way searches (warp_partition_point).
+// contiguous in bytes.Compare order); both are 32-way searches (warp_partition_point).  An exact
+// TERM item's window is [lo, lo + (term lo == p)).
 __global__ void __launch_bounds__(256) k5_windows(const K5Args a) {
   const uint64_t id = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   if (id >= (uint64_t)a.np * a.k) return;  // whole warps leave together
@@ -62,10 +64,20 @@ __global__ void __launch_bounds__(256) k5_windows(const K5Args a) {
     const uint32_t o = __ldg(sd.toff + i), n = __ldg(sd.toff + i + 1) - o;
     return term_compare(sd.tb + o, n, pb, pn) < 0;
   });
-  const uint32_t hi = warp_partition_point(lo, sd.n, [&](uint32_t i) {
-    const uint32_t o = __ldg(sd.toff + i), n = __ldg(sd.toff + i + 1) - o;
-    return has_prefix(sd.tb + o, n, pb, pn);
-  });
+  uint32_t hi;
+  if (a.kind && a.kind[p] == II2_ATOM_TERM) {  // uniform inside the warp
+    uint32_t eq = 0;
+    if (lo < sd.n) {
+      const uint32_t o = __ldg(sd.toff + lo), n = __ldg(sd.toff + lo + 1) - o;
+      eq = term_compare(sd.tb + o, n, pb, pn) == 0;
+    }
+    hi = lo + eq;
+  } else {
+    hi = warp_partition_point(lo, sd.n, [&](uint32_t i) {
+      const uint32_t o = __ldg(sd.toff + i), n = __ldg(sd.toff + i + 1) - o;
+      return has_prefix(sd.tb + o, n, pb, pn);
+    });
+  }
   if (lane_id() != 0) return;
   const uint64_t p0 = sd.poff[lo], p1 = sd.poff[hi];
   uint64_t len = p1 - p0;
@@ -112,7 +124,8 @@ k5_place(const GroupRec* __restrict__ recs, const uint64_t* __restrict__ off,
 }  // namespace
 
 int k5_prefix_search(const SegDesc* d_segs, int k, const uint8_t* d_pbytes, const uint32_t* d_poff,
-                     uint32_t np, PrefixOut& out, cudaStream_t s) {
+                     uint32_t np, PrefixOut& out, cudaStream_t s, const uint8_t* d_kind,
+                     uint64_t* h_value_off) {
   out.total = 0;
   II2_TRY(out.value_off.alloc((size_t)np + 1, s));
   II2_TRY(out.matched.alloc(np ? np : 1, s));
@@ -121,6 +134,7 @@ int k5_prefix_search(const SegDesc* d_segs, int k, const uint8_t* d_pbytes, cons
     II2_CUDA_TRY(cudaMemsetAsync(out.matched.p, 0, (np ? np : 1) * 4, s));
     II2_TRY(out.values.alloc(0, s));
     II2_CUDA_TRY(cudaStreamSynchronize(s));
+    if (h_value_off) memset(h_value_off, 0, ((size_t)np + 1) * 8);
     return II2_OK;
   }
   const uint64_t pairs = (uint64_t)np * k;
@@ -145,6 +159,7 @@ int k5_prefix_search(const SegDesc* d_segs, int k, const uint8_t* d_pbytes, cons
   a.k = k;
   a.pbytes = d_pbytes;
   a.poff = d_poff;
+  a.kind = d_kind;
   a.np = np;
   a.src_ptr = src_ptr.p;
   a.src_len = src_len.p;
@@ -188,6 +203,9 @@ int k5_prefix_search(const SegDesc* d_segs, int k, const uint8_t* d_pbytes, cons
   II2_TRY(exclusive_scan_u64(out.value_off.p, (uint64_t)np + 1, d_tot.p, s));
   II2_TRY(small_copy(h, d_tot.p, 8, s));
   II2_TRY(small_copy(h + 1, flags.p, 8, s));
+  if (h_value_off)
+    II2_CUDA_TRY(cudaMemcpyAsync(h_value_off, out.value_off.p, ((size_t)np + 1) * 8,
+                                 cudaMemcpyDeviceToHost, s));
   II2_CUDA_TRY(cudaStreamSynchronize(s));
   if ((uint32_t)h[1]) {
     set_last_error("prefix search: one segment holds more than 2^32-1 postings under a prefix");

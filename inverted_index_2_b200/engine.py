@@ -373,6 +373,38 @@ class Engine:
         blob = np.frombuffer(b"".join(prefixes) + b"\0", dtype=np.uint8).copy()
         return blob, off
 
+    @staticmethod
+    def _query_args(queries: list) -> tuple[A.QueryBatch, list]:
+        """Packs queries into ii2_query_batch's three CSR levels.  A query is a list of clauses,
+        a clause is (required: bool, [(bytes, is_prefix: bool), ...]).  Returns the struct and
+        the arrays it points into (keep them alive for the call)."""
+        atoms, kinds, clause_atom_off, excluded, query_clause_off = [], [], [0], [], [0]
+        for clauses in queries:
+            for required, alist in clauses:
+                for term, is_prefix in alist:
+                    atoms.append(bytes(term))
+                    kinds.append(A.II2_ATOM_PREFIX if is_prefix else A.II2_ATOM_TERM)
+                clause_atom_off.append(len(atoms))
+                excluded.append(0 if required else 1)
+            query_clause_off.append(len(excluded))
+        blob, aoff = Engine._prefix_args(atoms)
+        # one spare element each: no array is ever empty
+        kind = np.array(kinds + [0], dtype=np.uint8)
+        cao = np.array(clause_atom_off, dtype=np.uint32)
+        excl = np.array(excluded + [0], dtype=np.uint8)
+        qco = np.array(query_clause_off, dtype=np.uint32)
+        b = A.QueryBatch()
+        b.atom_bytes = A.np_ptr(blob, A.u8p)
+        b.atom_off = A.np_ptr(aoff, A.u32p)
+        b.atom_kind = A.np_ptr(kind, A.u8p)
+        b.natoms = len(atoms)
+        b.clause_atom_off = A.np_ptr(cao, A.u32p)
+        b.clause_excluded = A.np_ptr(excl, A.u8p)
+        b.nclauses = len(excluded)
+        b.query_clause_off = A.np_ptr(qco, A.u32p)
+        b.nqueries = len(queries)
+        return b, [blob, aoff, kind, cao, excl, qco]
+
     def _prefix_result(self, prefixes: list[bytes], out: A.PrefixOut) -> dict[bytes, np.ndarray]:
         """Zero-copy: the returned arrays are views of the library's pinned result buffer, which
         is released (ii2_prefix_out_free) when the last view is garbage collected."""
@@ -451,6 +483,44 @@ class Engine:
                                             removed.h if removed else None, C.byref(out)),
                     "lookup_dev")
         return self._lookup_result(out)
+
+    # ---- boolean term queries: AND / OR / NOT over exact terms and prefixes ------------------
+    def _query_result(self, out: A.QueryOut) -> list[np.ndarray]:
+        try:
+            n = int(out.n_queries)
+            off = A.from_ptr(out.value_off, n + 1, np.uint64)
+            vals = A.from_ptr(out.values, int(off[-1]) if n else 0, np.uint32)
+        finally:
+            self.lib.ii2_query_out_free(C.byref(out))
+        return [vals[int(off[i]):int(off[i + 1])] for i in range(n)]
+
+    def query(self, segs: list[FlatSegment], queries: list, removed=None) -> list[np.ndarray]:
+        """The values of every query over host views (see query_dev), aligned with `queries`."""
+        arr = views_array(segs)
+        batch, keep = self._query_args(queries)
+        if removed is None:
+            rp, nr, rkeep = C.cast(None, A.u32p), 0, None
+        else:
+            rkeep = np.ascontiguousarray(removed, dtype=np.uint32)
+            nr = len(rkeep)
+            if nr == 0:
+                rkeep = np.zeros(1, dtype=np.uint32)
+            rp = A.np_ptr(rkeep, A.u32p)
+        out = A.QueryOut()
+        self._check(self.lib.ii2_query(arr, len(segs), C.byref(batch), rp, nr, C.byref(out)), "query")
+        return self._query_result(out)
+
+    def query_dev(self, segs: list[DeviceSegment], queries: list,
+                  removed: DeviceRemoved | None = None) -> list[np.ndarray]:
+        """Boolean queries over resident segments in one call on their device.  A query is a list
+        of clauses (required: bool, [(bytes, is_prefix: bool), ...]); its result is the ascending
+        values in every required clause and in no excluded one (nor in `removed`), a clause
+        holding the values of any of its exact terms or prefixes."""
+        batch, keep = self._query_args(queries)
+        out = A.QueryOut()
+        self._check(self.lib.ii2_query_dev(self._handles(segs), len(segs), C.byref(batch),
+                                           removed.h if removed else None, C.byref(out)), "query_dev")
+        return self._query_result(out)
 
     # ---- codec -----------------------------------------------------------------------
     def intcomp_encode_batch(self, post: np.ndarray, post_off: np.ndarray):
