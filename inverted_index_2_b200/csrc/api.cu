@@ -297,21 +297,11 @@ k4_windows(const SegDesc* h_segs, SegDesc* d_segs, SegDesc* h_out,
 }
 
 // ------------------------------------------------------------------ the device pipeline
-// Point reads (see run_pipeline_impl): segments and postings the speculation covers.
-constexpr uint32_t kPointMaxSegs = 256;
-constexpr uint64_t kPointMaxPostings = 4096;
-// II2_POINT_READ (tuning / tests): 2 = the one-kernel point read (default), 1 = the general
-// kernels queued behind the windows kernel speculatively, 0 = a read like any other.
-static int point_read_mode() {
-  const char* e = getenv("II2_POINT_READ");
-  return (e && e[0] >= '0' && e[0] <= '2') ? e[0] - '0' : 2;
-}
-
 // segs: resident segments; [min,max] optional; rem optional.
 int run_pipeline_impl(ii2_seg* const* segs, int nseg, const uint8_t* min, size_t minlen,
                       bool has_min, const uint8_t* max, size_t maxlen, bool has_max,
                       const ii2_removed* rem, bool want_dec, bool want_enc, bool want_minmax,
-                      bool keep_empty, ii2_result** res_out, cudaStream_t s, bool allow_spec = true) {
+                      bool keep_empty, ii2_result** res_out, cudaStream_t s) {
   ProfScope pipe_scope("pipeline_total", s);
   std::unique_ptr<ii2_result> res(new ii2_result());
   res->stream = s;
@@ -324,53 +314,27 @@ int run_pipeline_impl(ii2_seg* const* segs, int nseg, const uint8_t* min, size_t
   }
   // segment table, sample bases and range bounds travel through one pinned block so that no
   // pageable copy stalls the stream
-  struct PinnedBlock {
-    void* p = nullptr;
-    ~PinnedBlock() { pinned_free(p); }
-  } stage;
   const size_t nsegx = nseg ? nseg : 1;
   const size_t stage_bytes = sizeof(SegDesc) * nsegx + 16 * nsegx + 8 * (nsegx + 1) + minlen + maxlen + 64;
-  stage.p = pinned_alloc(stage_bytes);
+  PinnedBlock stage(stage_bytes);
   if (!stage.p) return II2_ERR_NOMEM;
   SegDesc* h = static_cast<SegDesc*>(stage.p);
   uint64_t* h_post = reinterpret_cast<uint64_t*>(h + nsegx);  // (postings, term bytes) inside every window
   uint32_t* h_sbase = reinterpret_cast<uint32_t*>(h_post + 2 * nsegx);
   uint8_t* h_bounds = reinterpret_cast<uint8_t*>(h_sbase + 2 * (nsegx + 1));
-  uint64_t n_total64 = 0, n_in = 0, tb_in = 0;
-  for (int i = 0; i < nseg; i++) {
-    const ii2_seg* g = segs[i];
-    if (!g) return II2_ERR_INVALID;
-    h[i].tb = g->tb.p;
-    h[i].toff = g->toff.p;
-    h[i].post = g->post.p;
-    h[i].poff = g->poff.p;
-    h[i].n = g->n_terms;
-    h[i].lo = 0;
-    h[i].hi = g->n_terms;
-    h[i].base = (uint32_t)n_total64;
-    n_total64 += g->n_terms;
-    n_in += g->n_post;
-    tb_in += g->term_bytes_len;
-  }
+  uint64_t n_total64 = 0, n_in = 0, tb_in = 0;  // instances, postings and term bytes in the windows
+  II2_TRY(seg_table(h, segs, nseg, &n_total64));
   if (n_total64 >= (1ull << 32)) {
     set_last_error("more than 2^32-1 term instances in one call");
     return II2_ERR_UNSUPPORTED;
   }
+  const RemovedSet rs = removed_set(rem);
   // ---- Read(min == max), decoded output: the whole call is one kernel
-  if (allow_spec && point_read_mode() == 2 && nseg > 0 && has_min && has_max && minlen == maxlen &&
-      minlen <= kPointMaxTerm && (minlen == 0 || memcmp(min, max, minlen) == 0) && want_dec && !want_enc) {
+  if (nseg > 0 && has_min && has_max && minlen == maxlen && minlen <= kPointMaxTerm &&
+      (minlen == 0 || memcmp(min, max, minlen) == 0) && want_dec && !want_enc) {
     if (minlen) memcpy(h_bounds, min, minlen);
     uint64_t* const h_res = pinned_scratch() + 32;
-    RemovedSet rs0;
-    if (rem) {
-      rs0 = rem->set();
-    } else {
-      rs0.sorted = nullptr;
-      rs0.n = 0;
-      rs0.bitmap = nullptr;
-      rs0.bitmap_bits = 0;
-    }
-    II2_TRY(k4_point_read(h, nseg, h_bounds, (uint32_t)minlen, rs0, keep_empty, res->out, h_res, s));
+    II2_TRY(k4_point_read(h, nseg, h_bounds, (uint32_t)minlen, rs, keep_empty, res->out, h_res, s));
     II2_CUDA_TRY(cudaStreamSynchronize(s));
     if (h_res[0] == 1) {
       res->T = h_res[1];
@@ -391,23 +355,11 @@ int run_pipeline_impl(ii2_seg* const* segs, int nseg, const uint8_t* min, size_t
       *res_out = res.release();
       return II2_OK;
     }
-    // more than 4096 values: the general path below
+    // more than 4096 values: an ordinary read
   }
   DevBuf<SegDesc> d_segs;
   II2_TRY(d_segs.alloc_scratch(nsegx, s));
-  uint32_t n_total = (uint32_t)n_total64;
   const bool ranged = has_min || has_max;
-  bool spec = false;
-  auto windows_back = [&]() {  // after a synchronisation: the windows are in the pinned block
-    n_total64 = 0;
-    n_in = tb_in = 0;
-    for (int i = 0; i < nseg; i++) {
-      n_total64 += h[i].hi - h[i].lo;
-      n_in += h_post[2 * i];
-      tb_in += h_post[2 * i + 1];
-    }
-    n_total = (uint32_t)n_total64;
-  };
   if (ranged && nseg) {
     ProfScope win_scope("k4_windows_sync", s);
     DevBuf<uint8_t> d_bounds;
@@ -423,28 +375,25 @@ int run_pipeline_impl(ii2_seg* const* segs, int nseg, const uint8_t* min, size_t
     if (!ticket) return II2_ERR_NOMEM;
     II2_LAUNCH_CHAIN(k4_windows, div_up(nseg, 4), 256, 0, s, h, d_segs.p, h, h_post, nseg, bounds,
                      (uint32_t)minlen, has_min ? 1 : 0, (uint32_t)maxlen, has_max ? 1 : 0, ticket);
-    // A point read (min == max) holds at most one instance per segment, all of the same term:
-    // the rest of the call is queued behind the windows kernel with those bounds, without
-    // waiting for the windows (a round trip less); the plan empties itself on the device if
-    // the postings exceed the speculation, and the call is then run again the ordinary way.
-    spec = allow_spec && point_read_mode() >= 1 && has_min && has_max && minlen == maxlen &&
-           (minlen == 0 || memcmp(min, max, minlen) == 0) && nseg <= (int)kPointMaxSegs &&
-           k12_takes_fused((uint64_t)nseg, nseg);
-    if (spec) {
-      n_total = (uint32_t)nseg;
-      n_in = kPointMaxPostings;
-      tb_in = (uint64_t)nseg * minlen;
-    } else {
-      // the windows come back: the planner spreads its samples over them
-      II2_CUDA_TRY(cudaStreamSynchronize(s));
-      windows_back();
+    // the windows come back: the planner spreads its samples over them
+    II2_CUDA_TRY(cudaStreamSynchronize(s));
+    n_total64 = 0;
+    for (int i = 0; i < nseg; i++) {
+      n_total64 += h[i].hi - h[i].lo;
+      n_in += h_post[2 * i];
+      tb_in += h_post[2 * i + 1];
     }
-  } else if (nseg) {
-    II2_TRY(small_copy(d_segs.p, h, sizeof(SegDesc) * nseg, s));
+  } else {  // whole dictionaries
+    for (int i = 0; i < nseg; i++) {
+      n_in += segs[i]->n_post;
+      tb_in += segs[i]->term_bytes_len;
+    }
+    if (nseg) II2_TRY(small_copy(d_segs.p, h, sizeof(SegDesc) * nseg, s));
   }
+  const uint32_t n_total = (uint32_t)n_total64;
 
   EmitOut& out = res->out;
-  if (n_total == 0 && !spec) {  // nothing in range / no terms at all: empty result
+  if (n_total == 0) {  // nothing in range / no terms at all: empty result
     II2_TRY(out.term_bytes.alloc(0, s, 32));
     II2_TRY(out.term_off.alloc(1, s));
     II2_CUDA_TRY(cudaMemsetAsync(out.term_off.p, 0, 4, s));
@@ -466,31 +415,12 @@ int run_pipeline_impl(ii2_seg* const* segs, int nseg, const uint8_t* min, size_t
   plan.k = nseg;
   plan.n_total = n_total;
   plan.segs = d_segs.p;
-  plan.speculative = spec;
-  plan.spec_max_postings = kPointMaxPostings;
   II2_TRY(k1_build_plan(plan, h, h_sbase, s));
-  RemovedSet rs;
-  if (rem) {
-    rs = rem->set();
-  } else {
-    rs.sorted = nullptr;
-    rs.n = 0;
-    rs.bitmap = nullptr;
-    rs.bitmap_bits = 0;
-  }
   UnionOut u;
   // a small read: its result is placed before the host waits for the totals (one round trip
   // less); the arrays are sized by the window's own upper bounds, so only where those are small
   if (ranged && n_total <= 65536 && n_in <= (4u << 20) && tb_in <= (16u << 20)) u.early_out = &out;
   II2_TRY(k12_union(plan, rs, want_dec, want_enc, keep_empty, n_in, tb_in, u, s));
-  if (spec) {  // k12_union synchronised: the windows are back
-    windows_back();
-    if (n_total64 > (uint64_t)nseg || n_in > kPointMaxPostings) {  // the plan emptied itself
-      res.reset();
-      return run_pipeline_impl(segs, nseg, min, minlen, has_min, max, maxlen, has_max, rem, want_dec,
-                               want_enc, want_minmax, keep_empty, res_out, s, false);
-    }
-  }
   res->T = u.h_totals[0];
   res->TB = u.h_totals[1];
   res->P = u.h_totals[2];
@@ -504,9 +434,9 @@ int run_pipeline_impl(ii2_seg* const* segs, int nseg, const uint8_t* min, size_t
   }
   II2_TRY(k6_emit(plan, u, out, s));
 
-  uint8_t* mm = nullptr;
   if (want_minmax) {
-    mm = static_cast<uint8_t*>(pinned_alloc(8 + 2 * 65536));
+    PinnedBlock mm_blk(8 + 2 * 65536);
+    uint8_t* mm = static_cast<uint8_t*>(mm_blk.p);
     if (!mm) return II2_ERR_NOMEM;
     cudaError_t e = small_copy(mm, d_mm.p, 4096, s) == II2_OK ? cudaSuccess : cudaErrorUnknown;
     if (e == cudaSuccess) e = cudaStreamSynchronize(s);
@@ -519,14 +449,12 @@ int run_pipeline_impl(ii2_seg* const* segs, int nseg, const uint8_t* min, size_t
       }
     }
     if (e != cudaSuccess) {
-      pinned_free(mm);
       set_last_error("min/max copy: %s", cudaGetErrorString(e));
       return II2_ERR_CUDA;
     }
     res->min_term.assign(reinterpret_cast<const char*>(mm) + 8, ln[0]);
     res->max_term.assign(reinterpret_cast<const char*>(mm) + 8 + ln[0], ln[1]);
     res->has_minmax = u.terms_merged > 0;
-    pinned_free(mm);
   } else {
     II2_CUDA_TRY(cudaStreamSynchronize(s));
   }
@@ -534,17 +462,37 @@ int run_pipeline_impl(ii2_seg* const* segs, int nseg, const uint8_t* min, size_t
   return II2_OK;
 }
 
+// Runs impl(stream) on the calling thread's stream.  On failure the stream is drained (nothing
+// still writes the call's buffers) and *out is zeroed; the call's scratch is released either way.
+template <typename Out, typename Impl>
+int run_on_stream(Out* out, Impl&& impl) {
+  cudaStream_t s = cur_stream();
+  const int rc = impl(s);
+  if (rc != II2_OK) {
+    cudaStreamSynchronize(s);
+    memset(out, 0, sizeof(*out));
+  }
+  arena_reset(s);
+  return rc;
+}
+
+// Frees the host outputs of a call (ii2_merge_out, ii2_read_out, ii2_prefix_out ...).
+template <typename Out>
+void host_out_free(Out* o) {
+  if (!o) return;
+  delete static_cast<HostOwner*>(o->_owner);
+  memset(o, 0, sizeof(*o));
+}
+
 // Intermediates live in the calling thread's scratch arena for the duration of the call.
 int run_pipeline(ii2_seg* const* segs, int nseg, const uint8_t* min, size_t minlen, bool has_min,
                  const uint8_t* max, size_t maxlen, bool has_max, const ii2_removed* rem,
                  bool want_dec, bool want_enc, bool want_minmax, bool keep_empty,
                  ii2_result** res_out) {
-  cudaStream_t s = cur_stream();
-  const int rc = run_pipeline_impl(segs, nseg, min, minlen, has_min, max, maxlen, has_max, rem,
-                                   want_dec, want_enc, want_minmax, keep_empty, res_out, s);
-  if (rc != II2_OK) cudaStreamSynchronize(s);
-  arena_reset(s);
-  return rc;
+  return run_on_stream(res_out, [&](cudaStream_t s) {
+    return run_pipeline_impl(segs, nseg, min, minlen, has_min, max, maxlen, has_max, rem, want_dec,
+                             want_enc, want_minmax, keep_empty, res_out, s);
+  });
 }
 
 template <typename T>
@@ -565,13 +513,13 @@ int d2h(T** dst, const T* src, size_t n, HostOwner& own, cudaStream_t s) {
 
 // reads the accumulated result of k_seg_check (synchronises s)
 int seg_check_result(const uint32_t* d_stats, cudaStream_t s) {
-  uint32_t* hs = static_cast<uint32_t*>(pinned_alloc(8));
+  PinnedBlock blk(8);
+  uint32_t* hs = static_cast<uint32_t*>(blk.p);
   if (!hs) return II2_ERR_NOMEM;
   hs[0] = hs[1] = 0;
   cudaError_t e = small_copy(hs, d_stats, 8, s) == II2_OK ? cudaSuccess : cudaErrorUnknown;
   if (e == cudaSuccess) e = cudaStreamSynchronize(s);
   const uint32_t maxlen = hs[0], bad = hs[1];
-  pinned_free(hs);
   if (e != cudaSuccess) {
     set_last_error("segment check: %s", cudaGetErrorString(e));
     return II2_ERR_CUDA;
@@ -923,27 +871,12 @@ static int prefix_search_impl(ii2_seg* const* segs, int nseg, const uint8_t* pre
   const size_t nsegx = nseg ? nseg : 1;
   const size_t off_bytes = ((size_t)nprefix + 1) * 4;
   const size_t stage_bytes = sizeof(SegDesc) * nsegx + off_bytes + pbytes + 64;
-  struct PinnedBlock {
-    void* p = nullptr;
-    ~PinnedBlock() { pinned_free(p); }
-  } stage;
-  stage.p = pinned_alloc(stage_bytes);
+  PinnedBlock stage(stage_bytes);
   if (!stage.p) return II2_ERR_NOMEM;
   SegDesc* h = static_cast<SegDesc*>(stage.p);
   uint32_t* h_off = reinterpret_cast<uint32_t*>(h + nsegx);
   uint8_t* h_pb = reinterpret_cast<uint8_t*>(h_off + nprefix + 1);
-  for (int i = 0; i < nseg; i++) {
-    const ii2_seg* g = segs[i];
-    if (!g) return II2_ERR_INVALID;
-    h[i].tb = g->tb.p;
-    h[i].toff = g->toff.p;
-    h[i].post = g->post.p;
-    h[i].poff = g->poff.p;
-    h[i].n = g->n_terms;
-    h[i].lo = 0;
-    h[i].hi = g->n_terms;
-    h[i].base = 0;
-  }
+  II2_TRY(seg_table(h, segs, nseg));
   if (nprefix) {
     memcpy(h_off, prefix_off, off_bytes);
     if (pbytes) memcpy(h_pb, prefix_bytes, pbytes);
@@ -979,21 +912,12 @@ int ii2_prefix_search_dev(ii2_seg* const* segs, int nseg, const uint8_t* prefix_
   int dev = -1;
   II2_TRY(handles_device(segs, nseg, nullptr, &dev));
   II2_TRY(ctx_require_device(dev));
-  cudaStream_t s = cur_stream();
-  const int rc = prefix_search_impl(segs, nseg, prefix_bytes, prefix_off, nprefix, out, s);
-  if (rc != II2_OK) {
-    cudaStreamSynchronize(s);
-    memset(out, 0, sizeof(*out));
-  }
-  arena_reset(s);
-  return rc;
+  return run_on_stream(out, [&](cudaStream_t s) {
+    return prefix_search_impl(segs, nseg, prefix_bytes, prefix_off, nprefix, out, s);
+  });
 }
 
-void ii2_prefix_out_free(ii2_prefix_out* o) {
-  if (!o) return;
-  delete static_cast<HostOwner*>(o->_owner);
-  memset(o, 0, sizeof(*o));
-}
+void ii2_prefix_out_free(ii2_prefix_out* o) { host_out_free(o); }
 
 // ------------------------------------------------------------------ batched term lookup
 constexpr uint32_t kLookupMaxKey = 65535;  // bytes of one key
@@ -1037,26 +961,12 @@ static int lookup_impl(ii2_seg* const* segs, int nseg, const uint8_t* key_bytes,
   // segment table + key offsets + key bytes through one pinned block and one copy
   const size_t off_bytes = ((size_t)nkeys + 1) * 4;
   const size_t stage_bytes = sizeof(SegDesc) * nseg + off_bytes + kbytes + 64;
-  struct PinnedBlock {
-    void* p = nullptr;
-    ~PinnedBlock() { pinned_free(p); }
-  } stage;
-  stage.p = pinned_alloc(stage_bytes);
+  PinnedBlock stage(stage_bytes);
   if (!stage.p) return II2_ERR_NOMEM;
   SegDesc* h = static_cast<SegDesc*>(stage.p);
   uint32_t* h_off = reinterpret_cast<uint32_t*>(h + nseg);
   uint8_t* h_kb = reinterpret_cast<uint8_t*>(h_off + nkeys + 1);
-  for (int i = 0; i < nseg; i++) {
-    const ii2_seg* g = segs[i];
-    h[i].tb = g->tb.p;
-    h[i].toff = g->toff.p;
-    h[i].post = g->post.p;
-    h[i].poff = g->poff.p;
-    h[i].n = g->n_terms;
-    h[i].lo = 0;
-    h[i].hi = g->n_terms;
-    h[i].base = 0;
-  }
+  II2_TRY(seg_table(h, segs, nseg));
   memcpy(h_off, key_off, off_bytes);
   if (kbytes) memcpy(h_kb, key_bytes, kbytes);
   DevBuf<uint8_t> d_stage;
@@ -1065,19 +975,10 @@ static int lookup_impl(ii2_seg* const* segs, int nseg, const uint8_t* key_bytes,
   const SegDesc* d_segs = reinterpret_cast<const SegDesc*>(d_stage.p);
   const uint32_t* d_off = reinterpret_cast<const uint32_t*>(d_segs + nseg);
   const uint8_t* d_kb = reinterpret_cast<const uint8_t*>(d_off + nkeys + 1);
-  RemovedSet rs;
-  if (rem) {
-    rs = rem->set();
-  } else {
-    rs.sorted = nullptr;
-    rs.n = 0;
-    rs.bitmap = nullptr;
-    rs.bitmap_bits = 0;
-  }
   LookupOut lo;
   // plain reads keep empty lists; with a removed set an emptied key is not found (as
   // ii2_read_range_dev)
-  II2_TRY(k8_lookup(d_segs, nseg, n_post, d_kb, d_off, nkeys, rs, rem == nullptr, lo, s));
+  II2_TRY(k8_lookup(d_segs, nseg, n_post, d_kb, d_off, nkeys, removed_set(rem), rem == nullptr, lo, s));
   II2_TRY(d2h(&o->found, lo.found.p, nkeys, *own, s));
   II2_TRY(d2h(&o->post_off, lo.post_off.p, (size_t)nkeys + 1, *own, s));
   II2_TRY(d2h(&o->post, lo.post.p, (size_t)lo.total, *own, s));
@@ -1095,21 +996,12 @@ int ii2_lookup_dev(ii2_seg* const* segs, int nseg, const uint8_t* key_bytes,
   int dev = -1;
   II2_TRY(handles_device(segs, nseg, rem, &dev));
   II2_TRY(ctx_require_device(dev));
-  cudaStream_t s = cur_stream();
-  const int rc = lookup_impl(segs, nseg, key_bytes, key_off, nkeys, rem, out, s);
-  if (rc != II2_OK) {
-    cudaStreamSynchronize(s);
-    memset(out, 0, sizeof(*out));
-  }
-  arena_reset(s);
-  return rc;
+  return run_on_stream(out, [&](cudaStream_t s) {
+    return lookup_impl(segs, nseg, key_bytes, key_off, nkeys, rem, out, s);
+  });
 }
 
-void ii2_lookup_out_free(ii2_lookup_out* o) {
-  if (!o) return;
-  delete static_cast<HostOwner*>(o->_owner);
-  memset(o, 0, sizeof(*o));
-}
+void ii2_lookup_out_free(ii2_lookup_out* o) { host_out_free(o); }
 
 // ------------------------------------------------------------------ boolean term queries
 constexpr uint32_t kQueryMaxAtom = 65535;      // bytes of one atom (K5's term compare)
@@ -1245,25 +1137,10 @@ static int query_impl(ii2_seg* const* segs, int nseg, const ii2_query_batch* qb,
   const size_t o_bytes = place(ubytes);
   const size_t stage_bytes = cur;
   const size_t o_voff = place(8 * ((size_t)nu + 1));
-  struct PinnedBlock {
-    void* p = nullptr;
-    ~PinnedBlock() { pinned_free(p); }
-  } stage;
-  stage.p = pinned_alloc(cur);
+  PinnedBlock stage(cur);
   if (!stage.p) return II2_ERR_NOMEM;
   uint8_t* hb = static_cast<uint8_t*>(stage.p);
-  SegDesc* h = reinterpret_cast<SegDesc*>(hb + o_segs);
-  for (int i = 0; i < nseg; i++) {
-    const ii2_seg* g = segs[i];
-    h[i].tb = g->tb.p;
-    h[i].toff = g->toff.p;
-    h[i].post = g->post.p;
-    h[i].poff = g->poff.p;
-    h[i].n = g->n_terms;
-    h[i].lo = 0;
-    h[i].hi = g->n_terms;
-    h[i].base = 0;
-  }
+  II2_TRY(seg_table(reinterpret_cast<SegDesc*>(hb + o_segs), segs, nseg));
   uint32_t* h_aoff = reinterpret_cast<uint32_t*>(hb + o_aoff);
   uint8_t* h_kind = hb + o_kind;
   uint8_t* h_bytes = hb + o_bytes;
@@ -1324,17 +1201,8 @@ static int query_impl(ii2_seg* const* segs, int nseg, const ii2_query_batch* qb,
   hq.gin = h_gin;
   hq.gatom = h_gatom;
   hq.value_off = reinterpret_cast<uint64_t*>(hb + o_voff);
-  RemovedSet rs;
-  if (rem) {
-    rs = rem->set();
-  } else {
-    rs.sorted = nullptr;
-    rs.n = 0;
-    rs.bitmap = nullptr;
-    rs.bitmap_bits = 0;
-  }
   QueryOut qo;
-  II2_TRY(k9_query(d, hq, rs, qo, s));
+  II2_TRY(k9_query(d, hq, removed_set(rem), qo, s));
   II2_TRY(d2h(&o->values, qo.values.p, (size_t)qo.total, *own, s));
   II2_TRY(d2h(&o->value_off, qo.value_off.p, (size_t)nq + 1, *own, s));
   II2_CUDA_TRY(cudaStreamSynchronize(s));
@@ -1351,21 +1219,10 @@ int ii2_query_dev(ii2_seg* const* segs, int nseg, const ii2_query_batch* q, cons
   int dev = -1;
   II2_TRY(handles_device(segs, nseg, rem, &dev));
   II2_TRY(ctx_require_device(dev));
-  cudaStream_t s = cur_stream();
-  const int rc = query_impl(segs, nseg, q, rem, out, s);
-  if (rc != II2_OK) {
-    cudaStreamSynchronize(s);
-    memset(out, 0, sizeof(*out));
-  }
-  arena_reset(s);
-  return rc;
+  return run_on_stream(out, [&](cudaStream_t s) { return query_impl(segs, nseg, q, rem, out, s); });
 }
 
-void ii2_query_out_free(ii2_query_out* o) {
-  if (!o) return;
-  delete static_cast<HostOwner*>(o->_owner);
-  memset(o, 0, sizeof(*o));
-}
+void ii2_query_out_free(ii2_query_out* o) { host_out_free(o); }
 
 // ------------------------------------------------------------------ ingest batching
 static int ingest_impl(const ii2_doc_view* docs, int ndocs, const uint32_t* removed_sorted,
@@ -1392,11 +1249,7 @@ static int ingest_impl(const ii2_doc_view* docs, int ndocs, const uint32_t* remo
   // offsets rebased to one concatenated buffer, document starts and values: one pinned block
   const size_t off_bytes = ((size_t)N + 1) * 4, doff_bytes = ((size_t)ndocs + 1) * 8;
   const size_t stage_bytes = off_bytes + 8 + doff_bytes + (size_t)ndocs * 4 + 64;
-  struct PinnedBlock {
-    void* p = nullptr;
-    ~PinnedBlock() { pinned_free(p); }
-  } stage;
-  stage.p = pinned_alloc(stage_bytes);
+  PinnedBlock stage(stage_bytes);
   if (!stage.p) return II2_ERR_NOMEM;
   uint64_t* h_doff = static_cast<uint64_t*>(stage.p);
   uint32_t* h_vals = reinterpret_cast<uint32_t*>(h_doff + ndocs + 1);
@@ -1473,27 +1326,14 @@ int ii2_ingest(const ii2_doc_view* docs, int ndocs, const uint32_t* removed_sort
   if (!out || ndocs < 0 || (ndocs && !docs) || (nrem && !removed_sorted)) return II2_ERR_INVALID;
   memset(out, 0, sizeof(*out));
   II2_TRY(ctx_require());
-  cudaStream_t s = cur_stream();
-  const int rc = ingest_impl(docs, ndocs, removed_sorted, nrem, flags, out, s);
-  if (rc != II2_OK) {
-    cudaStreamSynchronize(s);
-    memset(out, 0, sizeof(*out));
-  }
-  arena_reset(s);
-  return rc;
+  return run_on_stream(out, [&](cudaStream_t s) {
+    return ingest_impl(docs, ndocs, removed_sorted, nrem, flags, out, s);
+  });
 }
 
-void ii2_merge_out_free(ii2_merge_out* o) {
-  if (!o) return;
-  delete static_cast<HostOwner*>(o->_owner);
-  memset(o, 0, sizeof(*o));
-}
+void ii2_merge_out_free(ii2_merge_out* o) { host_out_free(o); }
 
-void ii2_read_out_free(ii2_read_out* o) {
-  if (!o) return;
-  delete static_cast<HostOwner*>(o->_owner);
-  memset(o, 0, sizeof(*o));
-}
+void ii2_read_out_free(ii2_read_out* o) { host_out_free(o); }
 
 // ---- host-buffer entry points: upload, run, download --------------------------------
 struct SegList {
@@ -1692,14 +1532,11 @@ static int merge_pipelined(const ii2_seg_view* segs, int nseg, const uint32_t* r
   const size_t nx = (size_t)nseg;
   const size_t ref_bytes = (sizeof(SliceRef) * nx + 15) & ~(size_t)15;
   const size_t job_bytes = sizeof(GatherJob) * 4 * nx;
-  uint8_t* h_tab = static_cast<uint8_t*>(pinned_alloc((ref_bytes + job_bytes) * P));
-  struct PinGuard {
-    void* p;
-    ~PinGuard() { pinned_free(p); }
-  } tab_guard{h_tab};
+  PinnedBlock tab_blk((ref_bytes + job_bytes) * P);
+  uint8_t* h_tab = static_cast<uint8_t*>(tab_blk.p);
   if (!h_tab) return II2_ERR_NOMEM;
-  uint8_t* h_vtab = static_cast<uint8_t*>(pinned_alloc(sizeof(ValSlice) * nx * P + 64));
-  PinGuard vtab_guard{h_vtab};
+  PinnedBlock vtab_blk(sizeof(ValSlice) * nx * P + 64);
+  uint8_t* h_vtab = static_cast<uint8_t*>(vtab_blk.p);
   if (!h_vtab) return II2_ERR_NOMEM;
   auto enqueue_upload = [&](int p) -> int {
     parts[p].reset(new SegList());

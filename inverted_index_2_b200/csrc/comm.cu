@@ -291,12 +291,9 @@ int read_gather_impl(const ii2_result* local, int root, ii2_result** out, cudaSt
   // ---- sizes of every rank: one all-gather of {terms, term bytes, postings, -}
   DevBuf<uint64_t> d_sz;
   II2_TRY(d_sz.alloc_scratch(4 * (size_t)(world + 1), s));
-  uint64_t* h = static_cast<uint64_t*>(pinned_alloc(8 * 4 * (size_t)(world + 1)));
+  PinnedBlock h_blk(8 * 4 * (size_t)(world + 1));
+  uint64_t* h = static_cast<uint64_t*>(h_blk.p);
   if (!h) return II2_ERR_NOMEM;
-  struct Guard {
-    void* p;
-    ~Guard() { pinned_free(p); }
-  } guard{h};
   uint64_t* mine = h + 4 * (size_t)world;
   mine[0] = local->T;
   mine[1] = local->TB;
@@ -411,12 +408,9 @@ int prefix_gather_impl(const ii2_prefix_out* local, int root, ii2_prefix_out* ou
   const size_t row = (size_t)np + 1;
   II2_TRY(d_voff.alloc_scratch(row * (size_t)(world + 1), s));
   II2_TRY(d_m.alloc_scratch(((size_t)np + 16) * (size_t)(world + 1), s));
-  uint64_t* h_voff = static_cast<uint64_t*>(pinned_alloc(8 * row * (size_t)world + 64));
+  PinnedBlock voff_blk(8 * row * (size_t)world + 64);
+  uint64_t* h_voff = static_cast<uint64_t*>(voff_blk.p);
   if (!h_voff) return II2_ERR_NOMEM;
-  struct Guard {
-    void* p;
-    ~Guard() { pinned_free(p); }
-  } guard{h_voff};
   uint64_t* my_voff = d_voff.p + row * (size_t)world;
   uint8_t* my_m = d_m.p + (size_t)np * world;
   if (np) {
@@ -503,10 +497,6 @@ int prefix_union_on_root(const uint64_t* d_voff, const uint32_t* d_vals, const u
   out->matched = own->alloc<uint8_t>((size_t)np + 1);
   out->value_off = own->alloc<uint64_t>(row);
   if (!out->matched || !out->value_off) return II2_ERR_NOMEM;
-  struct Guard {
-    void* p;
-    ~Guard() { pinned_free(p); }
-  };
   // ---- per prefix: the sorted-unique union of its `world` lists (inverted_index.go:289-292)
   const uint64_t pairs = (uint64_t)np * world;
   DevBuf<uint64_t> src_ptr, d_vbase, d_off, d_tot;
@@ -525,9 +515,9 @@ int prefix_union_on_root(const uint64_t* d_voff, const uint32_t* d_vals, const u
   II2_TRY(d_tot.alloc_scratch(1, s));
   II2_TRY(d_mout.alloc_scratch(np, s));
   II2_CUDA_TRY(cudaMemsetAsync(flags.p, 0, 8, s));
-  uint64_t* h_small = static_cast<uint64_t*>(pinned_alloc(8 * (size_t)(world + 4)));
+  PinnedBlock small_blk(8 * (size_t)(world + 4));
+  uint64_t* h_small = static_cast<uint64_t*>(small_blk.p);
   if (!h_small) return II2_ERR_NOMEM;
-  Guard g2{h_small};
   for (int r = 0; r <= world; r++) h_small[r] = vbase[r];
   II2_TRY(small_copy(d_vbase.p, h_small, 8 * (size_t)(world + 1), s));
   k_prefix_sources<<<div_up(pairs, 256), 256, 0, s>>>(d_voff, d_vals, d_vbase.p, np, world, src_ptr.p,
@@ -540,10 +530,7 @@ int prefix_union_on_root(const uint64_t* d_voff, const uint32_t* d_vals, const u
   la.src_ptr = src_ptr.p;
   la.src_len = src_len.p;
   la.recs = recs.p;
-  la.rem.sorted = nullptr;
-  la.rem.n = 0;
-  la.rem.bitmap = nullptr;
-  la.rem.bitmap_bits = 0;
+  la.rem = RemovedSet{};
   la.want_enc = 0;
   la.keep_empty = 1;
   la.always_sort = 1;

@@ -27,15 +27,13 @@ struct ii2_removed {
   DevBuf<uint32_t> sorted;
   DevBuf<uint32_t> bitmap;
   uint64_t bitmap_bits = 0;
-  RemovedSet set() const {
-    RemovedSet r;
-    r.sorted = sorted.p;
-    r.n = n;
-    r.bitmap = bitmap_bits ? bitmap.p : nullptr;
-    r.bitmap_bits = bitmap_bits;
-    return r;
-  }
 };
+
+// The removed set of a call that takes an optional ii2_removed (empty for NULL).
+inline RemovedSet removed_set(const ii2_removed* rem) {
+  if (!rem) return RemovedSet{};
+  return RemovedSet{rem->sorted.p, rem->n, rem->bitmap_bits ? rem->bitmap.p : nullptr, rem->bitmap_bits};
+}
 
 struct ii2_result {
   int device = ctx_current_device();
@@ -63,6 +61,21 @@ inline int handles_device(ii2_seg* const* segs, int nseg, const ii2_removed* rem
     d = segs[i]->device;
   }
   *device = d;
+  return II2_OK;
+}
+
+// The segment table of a call: row i is segs[i] with its whole dictionary as the window, and its
+// instances are numbered after those of the rows before it (.base, which only the merge and
+// range-read pipeline reads).  II2_ERR_INVALID for a NULL segment; *n_inst = all instances.
+inline int seg_table(SegDesc* h, ii2_seg* const* segs, int nseg, uint64_t* n_inst = nullptr) {
+  uint64_t n = 0;
+  for (int i = 0; i < nseg; i++) {
+    const ii2_seg* g = segs[i];
+    if (!g) return II2_ERR_INVALID;
+    h[i] = SegDesc{g->tb.p, g->toff.p, g->post.p, g->poff.p, g->n_terms, 0, g->n_terms, (uint32_t)n};
+    n += g->n_terms;
+  }
+  if (n_inst) *n_inst = n;
   return II2_OK;
 }
 

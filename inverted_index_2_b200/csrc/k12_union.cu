@@ -1605,7 +1605,8 @@ int k2_large_run(LargeArgs la, uint32_t h_nl, DevBuf<uint32_t>& large_tmp,
 }
 
 // ---------------------------------------------------------------- host driver
-bool k12_takes_fused(uint64_t N, int k) {
+// Does a call of N instances over k segments take the fused bucket kernel?
+static bool k12_takes_fused(uint64_t N, int k) {
   const char* fused_env = getenv("II2_FUSED");
   const bool fused_on = fused_env ? atoi(fused_env) != 0 : N <= 65536;
   return fused_on && k12f_supported(k);

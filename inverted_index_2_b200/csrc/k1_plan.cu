@@ -312,13 +312,10 @@ k1_partition_chunks_raw(const SegDesc* __restrict__ segs, int k, const uint32_t*
 // One warp per bucket.  raw[0][b] = instances, raw[1][b] = input postings, raw[2][b] = staging
 // words (upper bound), raw[3][b] = term bytes of all instances (upper bound of the bucket's
 // merged term bytes).  Everything comes from the boundary tables the partition wrote.
-// sel != nullptr: rows were coalesced (k1_compact_rows) — row j of the tables is row sel[j] of the
-// fine partition, whose splitter is sample sel[j] - 1 (S_fine samples).
 __global__ void __launch_bounds__(256)
 k1_bucket_stats(int k, uint32_t S, SampleArrays sp, const uint32_t* __restrict__ part,
                 const uint32_t* __restrict__ btb, const uint64_t* __restrict__ bpo,
-                uint64_t* __restrict__ raw, uint32_t* __restrict__ bk_cpl,
-                const uint32_t* __restrict__ sel, uint32_t S_fine) {
+                uint64_t* __restrict__ raw, uint32_t* __restrict__ bk_cpl) {
   pdl_enter();
   const uint32_t b = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const uint32_t B = S + 1;
@@ -346,13 +343,11 @@ k1_bucket_stats(int k, uint32_t S, SampleArrays sp, const uint32_t* __restrict__
     raw[2ull * (B + 1) + b] = p + (p >> 2) + 6 * w;
     raw[3ull * (B + 1) + b] = t;
     uint32_t c = 0;
-    // the delimiting splitters of bucket b, if both exist (fine sample indexes)
-    const uint32_t r0 = sel ? sel[b] : b, r1 = sel ? sel[b + 1] : b + 1;
-    const uint32_t Sf = sel ? S_fine : S;
-    if (r0 >= 1 && r1 <= Sf && w) {
-      const uint8_t* x = reinterpret_cast<const uint8_t*>(sp.ptr[r0 - 1]);
-      const uint8_t* y = reinterpret_cast<const uint8_t*>(sp.ptr[r1 - 1]);
-      const uint32_t m = sp.len[r0 - 1] < sp.len[r1 - 1] ? sp.len[r0 - 1] : sp.len[r1 - 1];
+    // the delimiting splitters of bucket b (samples b - 1 and b), if both exist
+    if (b >= 1 && b < S && w) {
+      const uint8_t* x = reinterpret_cast<const uint8_t*>(sp.ptr[b - 1]);
+      const uint8_t* y = reinterpret_cast<const uint8_t*>(sp.ptr[b]);
+      const uint32_t m = sp.len[b - 1] < sp.len[b] ? sp.len[b - 1] : sp.len[b];
       while (c < m && x[c] == y[c]) c++;
     }
     bk_cpl[b] = c;
@@ -367,8 +362,7 @@ k1_bucket_stats(int k, uint32_t S, SampleArrays sp, const uint32_t* __restrict__
 __global__ void __launch_bounds__(256)
 k1_plan_single(const SegDesc* __restrict__ segs, int k, uint32_t* __restrict__ part,
                uint32_t* __restrict__ btb, uint64_t* __restrict__ bpo, uint64_t* __restrict__ bk_WP,
-               uint32_t* __restrict__ bk_cpl, uint64_t* __restrict__ totals, uint64_t max_w,
-               uint64_t max_p) {
+               uint32_t* __restrict__ bk_cpl, uint64_t* __restrict__ totals) {
   pdl_enter();
   __shared__ uint64_t ws[256 / 32 + 2];
   uint64_t w = 0, p = 0, t = 0;
@@ -391,8 +385,6 @@ k1_plan_single(const SegDesc* __restrict__ segs, int k, uint32_t* __restrict__ p
   block_exclusive_scan(p, ws, tp);
   block_exclusive_scan(t, ws, tt);
   if (threadIdx.x == 0) {
-    const bool fits = tw <= max_w && tp <= max_p;  // a speculative plan: else an empty bucket
-    if (!fits) tw = tp = tt = 0;
     const uint64_t v[4] = {tw, tp, tp + (tp >> 2) + 6 * tw, tt};  // as k1_bucket_stats
 #pragma unroll
     for (int j = 0; j < 4; j++) {
@@ -402,69 +394,6 @@ k1_plan_single(const SegDesc* __restrict__ segs, int k, uint32_t* __restrict__ p
     }
     bk_cpl[0] = 0;
   }
-}
-
-// ---- coalescing of a fine partition -----------------------------------------------------------
-// Evenly spaced terms of one segment are NOT evenly spaced in the merged order (the number of
-// other terms between two of them is negative-binomial: CV 0.2 at 64 segments), and a bucket
-// must fit a tile of the bucket kernel.  So the partition is made four times finer than needed
-// and whole fine buckets are joined: row r of the fine tables survives iff a multiple of the
-// target size lies in (C[r-1], C[r]], C[r] = instances before row r.  A final bucket then
-// holds target +- one fine bucket, and the number of final rows is bounded by N / target + 2
-// without asking the device: the table is padded with copies of the end row (empty buckets).
-__global__ void __launch_bounds__(256)
-k1_fine_sizes(const uint32_t* __restrict__ part, int k, uint32_t rows /* S_fine + 2 */,
-              uint64_t* __restrict__ cum) {
-  pdl_enter();
-  const uint32_t r = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;  // instances before row r
-  if (r >= rows) return;
-  uint64_t w = 0;
-  for (int s = lane_id(); s < k; s += 32) w += part[(uint64_t)r * k + s] - part[s];
-  w = warp_sum(w);
-  if (lane_id() == 0) cum[r] = w;
-}
-
-__global__ void __launch_bounds__(256)
-k1_select_rows(const uint64_t* __restrict__ cum, uint32_t rows, uint32_t target,
-               uint64_t* __restrict__ flag) {
-  pdl_enter();
-  const uint32_t r = blockIdx.x * blockDim.x + threadIdx.x;
-  if (r > rows) return;
-  uint64_t f = 0;
-  if (r == 0)
-    f = 1;  // window starts
-  else if (r < rows - 1)
-    f = cum[r] / target > cum[r - 1] / target ? 1 : 0;
-  flag[r] = f;  // flag[rows - 1] (window ends) and flag[rows] stay 0: the padding supplies them
-}
-
-__global__ void __launch_bounds__(256)
-k1_mark_rows(const uint64_t* __restrict__ idx, const uint64_t* __restrict__ cum, uint32_t rows,
-             uint32_t target, uint32_t* __restrict__ sel, uint32_t out_rows) {
-  pdl_enter();
-  const uint32_t r = blockIdx.x * blockDim.x + threadIdx.x;
-  if (r < rows - 1) {
-    const bool kept = r == 0 || cum[r] / target > cum[r - 1] / target;
-    if (kept && idx[r] < out_rows) sel[idx[r]] = r;
-  }
-  // rows past the kept ones: the end row
-  const uint64_t kept_total = idx[rows - 1];
-  if (r < out_rows && r >= kept_total) sel[r] = rows - 1;
-}
-
-__global__ void __launch_bounds__(256)
-k1_compact_rows(const uint32_t* __restrict__ sel, int k, uint32_t out_rows,
-                const uint32_t* __restrict__ part_f, const uint32_t* __restrict__ btb_f,
-                const uint64_t* __restrict__ bpo_f, uint32_t* __restrict__ part,
-                uint32_t* __restrict__ btb, uint64_t* __restrict__ bpo) {
-  pdl_enter();
-  const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= (uint64_t)out_rows * k) return;
-  const uint32_t j = (uint32_t)(i / k), s = (uint32_t)(i % k);
-  const uint64_t from = (uint64_t)sel[j] * k + s;
-  part[i] = part_f[from];
-  btb[i] = btb_f[from];
-  bpo[i] = bpo_f[from];
 }
 
 int k1_build_plan(MergePlan& plan, const SegDesc* h_segs, uint32_t* sbase, cudaStream_t s) {
@@ -489,26 +418,7 @@ int k1_build_plan(MergePlan& plan, const SegDesc* h_segs, uint32_t* sbase, cudaS
   // ... and a window of a few hundred instances (a point read) is ONE bucket: planning it costs
   // more launches than the bucket takes (k1_plan_single)
   constexpr uint32_t single_max = 768;
-  if (N <= single_max || plan.speculative) want = 0;
-  // II2_COALESCE=<fine> (default 1 = off): a partition `fine` times finer, coalesced afterwards.
-  // Measured on B200 (C2, profiles/r02_experiments.md): fine = 4 takes the buckets above 1024
-  // instances from 9.6 % to 2 %, but the finer partition costs +0.5 ms of plan time (0.38 ->
-  // 0.88 ms) for 0.3 ms saved in the bucket kernels: off by default, kept for skewed inputs.
-  // (II2_COALESCE_MIN=<buckets>: calls cut into fewer buckets keep the plain partition)
-  const uint32_t coalesce = [] {
-    const char* e = getenv("II2_COALESCE");
-    const long v = e ? atol(e) : 1;
-    return (v >= 1 && v <= 16) ? (uint32_t)v : 1u;
-  }();
-  const uint64_t coalesce_min = [] {
-    const char* e = getenv("II2_COALESCE_MIN");
-    const long v = e ? atol(e) : 2048;
-    return v >= 1 ? (uint64_t)v : 2048ull;
-  }();
-  const uint32_t fine =
-      (coalesce > 1 && want >= coalesce_min && want * coalesce < kMaxBuckets - 1) ? coalesce : 1;
-  const uint64_t want_final = want;
-  want *= fine;
+  if (N <= single_max) want = 0;
   if (want > kMaxBuckets - 1) want = kMaxBuckets - 1;
   uint32_t* cbase = sbase + (k + 1);
   sbase[0] = 0;
@@ -540,10 +450,8 @@ int k1_build_plan(MergePlan& plan, const SegDesc* h_segs, uint32_t* sbase, cudaS
     cbase[i + 1] = cbase[i] + (uint32_t)std::max<uint64_t>(1, (n + K1_CHUNK - 1) / K1_CHUNK);
   }
   const uint32_t S = sbase[k], n_chunks = cbase[k];  // S samples = S + 1 buckets of the partition
-  // final buckets: the partition's own, or the coalesced ones (an upper bound, padded)
-  const uint32_t target = (uint32_t)std::max<uint64_t>(1, N / std::max<uint64_t>(1, want_final));
-  const uint32_t B = fine > 1 ? (uint32_t)(N / target + 2) : S + 1;
-  plan.n_samples = B - 1;
+  const uint32_t B = S + 1;
+  plan.n_samples = S;
   plan.n_buckets = B;
   ProfScope scope("k1_plan", s);
   II2_TRY(plan.part.alloc_scratch((size_t)(B + 1) * k, s));
@@ -552,47 +460,23 @@ int k1_build_plan(MergePlan& plan, const SegDesc* h_segs, uint32_t* sbase, cudaS
   II2_TRY(plan.bpo.alloc_scratch((size_t)(B + 1) * k, s));
   II2_TRY(plan.bk_WP.alloc_scratch(4 * (size_t)(B + 1), s));
   II2_TRY(plan.totals.alloc_scratch(4, s));
-  DevBuf<uint32_t> part_f, btb_f, d_sel;
-  DevBuf<uint64_t> bpo_f, d_cum, d_idx;
-  uint32_t *p_part = plan.part.p, *p_btb = plan.btb.p;
-  uint64_t* p_bpo = plan.bpo.p;
-  if (fine > 1) {
-    II2_TRY(part_f.alloc_scratch((size_t)(S + 2) * k, s));
-    II2_TRY(btb_f.alloc_scratch((size_t)(S + 2) * k, s));
-    II2_TRY(bpo_f.alloc_scratch((size_t)(S + 2) * k, s));
-    II2_TRY(d_cum.alloc_scratch((size_t)S + 3, s));
-    II2_TRY(d_idx.alloc_scratch((size_t)S + 3, s));
-    II2_TRY(d_sel.alloc_scratch((size_t)B + 1, s));
-    p_part = part_f.p;
-    p_btb = btb_f.p;
-    p_bpo = bpo_f.p;
-  }
-  if (S == 0 && fine == 1) {
+  if (S == 0) {
     II2_LAUNCH_CHAIN(k1_plan_single, 1, 256, 0, s, plan.segs, k, plan.part.p, plan.btb.p, plan.bpo.p,
-                     plan.bk_WP.p, plan.bk_cpl.p, plan.totals.p,
-                     plan.speculative ? (uint64_t)N : ~0ull,
-                     plan.speculative ? plan.spec_max_postings : ~0ull);
+                     plan.bk_WP.p, plan.bk_cpl.p, plan.totals.p);
     return II2_OK;
-  }
-  if (plan.speculative) {
-    set_last_error("k1: a speculative plan must be the single bucket");
-    return II2_ERR_INVALID;
   }
   DevBuf<uint32_t> d_base, d_u32;
   DevBuf<uint64_t> d_u64;
-  const size_t Sx = S ? S : 1;
   II2_TRY(d_base.alloc_scratch(2 * (size_t)(k + 1), s));
-  II2_TRY(d_u64.alloc_scratch(6 * Sx, s));
-  II2_TRY(d_u32.alloc_scratch(4 * Sx, s));
+  II2_TRY(d_u64.alloc_scratch(6 * (size_t)S, s));
+  II2_TRY(d_u32.alloc_scratch(4 * (size_t)S, s));
   II2_TRY(small_copy(d_base.p, sbase, 2 * (size_t)(k + 1) * 4, s));  // sbase is pinned
   const uint32_t* d_sbase = d_base.p;
   const uint32_t* d_cbase = d_base.p + (k + 1);
-  SampleArrays sa{d_u64.p, d_u64.p + Sx, d_u64.p + 2 * Sx, d_u32.p, d_u32.p + Sx, d_u32.p + 2 * Sx};
-  SampleArrays sp{d_u64.p + 3 * Sx, d_u64.p + 4 * Sx, d_u64.p + 5 * Sx, d_u32.p + 3 * Sx, nullptr, nullptr};
-  if (S) {
-    II2_LAUNCH_CHAIN(k1_sample_keys, div_up(S, 256), 256, 0, s, plan.segs, k, d_sbase, S, sa);
-    II2_LAUNCH_CHAIN(k1_rank_samples, div_up((uint64_t)S * 32, 256), 256, 0, s, k, d_sbase, S, sa, sp);
-  }
+  SampleArrays sa{d_u64.p, d_u64.p + S, d_u64.p + 2 * S, d_u32.p, d_u32.p + S, d_u32.p + 2 * S};
+  SampleArrays sp{d_u64.p + 3 * S, d_u64.p + 4 * S, d_u64.p + 5 * S, d_u32.p + 3 * S, nullptr, nullptr};
+  II2_LAUNCH_CHAIN(k1_sample_keys, div_up(S, 256), 256, 0, s, plan.segs, k, d_sbase, S, sa);
+  II2_LAUNCH_CHAIN(k1_rank_samples, div_up((uint64_t)S * 32, 256), 256, 0, s, k, d_sbase, S, sa, sp);
   {
     constexpr size_t smem = (K1_CHUNK + 4 + 8) * 4 + K1_RAW_BYTES;
     static bool attr_set = false;
@@ -604,17 +488,11 @@ int k1_build_plan(MergePlan& plan, const SegDesc* h_segs, uint32_t* sbase, cudaS
     DevBuf<uint32_t> crank;
     II2_TRY(crank.alloc_scratch((size_t)n_chunks + 1, s));
     II2_LAUNCH_CHAIN(k1_chunk_ranks, div_up(n_chunks, 256), 256, 0, s, plan.segs, k, d_cbase, n_chunks, S, sp, crank.p);
-    II2_LAUNCH_CHAIN(k1_partition_chunks_raw, n_chunks, 256, smem, s, plan.segs, k, d_cbase, S, sp, crank.p, p_part, p_btb, p_bpo);
+    II2_LAUNCH_CHAIN(k1_partition_chunks_raw, n_chunks, 256, smem, s, plan.segs, k, d_cbase, S, sp, crank.p,
+                     plan.part.p, plan.btb.p, plan.bpo.p);
   }
-  if (fine > 1) {
-    const uint32_t rows = S + 2;
-    II2_LAUNCH_CHAIN(k1_fine_sizes, div_up((uint64_t)rows * 32, 256), 256, 0, s, p_part, k, rows, d_cum.p);
-    II2_LAUNCH_CHAIN(k1_select_rows, div_up((uint64_t)rows + 1, 256), 256, 0, s, d_cum.p, rows, target, d_idx.p);
-    II2_TRY(exclusive_scan_u64(d_idx.p, (uint64_t)rows + 1, nullptr, s));
-    II2_LAUNCH_CHAIN(k1_mark_rows, div_up(std::max<uint64_t>(rows, (uint64_t)B + 1), 256), 256, 0, s, d_idx.p, d_cum.p, rows, target, d_sel.p, B + 1);
-    II2_LAUNCH_CHAIN(k1_compact_rows, div_up((uint64_t)(B + 1) * k, 256), 256, 0, s, d_sel.p, k, B + 1, p_part, p_btb, p_bpo, plan.part.p, plan.btb.p, plan.bpo.p);
-  }
-  II2_LAUNCH_CHAIN(k1_bucket_stats, div_up((uint64_t)(B + 1) * 32, 256), 256, 0, s, k, B - 1, sp, plan.part.p, plan.btb.p, plan.bpo.p, plan.bk_WP.p, plan.bk_cpl.p, fine > 1 ? d_sel.p : nullptr, S);
+  II2_LAUNCH_CHAIN(k1_bucket_stats, div_up((uint64_t)(B + 1) * 32, 256), 256, 0, s, k, S, sp, plan.part.p,
+                   plan.btb.p, plan.bpo.p, plan.bk_WP.p, plan.bk_cpl.p);
   II2_TRY(exclusive_scan_multi_u64(plan.bk_WP.p, plan.bk_WP.p, B + 1, 4, plan.totals.p, s));
   return II2_OK;
 }

@@ -179,10 +179,7 @@ int k5_prefix_search(const SegDesc* d_segs, int k, const uint8_t* d_pbytes, cons
   la.src_ptr = src_ptr.p;
   la.src_len = src_len.p;
   la.recs = recs.p;
-  la.rem.sorted = nullptr;
-  la.rem.n = 0;
-  la.rem.bitmap = nullptr;
-  la.rem.bitmap_bits = 0;
+  la.rem = RemovedSet{};
   la.want_enc = 0;
   la.keep_empty = 1;
   la.always_sort = 1;

@@ -296,10 +296,7 @@ int k9_query(const QueryDev& d, const QueryHost& h, const RemovedSet& rem, Query
     la.src_ptr = src_ptr.p;
     la.src_len = src_len.p;
     la.recs = recs.p;
-    la.rem.sorted = nullptr;
-    la.rem.n = 0;
-    la.rem.bitmap = nullptr;
-    la.rem.bitmap_bits = 0;
+    la.rem = RemovedSet{};
     la.want_enc = 0;
     la.keep_empty = 1;
     la.always_sort = 1;

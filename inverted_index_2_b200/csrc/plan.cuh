@@ -36,12 +36,6 @@ struct MergePlan {
   const uint64_t* bk_E() const { return bk_WP.p + 2 * (size_t)(n_buckets + 1); }
   const uint64_t* bk_TB() const { return bk_WP.p + 3 * (size_t)(n_buckets + 1); }
   DevBuf<uint64_t> totals;        // [4] {Σ instances, Σ postings in, Σ staging words, Σ term bytes}
-  // A point read is planned BEFORE its windows are back on the host (api.cu): the plan is the
-  // single bucket whatever the window sizes, n_total is a bound, and the plan empties itself on
-  // the device when the windows hold more than `spec_max_postings` postings or more than
-  // n_total instances (the buffers behind it were sized for those).
-  bool speculative = false;
-  uint64_t spec_max_postings = 0;
 };
 
 // K1: choose splitters and partition every segment (the k-way merge of the term dictionaries,

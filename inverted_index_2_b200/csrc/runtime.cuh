@@ -115,6 +115,14 @@ struct ProfScope {
 // Pinned host memory with a size-class cache (cudaHostAlloc is far too slow per call).
 void* pinned_alloc(size_t bytes);
 void pinned_free(void* p);  // also accepts nullptr
+// A pinned block that is freed when it goes out of scope; p == nullptr if the allocation failed.
+struct PinnedBlock {
+  void* p;
+  explicit PinnedBlock(size_t bytes) : p(pinned_alloc(bytes)) {}
+  PinnedBlock(const PinnedBlock&) = delete;
+  PinnedBlock& operator=(const PinnedBlock&) = delete;
+  ~PinnedBlock() { pinned_free(p); }
+};
 // 256 bytes of pinned memory owned by the calling thread: the landing place of the small
 // device->host readbacks (totals, flags).  A pageable destination would make the copy wait for
 // every other transfer in flight, including the next range's staging on the second stream.

@@ -86,8 +86,6 @@ struct K12fArgs {
   uint32_t* def_list;
 };
 bool k12f_supported(int k);
-// Will k12_union take the fused bucket kernel for a call of N instances over k segments?
-bool k12_takes_fused(uint64_t N, int k);
 int k12f_launch(const K12fArgs& a, uint32_t n_buckets, cudaStream_t s);
 
 int k2_large_run(LargeArgs la, uint32_t n_groups, DevBuf<uint32_t>& large_tmp,

@@ -332,14 +332,11 @@ def test_merge_pipelined_by_term_range(engine, orc, monkeypatch):
     monkeypatch.delenv("II2_MERGE_PARTS", raising=False)
 
 
-@pytest.mark.parametrize("bucket,fine", [("64", "4"), ("200", "3"), ("32", "8"), ("1024", "2")])
-def test_merge_with_coalesced_partition(engine, orc, monkeypatch, bucket, fine, merge_path):
-    """Large calls partition the term space finer than needed and join whole fine buckets up to
-    the target size (k1_plan.cu, coalescing); forced on here for a small call.  Unequal segment
-    sizes, a range read and the padding buckets at the end of the table are covered."""
+@pytest.mark.parametrize("bucket", ["64", "200", "32", "1024"])
+def test_merge_with_small_buckets(engine, orc, monkeypatch, bucket, merge_path):
+    """A small call cut into many buckets (II2_BUCKET sets the instances per bucket): unequal
+    segment sizes, a tiny segment and a range read are covered."""
     monkeypatch.setenv("II2_BUCKET", bucket)
-    monkeypatch.setenv("II2_COALESCE", fine)
-    monkeypatch.setenv("II2_COALESCE_MIN", "4")
     w = synth.make_workload(40000, 9, 500000, universe=1 << 18, removed_frac=0.07, seed=91,
                             max_len=200)
     segs = list(w.segments)
@@ -348,8 +345,7 @@ def test_merge_with_coalesced_partition(engine, orc, monkeypatch, bucket, fine, 
     lo = synth.term_at(w.term_bytes, w.term_off, 3000)
     hi = synth.term_at(w.term_bytes, w.term_off, 31000)
     assert_read_equal(engine.read_range(segs, lo, hi), orc.read_range(segs, lo, hi))
-    for v in ("II2_BUCKET", "II2_COALESCE", "II2_COALESCE_MIN"):
-        monkeypatch.delenv(v, raising=False)
+    monkeypatch.delenv("II2_BUCKET", raising=False)
 
 
 def test_merge_pipelined_val_views(engine, orc, monkeypatch):
@@ -491,14 +487,13 @@ def test_read_range_matches_oracle(engine, orc, merge_path):
                           orc.read_range(w.segments, lo, hi, removed=w.removed))
 
 
-def test_point_reads(engine, orc, merge_path, monkeypatch):
-    """min == max: one kernel does the whole read (k4_point_kernel, <= 4096 values); failing that,
-    on the fused path the call is queued behind the windows kernel without waiting
-    for the windows (at most one instance per segment, postings speculated <= 4096).  A term that
-    is everywhere, in one segment, nowhere (between terms, before the first, after the last), the
-    empty term; with and without the removed filter; a term whose lists exceed the speculation
-    (the plan empties itself on the device and the call runs again); a term of > 256 values (the
-    bucket is deferred to the general kernels); the same with the speculation switched off."""
+def test_point_reads(engine, orc, merge_path):
+    """min == max: one kernel does the whole read (k4_point_kernel: <= 4096 values, terms <= 8192
+    bytes); when it declines, or the term is longer, the call continues as an ordinary read.  A
+    term that is everywhere, in one segment, nowhere (between terms, before the first, after the
+    last), the empty term; with and without the removed filter; terms of > 4096 values; a term of
+    > 256 values (the bucket is deferred to the general kernels); a term of > 8192 bytes in two
+    segments and one that is absent; one-term windows with min < max (the ordinary kernels)."""
     rng = np.random.default_rng(5)
     nseg = 9
     per_seg = [[] for _ in range(nseg)]
@@ -512,19 +507,18 @@ def test_point_reads(engine, orc, merge_path, monkeypatch):
     per_seg[6].append((b"hollow", []))
     per_seg[7].append((b"solo_big", rng.integers(0, 1 << 20, size=5000).tolist()))   # one source, > 4096
     per_seg[4].append((b"", [4, 2]))                  # the empty term
+    long_term = b"L" * 9000                           # longer than the point kernel stages
+    per_seg[1].append((long_term, [1, 3]))
+    per_seg[2].append((long_term, [2, 3, 70]))
     segs = [FlatSegment.from_items(sorted(x)) for x in per_seg]
     removed = np.unique(rng.integers(0, 5000, size=800)).astype(np.uint32)
     terms = [b"everywhere", b"only3", b"", b"big", b"mid", b"filler04", b"absent", b"everywhera", b"zzz",
-             b"\x00", b"filler", b"hollow", b"solo_big"]
-    for mode in (None, "1", "0"):   # the one-kernel read, the speculative chain, a read like any other
-        if mode is None:
-            monkeypatch.delenv("II2_POINT_READ", raising=False)
-        else:
-            monkeypatch.setenv("II2_POINT_READ", mode)
-        for t in terms:
-            assert_read_equal(engine.read_range(segs, t, t), orc.read_range(segs, t, t))
-            assert_read_equal(engine.read_range(segs, t, t, removed=removed),
-                              orc.read_range(segs, t, t, removed=removed))
+             b"\x00", b"filler", b"hollow", b"solo_big", long_term, b"L" * 8999 + b"M"]
+    windows = [(t, t) for t in terms] + [(t, t + b"\x00") for t in (b"everywhere", b"big")]
+    for lo, hi in windows:
+        assert_read_equal(engine.read_range(segs, lo, hi), orc.read_range(segs, lo, hi))
+        assert_read_equal(engine.read_range(segs, lo, hi, removed=removed),
+                          orc.read_range(segs, lo, hi, removed=removed))
     # resident segments: the same through the device API, results released between calls
     dsegs = [engine.upload(x) for x in segs]
     for t in terms:
