@@ -8,6 +8,8 @@
         keys per call, against a loop of point reads for Q <= 256
   query  boolean queries (ii2_query_dev) on the C2 and C3 workloads, Q = 1 .. 4096 per call, three
         shapes, against lookup_dev + prefix_search_dev + host numpy set operations
+  pattern  glob and fuzzy term patterns (ii2_pattern_search_dev) on the C3 workload, 1 .. 256 per
+        call in four groups, against read_range_dev + download + host filter and union
   multidev  one process over every visible GPU (Engine(devices=...)): weak-scaling compaction from
         one host thread per device, a 1 % read partitioned over the devices + ii2_read_gather_devices,
         and ii2_prefix_gather_devices of the prefix batch; each checked against one device
@@ -278,6 +280,149 @@ def query(eng, a):
     print(json.dumps({"config": "boolean queries (ii2_query_dev, results downloaded) vs lookup_dev + "
                                 "prefix_search_dev + host numpy set operations", "cards": card,
                       "terms": a.terms, "postings": a.postings, "results": rows}))
+
+
+def _host_patterns(terms_blob, starts, lists, pats):
+    """The host alternative's filter + union over the downloaded merged range: globs as one
+    multi-line regex scan of the newline-joined terms (C3 terms are letters only), fuzzy patterns
+    by the numpy edit-distance program of tests/test_gpu_pattern.py."""
+    import re
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    from test_gpu_pattern import glob_regex, levenshtein
+    post, post_off = lists
+    out = []
+    for p in pats:
+        if isinstance(p, bytes):
+            rx, _ = glob_regex(p)
+            body = rx.pattern.replace(b".", b"[^\n]")  # a term never spans a line
+            hits = [m.start() for m in re.finditer(rb"(?m)^(?:" + body + rb")$", terms_blob)]
+            idx = np.searchsorted(starts, np.array(hits, dtype=np.int64))
+        else:
+            q, k, plen = p
+            ts = terms_blob.split(b"\n")
+            idx = np.arange(len(ts), dtype=np.int64) if plen == 0 else \
+                np.array([i for i, t in enumerate(ts) if t[:plen] == q[:plen]], dtype=np.int64)
+            if len(idx):
+                idx = idx[levenshtein([ts[i][plen:] for i in idx], q[plen:]) <= k]
+        if len(idx) == 0:
+            out.append(None)
+            continue
+        lo, hi = post_off[idx].astype(np.int64), post_off[idx + 1].astype(np.int64)
+        sel = np.repeat(lo - np.cumsum(np.concatenate([[0], (hi - lo)[:-1]])), hi - lo) + \
+            np.arange(int((hi - lo).sum()))
+        out.append(np.unique(post[sel]).astype(np.uint32))
+    return out
+
+
+def pattern(eng, a):
+    """Wildcard and fuzzy term patterns (ii2_pattern_search_dev, results downloaded) on the
+    resident C3 workload (256 segments), batches of 1 / 16 / 256 patterns in four groups: anchored
+    globs (3-byte literal prefix), unanchored globs (*abc*), fuzzy k = 1 / 2 with P = 0 and with
+    P = 2.  Each batch of 1 and 16 is also answered the way a caller does without it: an open
+    ii2_read_range_dev, the download, the filter and the union on the host; the answers must agree
+    (`verified`).  The host filter of 256 patterns takes minutes, so the 256 batch is verified by
+    its first 16 answers, which must equal the 16 batch's.  Scanned bytes are the term bytes and
+    offsets of every window the patterns' groups read (unanchored patterns share one scan per
+    group of 16), over the call's median time and over the k10_match phase."""
+    card = _card()
+    w = synth.make_workload(a.terms, 256, a.postings, seed=0xC3, presence=0.125)
+    dsegs = [eng.upload(s) for s in w.segments]
+    n = len(w.term_off) - 1
+    tlen = np.diff(w.term_off).astype(np.int64)
+    inst = np.zeros(n + 1, dtype=np.int64)  # instances and term bytes of global terms [0, i)
+    ibytes = np.zeros(n + 1, dtype=np.int64)
+    for ids in w.seg_term_ids:
+        np.add.at(inst, ids + 1, 1)
+        np.add.at(ibytes, ids + 1, tlen[ids])
+    inst, ibytes = np.cumsum(inst), np.cumsum(ibytes)
+    terms = [synth.term_at(w.term_bytes, w.term_off, i) for i in range(n)]
+
+    def window(prefix):  # global term ids [lo, hi) that start with prefix
+        import bisect
+        lo = bisect.bisect_left(terms, prefix)
+        hi = bisect.bisect_left(terms, prefix + b"\xff" * 8) if prefix else n
+        return lo, hi
+
+    def scanned(pats):
+        full = int(ibytes[n] + 4 * inst[n])
+        unanchored, b = 0, 0
+        for p in pats:
+            pre = p[:3] if isinstance(p, bytes) and not p.startswith(b"*") else (p[0][:p[2]] if not isinstance(p, bytes) else b"")
+            if not pre:
+                unanchored += 1
+                continue
+            lo, hi = window(pre)
+            b += int(ibytes[hi] - ibytes[lo] + 4 * (inst[hi] - inst[lo]))
+        return b + (unanchored + 15) // 16 * full
+
+    rng = np.random.default_rng(10)
+    picks = [terms[int(i)] for i in rng.integers(0, n, size=256)]
+    groups = {
+        "glob_anchored": [t[:3] + b"*" + t[5:7] + b"*" for t in picks],
+        "glob_unanchored": [b"*" + t[3:6] + b"*" for t in picks],
+        "fuzzy_p0": [(t[:-1] + b"q", 1 + i % 2, 0) for i, t in enumerate(picks)],
+        "fuzzy_p2": [(t[:-1] + b"q", 1 + i % 2, 2) for i, t in enumerate(picks)],
+    }
+    host_data = None
+    rows = []
+    for gname, allp in groups.items():
+        ref16 = None
+        for q in (1, 16, 256):
+            pats = allp[:q]
+            res = None
+
+            def call():
+                nonlocal res
+                res = eng.pattern_search_dev(dsegs, pats)
+            med, p99 = timed(call, 20 if q <= 16 else 5)
+            eng.prof_enable(True)
+            call()
+            phases = {p["name"]: round(1e3 * p["ms"] / max(1, p["count"]), 1) for p in eng.prof_read()}
+            eng.prof_enable(False)
+            sb = scanned(pats)
+            row = {"group": gname, "patterns": q, "median_us": 1e6 * med, "p99_us": 1e6 * p99,
+                   "matched_patterns": int(sum(r is not None for r in res)),
+                   "values_out": int(sum(len(r) for r in res if r is not None)),
+                   "scanned_bytes": sb, "scan_gbs_call": sb / med / 1e9,
+                   "scan_gbs_match_phase": sb / (phases.get("k10_match", 0) * 1e-6) / 1e9
+                   if phases.get("k10_match") else None,
+                   "copy_ceiling_gbs": PEAK, "phase_us": phases}
+            if q <= 16:
+                hv = None
+
+                def host():
+                    nonlocal hv, host_data
+                    r = eng.read_range_dev(dsegs, None, None)
+                    d = r.download_read()
+                    r.release()
+                    blob = d.term_bytes.tobytes()
+                    starts = d.term_off[:-1].astype(np.int64) + np.arange(d.n_terms)
+                    joined = b"\n".join(blob[d.term_off[i]:d.term_off[i + 1]] for i in range(d.n_terms))
+                    host_data = (joined, starts, (d.post, d.post_off.astype(np.int64)))
+                    hv = _host_patterns(joined, starts, host_data[2], pats)
+                t0 = time.perf_counter()  # once: the host alternative takes seconds
+                host()
+                hmed = time.perf_counter() - t0
+                ok = all((x is None and y is None) or (x is not None and y is not None and np.array_equal(x, y))
+                         for x, y in zip(res, hv))
+                row.update({"host_median_us": 1e6 * hmed, "speedup_vs_host": hmed / med, "verified": bool(ok)})
+                if q == 16:
+                    ref16 = res
+            else:
+                ok = all((x is None and y is None) or (x is not None and y is not None and np.array_equal(x, y))
+                         for x, y in zip(res[:16], ref16))
+                row.update({"host": "not run (minutes of host filtering); the first 16 answers equal "
+                                    "the verified 16-pattern batch", "verified": bool(ok)})
+            rows.append(row)
+            print(json.dumps(row), file=sys.stderr, flush=True)
+            if not row["verified"]:
+                raise SystemExit(f"pattern: {gname} x {q} differs from the host answers")
+    for s in dsegs:
+        s.release()
+    print(json.dumps({"config": "term patterns (ii2_pattern_search_dev, results downloaded) vs "
+                                "read_range_dev + download + host filter and union", "cards": card,
+                      "terms": a.terms, "postings": w.postings_in, "term_instances": w.term_instances,
+                      "results": rows}))
 
 
 def c1(eng, a):
@@ -595,6 +740,8 @@ def main():
         lookup(eng, a)
     if "query" in a.which:
         query(eng, a)
+    if "pattern" in a.which:
+        pattern(eng, a)
 
 
 if __name__ == "__main__":

@@ -386,6 +386,57 @@ int ii2_query(const ii2_seg_view* segs, int nseg, const ii2_query_batch* q,
               const uint32_t* removed_sorted, uint64_t nrem, ii2_query_out* out);
 void ii2_query_out_free(ii2_query_out* out);
 
+/* ---- term patterns: wildcard (glob) and fuzzy matching of terms, the
+ *      counterpart of vellum's fst.Search(automaton, ...); many patterns per call
+ *      (an extension beyond the reference's read surface) ---------------------- */
+#define II2_PATTERN_GLOB 0
+#define II2_PATTERN_FUZZY 1
+typedef struct ii2_pattern_batch {
+  const uint8_t* pat_bytes;   /* pattern i = pat_bytes[pat_off[i] .. pat_off[i+1])        */
+  const uint32_t* pat_off;    /* npat + 1, starts at 0, monotone                         */
+  const uint8_t* pat_kind;    /* npat: II2_PATTERN_*                                     */
+  const uint8_t* max_edits;   /* npat: FUZZY only, 0..2 (may be NULL if no FUZZY)        */
+  const uint32_t* prefix_len; /* npat: FUZZY only, leading bytes that must match exactly
+                               * (NULL = 0 for every pattern)                            */
+  uint32_t npat;
+} ii2_pattern_batch;
+
+/* Semantics.  Every match is byte-wise, case-sensitive and anchored at both ends of
+ * the term.
+ *   - GLOB: `*` matches any run of bytes (also an empty one); `?` matches exactly
+ *     one byte; `[...]` matches one byte of a set, with ranges `a-z`; `[!...]` or
+ *     `[^...]` negates the set; a `]` placed first (after the negation) is a
+ *     literal; a `-` first or last is a literal; a range whose ends are reversed
+ *     (`[z-a]`) adds no byte.  `\x` makes any byte x a literal, inside a set too.
+ *     Every other byte is a literal.  A `[` without its closing `]`, or a trailing
+ *     `\`, is II2_ERR_INVALID.  The empty pattern matches only the empty term.
+ *   - FUZZY (pattern q, k = max_edits[i], P = prefix_len[i]): term t matches when
+ *     t[0..P) == q[0..P) and the Levenshtein distance between t[P..] and q[P..] is
+ *     at most k (insertions, deletions and substitutions of single bytes cost 1;
+ *     no transpositions).  Distances count BYTES, not runes: a multi-byte UTF-8
+ *     character can cost more than one edit.  P > len(q) is II2_ERR_INVALID.
+ *   - Output: matched[i] != 0 when at least one term instance matches pattern i,
+ *     even one whose list is empty (as in PrefixSearch); values of pattern i are
+ *     the sorted-unique union of the values of every matching term over all
+ *     segments.  No removed filter (reads never filter, quirk Q2), so the output is
+ *     an ii2_prefix_out that ii2_prefix_gather and ii2_prefix_gather_devices merge
+ *     as they merge prefix searches over the same pattern list.
+ *   - Patterns may repeat and come in any order.  npat == 0 or nseg == 0 gives
+ *     empty results.
+ * ii2_pattern_search_dev runs on the device of its handles (handles of two devices:
+ * II2_ERR_INVALID); ii2_pattern_search uploads the views to the device the thread
+ * selected.  Outputs are pinned host memory; free them with ii2_prefix_out_free.
+ * On error *out is zeroed.  II2_ERR_INVALID (checked before any launch): NULL out,
+ * q or arrays, pat_off not starting at 0 or not monotone, an unknown kind, the
+ * grammar errors above.  II2_ERR_UNSUPPORTED: a glob of more than 63 elements
+ * (items other than `*`), len(q) - P > 64 for a fuzzy pattern, max_edits > 2, a
+ * pattern longer than 65 535 bytes, more than 1024 segments, npat x nseg >= 2^32,
+ * one pattern's matched postings >= 2^32. */
+int ii2_pattern_search_dev(ii2_seg* const* segs, int nseg, const ii2_pattern_batch* q,
+                           ii2_prefix_out* out);
+int ii2_pattern_search(const ii2_seg_view* segs, int nseg, const ii2_pattern_batch* q,
+                       ii2_prefix_out* out);
+
 /* ---- cross-shard exchange: one process per GPU, contiguous shard-key ranges per
  *      rank (shardKey, shard.go:362-378), NCCL over NVLink --------------------
  * Compaction needs no exchange (shards never interact, shard.go:19-20).  Reads

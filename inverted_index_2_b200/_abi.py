@@ -30,6 +30,9 @@ II2_RESULT_DECODED = 2
 II2_ATOM_TERM = 0
 II2_ATOM_PREFIX = 1
 
+II2_PATTERN_GLOB = 0
+II2_PATTERN_FUZZY = 1
+
 u8p = C.POINTER(C.c_uint8)
 u32p = C.POINTER(C.c_uint32)
 u64p = C.POINTER(C.c_uint64)
@@ -137,6 +140,17 @@ class QueryOut(C.Structure):
     ]
 
 
+class PatternBatch(C.Structure):
+    _fields_ = [
+        ("pat_bytes", u8p),
+        ("pat_off", u32p),
+        ("pat_kind", u8p),
+        ("max_edits", u8p),
+        ("prefix_len", u32p),
+        ("npat", C.c_uint32),
+    ]
+
+
 class FstTerms(C.Structure):
     _fields_ = [
         ("n_terms", C.c_uint64),
@@ -231,6 +245,10 @@ PROTOTYPES = {
     "ii2_query": (C.c_int, [C.POINTER(SegView), C.c_int, C.POINTER(QueryBatch), u32p, C.c_uint64,
                             C.POINTER(QueryOut)]),
     "ii2_query_out_free": (None, [C.POINTER(QueryOut)]),
+    "ii2_pattern_search_dev": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.POINTER(PatternBatch),
+                                         C.POINTER(PrefixOut)]),
+    "ii2_pattern_search": (C.c_int, [C.POINTER(SegView), C.c_int, C.POINTER(PatternBatch),
+                                     C.POINTER(PrefixOut)]),
     "ii2_comm_unique_id": (C.c_int, [u8p]),
     "ii2_comm_init": (C.c_int, [u8p, C.c_int, C.c_int]),
     "ii2_comm_info": (C.c_int, [C.POINTER(C.c_int), C.POINTER(C.c_int)]),

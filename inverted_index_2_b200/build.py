@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libii2.so")
 SOURCES = ["runtime.cu", "k3a_intcomp.cu", "k1_plan.cu", "k12_union.cu", "k12_fused.cu", "k6_emit.cu",
-           "k5_prefix.cu", "k7_ingest.cu", "k8_lookup.cu", "k9_query.cu", "k3b_bitmask.cu", "api.cu", "comm.cu", "fst_v1.cpp", "removed_gob.cpp"]
+           "k5_prefix.cu", "k7_ingest.cu", "k8_lookup.cu", "k9_query.cu", "k10_pattern.cu", "k3b_bitmask.cu", "api.cu", "comm.cu", "fst_v1.cpp", "removed_gob.cpp"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC"]
 

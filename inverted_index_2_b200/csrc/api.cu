@@ -12,6 +12,7 @@
 #include "ingest.cuh"
 #include "lookup.cuh"
 #include "prefix.cuh"
+#include "pattern.cuh"
 #include "query.cuh"
 #include "handles.cuh"
 #include "union.cuh"
@@ -856,6 +857,22 @@ int ii2_result_device(const ii2_result* r, int* device) {
 }
 
 // ------------------------------------------------------------------ PrefixSearch
+// The n items of a device PrefixOut into *o (pinned host memory owned by o->_owner).
+static int prefix_out_download(const PrefixOut& po, uint32_t n, ii2_prefix_out* o, cudaStream_t s) {
+  std::unique_ptr<HostOwner> own(new HostOwner());
+  uint32_t* h_matched = nullptr;
+  II2_TRY(d2h(&o->values, po.values.p, (size_t)po.total, *own, s));
+  II2_TRY(d2h(&o->value_off, po.value_off.p, (size_t)n + 1, *own, s));
+  II2_TRY(d2h(&h_matched, po.matched.p, (size_t)(n ? n : 1), *own, s));
+  II2_CUDA_TRY(cudaStreamSynchronize(s));
+  o->matched = own->alloc<uint8_t>((size_t)n + 1);
+  if (!o->matched) return II2_ERR_NOMEM;
+  for (uint32_t i = 0; i < n; i++) o->matched[i] = h_matched[i] ? 1 : 0;
+  o->n_prefixes = n;
+  o->_owner = own.release();
+  return II2_OK;
+}
+
 static int prefix_search_impl(ii2_seg* const* segs, int nseg, const uint8_t* prefix_bytes,
                               const uint32_t* prefix_off, uint32_t nprefix, ii2_prefix_out* o,
                               cudaStream_t s) {
@@ -891,18 +908,7 @@ static int prefix_search_impl(ii2_seg* const* segs, int nseg, const uint8_t* pre
   const uint8_t* d_pb = reinterpret_cast<const uint8_t*>(d_off + nprefix + 1);
   PrefixOut po;
   II2_TRY(k5_prefix_search(d_segs, nseg, d_pb, d_off, nprefix, po, s));
-  std::unique_ptr<HostOwner> own(new HostOwner());
-  uint32_t* h_matched = nullptr;
-  II2_TRY(d2h(&o->values, po.values.p, (size_t)po.total, *own, s));
-  II2_TRY(d2h(&o->value_off, po.value_off.p, (size_t)nprefix + 1, *own, s));
-  II2_TRY(d2h(&h_matched, po.matched.p, (size_t)(nprefix ? nprefix : 1), *own, s));
-  II2_CUDA_TRY(cudaStreamSynchronize(s));
-  o->matched = own->alloc<uint8_t>((size_t)nprefix + 1);
-  if (!o->matched) return II2_ERR_NOMEM;
-  for (uint32_t i = 0; i < nprefix; i++) o->matched[i] = h_matched[i] ? 1 : 0;
-  o->n_prefixes = nprefix;
-  o->_owner = own.release();
-  return II2_OK;
+  return prefix_out_download(po, nprefix, o, s);
 }
 
 int ii2_prefix_search_dev(ii2_seg* const* segs, int nseg, const uint8_t* prefix_bytes,
@@ -1223,6 +1229,265 @@ int ii2_query_dev(ii2_seg* const* segs, int nseg, const ii2_query_batch* q, cons
 }
 
 void ii2_query_out_free(ii2_query_out* o) { host_out_free(o); }
+
+// ------------------------------------------------------------------ term patterns (K10)
+// Compiles pattern i into t (+ its search prefix into pre): II2_OK, II2_ERR_INVALID (grammar) or
+// II2_ERR_UNSUPPORTED (a limit), with the message in last error.
+static int pattern_compile(uint32_t i, const uint8_t* p, uint32_t n, uint8_t kind, uint32_t k,
+                           uint32_t plen, PatTab& t, std::string& pre) {
+  memset(&t, 0, sizeof(t));
+  t.kind = kind;
+  pre.clear();
+  if (kind == II2_PATTERN_FUZZY) {
+    if (plen > n) {
+      set_last_error("pattern %u: exact prefix of %u bytes is longer than the pattern (%u)", i, plen, n);
+      return II2_ERR_INVALID;
+    }
+    if (n > kPatMaxBytes || n - plen > kPatMaxFuzzy || k > kPatMaxEdits) {
+      set_last_error("pattern %u: fuzzy pattern of %u bytes after a %u-byte prefix, %u edits "
+                     "(max %u bytes, %u edits)", i, n - plen, plen, k, kPatMaxFuzzy, kPatMaxEdits);
+      return II2_ERR_UNSUPPORTED;
+    }
+    t.m = n - plen;
+    t.k = k;
+    t.skip = plen;
+    for (uint32_t j = 0; j < t.m; j++) t.mask[p[plen + j]] |= 1ull << j;
+    pre.assign(reinterpret_cast<const char*>(p), plen);
+    return II2_OK;
+  }
+  // GLOB: element e (0-based, items other than `*`) is NFA state e + 1
+  uint32_t e = 0;
+  bool literal_run = true;  // no metacharacter yet: the bytes so far are the literal prefix
+  auto set = [&](uint8_t c) {
+    if (e < kPatMaxGlob) t.mask[c] |= 1ull << (e + 1);
+  };
+  for (uint32_t j = 0; j < n;) {
+    const uint8_t c = p[j];
+    if (c == '*') {
+      if (e <= kPatMaxGlob) t.loop |= 1ull << e;
+      literal_run = false;
+      j++;
+    } else if (c == '?') {
+      for (int b = 0; b < 256; b++) set((uint8_t)b);
+      literal_run = false;
+      e++;
+      j++;
+    } else if (c == '[') {
+      uint32_t q = j + 1;
+      bool neg = false;
+      if (q < n && (p[q] == '!' || p[q] == '^')) {
+        neg = true;
+        q++;
+      }
+      bool in[256] = {};
+      bool first = true, closed = false;
+      while (q < n) {
+        if (p[q] == ']' && !first) {
+          closed = true;
+          break;
+        }
+        first = false;
+        uint8_t lo = p[q];
+        if (lo == '\\') {
+          if (++q >= n) break;
+          lo = p[q];
+        }
+        q++;
+        uint8_t hi = lo;
+        if (q + 1 < n && p[q] == '-' && p[q + 1] != ']') {
+          q++;
+          hi = p[q];
+          if (hi == '\\') {
+            if (++q >= n) break;
+            hi = p[q];
+          }
+          q++;
+        }
+        for (int b = lo; b <= hi; b++) in[b] = true;
+      }
+      if (!closed) {
+        set_last_error("pattern %u: `[` at byte %u has no closing `]`", i, j);
+        return II2_ERR_INVALID;
+      }
+      for (int b = 0; b < 256; b++)
+        if (in[b] != neg) set((uint8_t)b);
+      literal_run = false;
+      e++;
+      j = q + 1;
+    } else {
+      uint8_t lit = c;
+      if (c == '\\') {
+        if (j + 1 >= n) {
+          set_last_error("pattern %u ends with an escape `\\`", i);
+          return II2_ERR_INVALID;
+        }
+        lit = p[++j];
+      }
+      set(lit);
+      if (literal_run) pre.push_back((char)lit);
+      e++;
+      j++;
+    }
+  }
+  if (n > kPatMaxBytes || e > kPatMaxGlob) {
+    set_last_error("pattern %u: glob of %u bytes, %u elements (max %u bytes, %u elements)", i, n, e,
+                   kPatMaxBytes, kPatMaxGlob);
+    return II2_ERR_UNSUPPORTED;
+  }
+  t.accept = 1ull << e;
+  t.skip = (uint32_t)pre.size();
+  return II2_OK;
+}
+
+static int pattern_search_impl(ii2_seg* const* segs, int nseg, const ii2_pattern_batch* q,
+                               ii2_prefix_out* o, cudaStream_t s) {
+  ProfScope pipe_scope("pattern_total", s);
+  const uint32_t npat = q->npat;
+  if (!q->pat_off || (npat && !q->pat_kind)) {
+    set_last_error("pattern search: NULL batch array");
+    return II2_ERR_INVALID;
+  }
+  if (q->pat_off[0] != 0) return II2_ERR_INVALID;
+  for (uint32_t i = 0; i < npat; i++) {
+    if (q->pat_off[i + 1] < q->pat_off[i]) return II2_ERR_INVALID;
+    if (q->pat_kind[i] > II2_PATTERN_FUZZY) {
+      set_last_error("pattern %u has unknown kind %u", i, q->pat_kind[i]);
+      return II2_ERR_INVALID;
+    }
+    if (q->pat_kind[i] == II2_PATTERN_FUZZY && !q->max_edits) {
+      set_last_error("pattern search: fuzzy pattern %u without max_edits", i);
+      return II2_ERR_INVALID;
+    }
+  }
+  if (q->pat_off[npat] && !q->pat_bytes) return II2_ERR_INVALID;
+  for (int i = 0; i < nseg; i++)
+    if (!segs[i]) return II2_ERR_INVALID;
+  // compile every distinct pattern (grammar errors before limits)
+  std::vector<PatTab> tabs;
+  std::vector<std::string> pres;
+  std::vector<uint32_t> uid(npat);
+  int unsupported = II2_OK;
+  {
+    std::unordered_map<std::string, uint32_t> seen;
+    std::string key, pre;
+    PatTab t;
+    for (uint32_t i = 0; i < npat; i++) {
+      const uint32_t o0 = q->pat_off[i], n = q->pat_off[i + 1] - o0;
+      const uint8_t kind = q->pat_kind[i];
+      const uint32_t k = kind == II2_PATTERN_FUZZY ? q->max_edits[i] : 0;
+      const uint32_t plen = kind == II2_PATTERN_FUZZY && q->prefix_len ? q->prefix_len[i] : 0;
+      key.assign(reinterpret_cast<const char*>(&kind), 1);
+      key.append(reinterpret_cast<const char*>(&k), 4);
+      key.append(reinterpret_cast<const char*>(&plen), 4);
+      if (n) key.append(reinterpret_cast<const char*>(q->pat_bytes + o0), n);
+      auto it = seen.find(key);
+      if (it != seen.end()) {
+        uid[i] = it->second;
+        continue;
+      }
+      const int rc = pattern_compile(i, q->pat_bytes + o0, n, kind, k, plen, t, pre);
+      if (rc == II2_ERR_INVALID) return rc;
+      if (rc != II2_OK) {
+        if (unsupported == II2_OK) unsupported = rc;
+        continue;
+      }
+      uid[i] = (uint32_t)tabs.size();
+      seen.emplace(key, uid[i]);
+      tabs.push_back(t);
+      pres.push_back(pre);
+    }
+  }
+  if (unsupported != II2_OK) return unsupported;
+  if (nseg > kMaxSegs) {
+    set_last_error("%d segments in one call (max %d per pass)", nseg, kMaxSegs);
+    return II2_ERR_UNSUPPORTED;
+  }
+  if ((uint64_t)npat * (uint64_t)nseg >= (1ull << 32)) {
+    set_last_error("pattern search: %u patterns x %d segments exceed 2^32 pairs", npat, nseg);
+    return II2_ERR_UNSUPPORTED;
+  }
+  if (npat == 0 || nseg == 0) {  // nothing can match
+    PatternDev d = {};
+    d.k = nseg;
+    d.npat = npat;
+    PrefixOut po;
+    II2_TRY(k10_pattern_search(d, po, s));
+    return prefix_out_download(po, npat, o, s);
+  }
+  // internal order: every anchored pattern (one with a search prefix) is a group of its own, the
+  // unanchored ones share groups of kPatGroup (one scan of the dictionary per group)
+  const uint32_t nu = (uint32_t)tabs.size();
+  std::vector<uint32_t> order, pos(nu);
+  for (uint32_t u = 0; u < nu; u++)
+    if (!pres[u].empty()) order.push_back(u);
+  const uint32_t n_anchored = (uint32_t)order.size();
+  for (uint32_t u = 0; u < nu; u++)
+    if (pres[u].empty()) order.push_back(u);
+  for (uint32_t r = 0; r < nu; r++) pos[order[r]] = r;
+  std::vector<PatGroup> groups;
+  size_t pre_bytes = 0;
+  for (uint32_t r = 0; r < n_anchored; r++) {
+    const std::string& pr = pres[order[r]];
+    groups.push_back(PatGroup{r, 1, (uint32_t)pre_bytes, (uint32_t)pr.size()});
+    pre_bytes += pr.size();
+  }
+  for (uint32_t r = n_anchored; r < nu; r += kPatGroup)
+    groups.push_back(PatGroup{r, std::min(kPatGroup, nu - r), 0, 0});
+  const uint32_t ng = (uint32_t)groups.size();
+  // segment table, tables, groups, output map and prefix bytes through one pinned block and one copy
+  size_t cur = 0;
+  auto place = [&](size_t bytes) {
+    const size_t at = cur;
+    cur = (cur + bytes + 15) & ~(size_t)15;
+    return at;
+  };
+  const size_t o_segs = place(sizeof(SegDesc) * nseg);
+  const size_t o_tabs = place(sizeof(PatTab) * nu);
+  const size_t o_groups = place(sizeof(PatGroup) * ng);
+  const size_t o_uid = place(4 * (size_t)npat);
+  const size_t o_pre = place(pre_bytes);
+  PinnedBlock stage(cur);
+  if (!stage.p) return II2_ERR_NOMEM;
+  uint8_t* hb = static_cast<uint8_t*>(stage.p);
+  II2_TRY(seg_table(reinterpret_cast<SegDesc*>(hb + o_segs), segs, nseg));
+  PatTab* h_tabs = reinterpret_cast<PatTab*>(hb + o_tabs);
+  for (uint32_t r = 0; r < nu; r++) h_tabs[r] = tabs[order[r]];
+  if (ng) memcpy(hb + o_groups, groups.data(), sizeof(PatGroup) * ng);
+  uint32_t* h_uid = reinterpret_cast<uint32_t*>(hb + o_uid);
+  for (uint32_t i = 0; i < npat; i++) h_uid[i] = pos[uid[i]];
+  for (uint32_t r = 0; r < n_anchored; r++) {
+    const std::string& pr = pres[order[r]];
+    memcpy(hb + o_pre + groups[r].pre_off, pr.data(), pr.size());
+  }
+  DevBuf<uint8_t> d_stage;
+  II2_TRY(d_stage.alloc_scratch(cur, s, 32));
+  II2_CUDA_TRY(cudaMemcpyAsync(d_stage.p, stage.p, cur, cudaMemcpyHostToDevice, s));
+  uint8_t* db = d_stage.p;
+  PatternDev d;
+  d.segs = reinterpret_cast<const SegDesc*>(db + o_segs);
+  d.k = nseg;
+  d.tabs = reinterpret_cast<const PatTab*>(db + o_tabs);
+  d.nu = nu;
+  d.groups = reinterpret_cast<const PatGroup*>(db + o_groups);
+  d.ng = ng;
+  d.pre = db + o_pre;
+  d.uid = reinterpret_cast<const uint32_t*>(db + o_uid);
+  d.npat = npat;
+  PrefixOut po;
+  II2_TRY(k10_pattern_search(d, po, s));
+  return prefix_out_download(po, npat, o, s);
+}
+
+int ii2_pattern_search_dev(ii2_seg* const* segs, int nseg, const ii2_pattern_batch* q,
+                           ii2_prefix_out* out) {
+  if (!out) return II2_ERR_INVALID;
+  memset(out, 0, sizeof(*out));
+  if (!q || nseg < 0 || (nseg && !segs)) return II2_ERR_INVALID;
+  int dev = -1;
+  II2_TRY(handles_device(segs, nseg, nullptr, &dev));
+  II2_TRY(ctx_require_device(dev));
+  return run_on_stream(out, [&](cudaStream_t s) { return pattern_search_impl(segs, nseg, q, out, s); });
+}
 
 // ------------------------------------------------------------------ ingest batching
 static int ingest_impl(const ii2_doc_view* docs, int ndocs, const uint32_t* removed_sorted,
@@ -2009,6 +2274,21 @@ int ii2_query(const ii2_seg_view* segs, int nseg, const ii2_query_batch* q,
   if (removed_sorted) II2_TRY(ii2_removed_upload(removed_sorted, nrem, &rem));
   std::unique_ptr<ii2_removed> rem_guard(rem);
   return ii2_query_dev(list.v.data(), nseg, q, rem, out);
+}
+
+int ii2_pattern_search(const ii2_seg_view* segs, int nseg, const ii2_pattern_batch* q,
+                       ii2_prefix_out* out) {
+  if (!out) return II2_ERR_INVALID;
+  memset(out, 0, sizeof(*out));
+  if (!q || nseg < 0 || (nseg && !segs)) return II2_ERR_INVALID;
+  II2_TRY(ctx_require());
+  SegList list;
+  for (int i = 0; i < nseg; i++) {
+    ii2_seg* g = nullptr;
+    II2_TRY(ii2_seg_upload(&segs[i], &g));
+    list.v.push_back(g);
+  }
+  return ii2_pattern_search_dev(list.v.data(), nseg, q, out);
 }
 
 }  // extern "C"

@@ -24,15 +24,6 @@ namespace ii2 {
 
 namespace {
 
-// bytes.HasPrefix(t, p)
-__device__ __forceinline__ bool has_prefix(const uint8_t* t, uint32_t nt, const uint8_t* p,
-                                           uint32_t np) {
-  if (nt < np) return false;
-  for (uint32_t i = 0; i < np; i++)
-    if (t[i] != p[i]) return false;
-  return true;
-}
-
 struct K5Args {
   const SegDesc* segs;
   int k;
@@ -48,9 +39,7 @@ struct K5Args {
   uint32_t* flags;     // [0] = a slice longer than 2^32-1 postings
 };
 
-// One WARP per (prefix, segment): lo = first term >= p (every term with prefix p is >= p),
-// hi = first term at or after lo that does not start with p (terms with a common prefix are
-// contiguous in bytes.Compare order); both are 32-way searches (warp_partition_point).  An exact
+// One WARP per (prefix, segment): the window of the prefix (prefix_window_lo / _hi).  An exact
 // TERM item's window is [lo, lo + (term lo == p)).
 __global__ void __launch_bounds__(256) k5_windows(const K5Args a) {
   const uint64_t id = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -60,10 +49,7 @@ __global__ void __launch_bounds__(256) k5_windows(const K5Args a) {
   const SegDesc sd = a.segs[s];
   const uint8_t* pb = a.pbytes + a.poff[p];
   const uint32_t pn = a.poff[p + 1] - a.poff[p];
-  const uint32_t lo = warp_partition_point(0u, sd.n, [&](uint32_t i) {
-    const uint32_t o = __ldg(sd.toff + i), n = __ldg(sd.toff + i + 1) - o;
-    return term_compare(sd.tb + o, n, pb, pn) < 0;
-  });
+  const uint32_t lo = prefix_window_lo(sd, pb, pn);
   uint32_t hi;
   if (a.kind && a.kind[p] == II2_ATOM_TERM) {  // uniform inside the warp
     uint32_t eq = 0;
@@ -73,10 +59,7 @@ __global__ void __launch_bounds__(256) k5_windows(const K5Args a) {
     }
     hi = lo + eq;
   } else {
-    hi = warp_partition_point(lo, sd.n, [&](uint32_t i) {
-      const uint32_t o = __ldg(sd.toff + i), n = __ldg(sd.toff + i + 1) - o;
-      return has_prefix(sd.tb + o, n, pb, pn);
-    });
+    hi = prefix_window_hi(sd, lo, pb, pn);
   }
   if (lane_id() != 0) return;
   const uint64_t p0 = sd.poff[lo], p1 = sd.poff[hi];
@@ -191,32 +174,41 @@ int k5_prefix_search(const SegDesc* d_segs, int k, const uint8_t* d_pbytes, cons
     ProfScope scope("k5_union", s);
     II2_TRY(k2_large_run(la, np, tmp, enc, s));
   }
+  return place_unions(recs.p, np, out, flags.p,
+                      "prefix search: one segment holds more than 2^32-1 postings under a prefix",
+                      "k5_place", h_value_off, s);
+}
+
+int place_unions(const GroupRec* recs, uint32_t np, PrefixOut& out, const uint32_t* d_flag,
+                 const char* flag_msg, const char* place_name, uint64_t* h_value_off,
+                 cudaStream_t s) {
   uint64_t* h = pinned_scratch();
   if (!h) return II2_ERR_NOMEM;
   DevBuf<uint64_t> d_tot;
   II2_TRY(d_tot.alloc_scratch(1, s));
-  k5_counts<<<div_up((uint64_t)np + 1, 256), 256, 0, s>>>(recs.p, np, out.value_off.p);
+  k5_counts<<<div_up((uint64_t)np + 1, 256), 256, 0, s>>>(recs, np, out.value_off.p);
   II2_LAUNCHED();
   II2_TRY(exclusive_scan_u64(out.value_off.p, (uint64_t)np + 1, d_tot.p, s));
   II2_TRY(small_copy(h, d_tot.p, 8, s));
-  II2_TRY(small_copy(h + 1, flags.p, 8, s));
+  h[1] = 0;
+  if (d_flag) II2_TRY(small_copy(h + 1, d_flag, 8, s));
   if (h_value_off)
     II2_CUDA_TRY(cudaMemcpyAsync(h_value_off, out.value_off.p, ((size_t)np + 1) * 8,
                                  cudaMemcpyDeviceToHost, s));
   II2_CUDA_TRY(cudaStreamSynchronize(s));
   if ((uint32_t)h[1]) {
-    set_last_error("prefix search: one segment holds more than 2^32-1 postings under a prefix");
+    set_last_error("%s", flag_msg);
     return II2_ERR_UNSUPPORTED;
   }
   out.total = h[0];
   II2_TRY(out.values.alloc((size_t)out.total, s));
   if (out.total) {
-    ProfScope scope("k5_place", s);
+    ProfScope scope(place_name, s);
     const unsigned gx = (unsigned)std::max<uint64_t>(
         1, std::min<uint64_t>(1024, (out.total / np + 2047) / 2048));
     for (uint32_t y0 = 0; y0 < np; y0 += 32768) {
       const uint32_t ny = std::min<uint32_t>(32768, np - y0);
-      k5_place<<<dim3(gx, ny), 256, 0, s>>>(recs.p + y0, out.value_off.p + y0, out.values.p);
+      k5_place<<<dim3(gx, ny), 256, 0, s>>>(recs + y0, out.value_off.p + y0, out.values.p);
       II2_LAUNCHED();
     }
   }

@@ -522,6 +522,75 @@ class Engine:
                                            removed.h if removed else None, C.byref(out)), "query_dev")
         return self._query_result(out)
 
+    # ---- term patterns: wildcard (glob) and fuzzy matching --------------------------------
+    @staticmethod
+    def _pattern_args(patterns: list) -> tuple[A.PatternBatch, list]:
+        """Packs patterns into ii2_pattern_batch: `bytes` is a glob, (bytes, max_edits,
+        prefix_len) a fuzzy pattern.  Returns the struct and the arrays it points into (keep
+        them alive for the call)."""
+        pats, kinds, edits, plens = [], [], [], []
+        for p in patterns:
+            if isinstance(p, (bytes, bytearray)):
+                pats.append(bytes(p))
+                kinds.append(A.II2_PATTERN_GLOB)
+                edits.append(0)
+                plens.append(0)
+            else:
+                q, k, plen = p
+                pats.append(bytes(q))
+                kinds.append(A.II2_PATTERN_FUZZY)
+                edits.append(int(k))
+                plens.append(int(plen))
+        blob, off = Engine._prefix_args(pats)
+        # one spare element each: no array is ever empty
+        kind = np.array(kinds + [0], dtype=np.uint8)
+        med = np.array(edits + [0], dtype=np.uint8)
+        pl = np.array(plens + [0], dtype=np.uint32)
+        b = A.PatternBatch()
+        b.pat_bytes = A.np_ptr(blob, A.u8p)
+        b.pat_off = A.np_ptr(off, A.u32p)
+        b.pat_kind = A.np_ptr(kind, A.u8p)
+        b.max_edits = A.np_ptr(med, A.u8p)
+        b.prefix_len = A.np_ptr(pl, A.u32p)
+        b.npat = len(pats)
+        return b, [blob, off, kind, med, pl]
+
+    def _pattern_result(self, out: A.PrefixOut) -> list[np.ndarray | None]:
+        try:
+            n = int(out.n_prefixes)
+            matched = A.from_ptr(out.matched, n, np.uint8)
+            off = A.from_ptr(out.value_off, n + 1, np.uint64)
+            vals = A.from_ptr(out.values, int(off[-1]) if n else 0, np.uint32)
+        finally:
+            self.lib.ii2_prefix_out_free(C.byref(out))
+        return [vals[int(off[i]):int(off[i + 1])] if matched[i] else None for i in range(n)]
+
+    def pattern_search(self, segs: list[FlatSegment], patterns: list) -> list[np.ndarray | None]:
+        """pattern_search_dev over host views (uploaded for the call)."""
+        arr = views_array(segs)
+        batch, keep = self._pattern_args(patterns)
+        out = A.PrefixOut()
+        self._check(self.lib.ii2_pattern_search(arr, len(segs), C.byref(batch), C.byref(out)),
+                    "pattern_search")
+        return self._pattern_result(out)
+
+    def pattern_search_dev_out(self, segs: list[DeviceSegment], patterns: list) -> A.PrefixOut:
+        """ii2_pattern_search_dev's raw output (a prefix output: input of prefix_gather_devices,
+        with the pattern list in place of the prefixes); free it with prefix_out_free."""
+        batch, keep = self._pattern_args(patterns)
+        out = A.PrefixOut()
+        self._check(self.lib.ii2_pattern_search_dev(self._handles(segs), len(segs), C.byref(batch),
+                                                    C.byref(out)), "pattern_search_dev")
+        return out
+
+    def pattern_search_dev(self, segs: list[DeviceSegment], patterns: list) -> list[np.ndarray | None]:
+        """Wildcard and fuzzy term matching over resident segments in one call on their device.
+        A pattern is `bytes` (a glob: `*`, `?`, `[...]`, `\\x`) or (bytes, max_edits, prefix_len)
+        (terms within max_edits byte edits of it whose first prefix_len bytes are equal).  Aligned
+        with `patterns`: the sorted-unique values of every matching term, or None when no term
+        matches."""
+        return self._pattern_result(self.pattern_search_dev_out(segs, patterns))
+
     # ---- codec -----------------------------------------------------------------------
     def intcomp_encode_batch(self, post: np.ndarray, post_off: np.ndarray):
         post = np.ascontiguousarray(post, dtype=np.uint32)
