@@ -10,6 +10,8 @@
         shapes, against lookup_dev + prefix_search_dev + host numpy set operations
   pattern  glob and fuzzy term patterns (ii2_pattern_search_dev) on the C3 workload, 1 .. 256 per
         call in four groups, against read_range_dev + download + host filter and union
+  pattern_terms  the terms each pattern matches (ii2_pattern_terms_dev) for the same four groups and
+        `*`, beside ii2_pattern_search_dev on the same patterns, checked against the host answer
   multidev  one process over every visible GPU (Engine(devices=...)): weak-scaling compaction from
         one host thread per device, a 1 % read partitioned over the devices + ii2_read_gather_devices,
         and ii2_prefix_gather_devices of the prefix batch; each checked against one device
@@ -314,6 +316,18 @@ def _host_patterns(terms_blob, starts, lists, pats):
     return out
 
 
+def _pattern_groups(terms):
+    """The four pattern groups of --which pattern and pattern_terms, 256 patterns each."""
+    rng = np.random.default_rng(10)
+    picks = [terms[int(i)] for i in rng.integers(0, len(terms), size=256)]
+    return {
+        "glob_anchored": [t[:3] + b"*" + t[5:7] + b"*" for t in picks],
+        "glob_unanchored": [b"*" + t[3:6] + b"*" for t in picks],
+        "fuzzy_p0": [(t[:-1] + b"q", 1 + i % 2, 0) for i, t in enumerate(picks)],
+        "fuzzy_p2": [(t[:-1] + b"q", 1 + i % 2, 2) for i, t in enumerate(picks)],
+    }
+
+
 def pattern(eng, a):
     """Wildcard and fuzzy term patterns (ii2_pattern_search_dev, results downloaded) on the
     resident C3 workload (256 segments), batches of 1 / 16 / 256 patterns in four groups: anchored
@@ -355,14 +369,7 @@ def pattern(eng, a):
             b += int(ibytes[hi] - ibytes[lo] + 4 * (inst[hi] - inst[lo]))
         return b + (unanchored + 15) // 16 * full
 
-    rng = np.random.default_rng(10)
-    picks = [terms[int(i)] for i in rng.integers(0, n, size=256)]
-    groups = {
-        "glob_anchored": [t[:3] + b"*" + t[5:7] + b"*" for t in picks],
-        "glob_unanchored": [b"*" + t[3:6] + b"*" for t in picks],
-        "fuzzy_p0": [(t[:-1] + b"q", 1 + i % 2, 0) for i, t in enumerate(picks)],
-        "fuzzy_p2": [(t[:-1] + b"q", 1 + i % 2, 2) for i, t in enumerate(picks)],
-    }
+    groups = _pattern_groups(terms)
     host_data = None
     rows = []
     for gname, allp in groups.items():
@@ -421,6 +428,99 @@ def pattern(eng, a):
         s.release()
     print(json.dumps({"config": "term patterns (ii2_pattern_search_dev, results downloaded) vs "
                                 "read_range_dev + download + host filter and union", "cards": card,
+                      "terms": a.terms, "postings": w.postings_in, "term_instances": w.term_instances,
+                      "results": rows}))
+
+
+def pattern_terms(eng, a):
+    """The terms each pattern matches (ii2_pattern_terms_dev, results downloaded) on the resident
+    C3 workload (256 segments): the four groups of --which pattern at 1 / 16 / 256 patterns, and
+    `*` (every distinct term of the dictionary).  Each batch is timed beside ii2_pattern_search_dev
+    on the same patterns (both as raw C-ABI calls into pinned memory, no Python conversion) and
+    checked against the host answer from the generator's dictionary: a regex scan of the
+    newline-joined terms for globs, the numpy edit-distance program of tests/test_gpu_pattern.py
+    over the length-compatible candidates for fuzzy patterns, instance and posting counts from the
+    generator's segments."""
+    import ctypes as C
+    import re
+
+    from inverted_index_2_b200 import _abi as A
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    from test_gpu_pattern import glob_regex, levenshtein
+    card = _card()
+    w = synth.make_workload(a.terms, 256, a.postings, seed=0xC3, presence=0.125)
+    dsegs = [eng.upload(s) for s in w.segments]
+    n = len(w.term_off) - 1
+    terms = [synth.term_at(w.term_bytes, w.term_off, i) for i in range(n)]  # ascending
+    tlen = np.array([len(t) for t in terms], dtype=np.int64)
+    inst = np.zeros(n, dtype=np.int64)
+    post = np.zeros(n, dtype=np.int64)
+    for seg, ids in zip(w.segments, w.seg_term_ids):
+        np.add.at(inst, ids, 1)
+        np.add.at(post, ids, np.diff(seg.post_off).astype(np.int64))
+    joined = b"\n".join(terms)  # C3 terms are letters only
+    starts = np.cumsum(np.concatenate([[0], tlen[:-1] + 1]))
+
+    def host(p):
+        if isinstance(p, bytes):
+            body = glob_regex(p)[0].pattern.replace(b".", b"[^\n]")  # a term never spans a line
+            hits = [m.start() for m in re.finditer(rb"(?m)^(?:" + body + rb")$", joined)]
+            ids = np.searchsorted(starts, np.array(hits, dtype=np.int64))
+            dist = np.zeros(len(ids), dtype=np.int64)
+        else:
+            q, k, plen = p
+            ids = np.nonzero(np.abs(tlen - len(q)) <= k)[0]
+            if plen:
+                ids = np.array([i for i in ids if terms[i][:plen] == q[:plen]], dtype=np.int64)
+            dist = levenshtein([terms[i][plen:] for i in ids], q[plen:]) if len(ids) else np.zeros(0)
+            ids, dist = ids[dist <= k], dist[dist <= k]
+        keep = inst[ids] > 0
+        ids, dist = ids[keep], dist[keep]
+        return [(terms[i], int(inst[i]), int(post[i]), int(d)) for i, d in zip(ids, dist)]
+
+    handles = eng._handles(dsegs)
+
+    def raw_terms(pats):
+        batch, keep = eng._pattern_args(pats)
+        out = A.TermsOut()
+        eng._check(eng.lib.ii2_pattern_terms_dev(handles, len(dsegs), C.byref(batch), C.byref(out)),
+                   "pattern_terms_dev")
+        return out
+
+    groups = _pattern_groups(terms)
+    groups["star"] = [b"*"]
+    rows = []
+    for gname, allp in groups.items():
+        for q in ((1,) if gname == "star" else (1, 16, 256)):
+            pats = allp[:q]
+
+            def call():
+                eng.lib.ii2_terms_out_free(C.byref(raw_terms(pats)))
+
+            def search():
+                eng.prefix_out_free(eng.pattern_search_dev_out(dsegs, pats))
+            reps = 20 if q <= 16 and gname != "star" else 5
+            med, p99 = timed(call, reps)
+            smed, _ = timed(search, reps)
+            eng.prof_enable(True)
+            call()
+            phases = {p["name"]: round(1e3 * p["ms"] / max(1, p["count"]), 1) for p in eng.prof_read()}
+            eng.prof_enable(False)
+            got = eng._terms_result(raw_terms(pats))
+            ok = all(g == host(p) for g, p in zip(got, pats))
+            row = {"group": gname, "patterns": q, "median_us": 1e6 * med, "p99_us": 1e6 * p99,
+                   "search_median_us": 1e6 * smed, "terms_over_search": med / smed,
+                   "terms_out": int(sum(len(g) for g in got)),
+                   "instances_out": int(sum(x[1] for g in got for x in g)),
+                   "phase_us": phases, "verified": bool(ok)}
+            rows.append(row)
+            print(json.dumps(row), file=sys.stderr, flush=True)
+            if not ok:
+                raise SystemExit(f"pattern_terms: {gname} x {q} differs from the host answers")
+    for s in dsegs:
+        s.release()
+    print(json.dumps({"config": "pattern terms (ii2_pattern_terms_dev, results downloaded) beside "
+                                "ii2_pattern_search_dev on the same patterns", "cards": card,
                       "terms": a.terms, "postings": w.postings_in, "term_instances": w.term_instances,
                       "results": rows}))
 
@@ -723,25 +823,28 @@ def main():
     ap.add_argument("--terms", type=int, default=1_000_000)
     ap.add_argument("--postings", type=int, default=100_000_000)
     a = ap.parse_args()
-    if "multidev" in a.which:  # binds every visible device: a process of its own
+    which = a.which.split(",")
+    if "multidev" in which:  # binds every visible device: a process of its own
         multidev(a)
         return
     from inverted_index_2_b200.engine import Engine
     eng = Engine(0)
-    if "c1" in a.which:
+    if "c1" in which:
         c1(eng, a)
-    if "c3" in a.which:
+    if "c3" in which:
         c3(eng, a)
-    if "c4" in a.which:
+    if "c4" in which:
         c4(eng, a)
-    if "prefix" in a.which:
+    if "prefix" in which:
         prefix(eng, a)
-    if "lookup" in a.which:
+    if "lookup" in which:
         lookup(eng, a)
-    if "query" in a.which:
+    if "query" in which:
         query(eng, a)
-    if "pattern" in a.which:
+    if "pattern" in which:
         pattern(eng, a)
+    if "pattern_terms" in which:
+        pattern_terms(eng, a)
 
 
 if __name__ == "__main__":

@@ -437,6 +437,49 @@ int ii2_pattern_search_dev(ii2_seg* const* segs, int nseg, const ii2_pattern_bat
 int ii2_pattern_search(const ii2_seg_view* segs, int nseg, const ii2_pattern_batch* q,
                        ii2_prefix_out* out);
 
+/* ---- the terms a pattern matches: the keys vellum's fst.Search(automaton, ...)
+ *      yields, for every pattern of a batch ------------------------------------ */
+typedef struct ii2_terms_out {
+  uint64_t n_patterns;
+  uint64_t n_terms;            /* over all patterns                                        */
+  uint64_t* pattern_term_off;  /* n_patterns + 1: pattern i's terms are [off[i], off[i+1]) */
+  uint8_t* term_bytes;         /* term j = term_bytes[term_off[j] .. term_off[j+1])        */
+  uint64_t* term_off;          /* n_terms + 1                                              */
+  uint32_t* segments;          /* n_terms: term instances in the call's segment list       */
+  uint64_t* postings;          /* n_terms: sum of the stored lengths of those lists        */
+  uint8_t* distance;           /* n_terms: FUZZY: Levenshtein distance; GLOB: 0            */
+  void* _owner;
+} ii2_terms_out;
+
+/* The same batch, grammar, limits and error codes as ii2_pattern_search_dev (all
+ * checked before any launch), but the output is the matching TERMS rather than the
+ * union of their lists:
+ *   - Pattern i's terms are the distinct terms that match it in at least one
+ *     segment, ascending by bytes.Compare.  A term whose lists are all empty is
+ *     included (postings = 0), so pattern i has terms exactly when
+ *     ii2_pattern_search_dev sets matched[i] for the same batch.
+ *   - segments: the term's instances over the call's segment list (a handle passed
+ *     twice counts twice).
+ *   - postings: the sum of the stored lengths of those lists, duplicates counted and
+ *     nothing unioned: an upper bound on the term's document count.  The exact
+ *     values are one ii2_lookup_dev key, or one TERM atom of ii2_query_dev, away.
+ *   - distance: FUZZY: the byte Levenshtein distance between t[P..] and q[P..]
+ *     (at most max_edits); GLOB: 0.
+ *   - Patterns may repeat (each position gets its own copy) and come in any order.
+ *     npat == 0 or nseg == 0 gives empty results.  No removed filter (reads never
+ *     filter, quirk Q2).
+ * ii2_pattern_terms_dev runs on the device of its handles (handles of two devices:
+ * II2_ERR_INVALID); ii2_pattern_terms uploads the views to the device the thread
+ * selected.  Outputs are pinned host memory; free them with ii2_terms_out_free.  On
+ * error *out is zeroed.  II2_ERR_UNSUPPORTED, besides the limits of pattern search
+ * (the 2^32 postings limit of one union does not apply): the call's matched term
+ * instances, or their term bytes, reach 2^32. */
+int ii2_pattern_terms_dev(ii2_seg* const* segs, int nseg, const ii2_pattern_batch* q,
+                          ii2_terms_out* out);
+int ii2_pattern_terms(const ii2_seg_view* segs, int nseg, const ii2_pattern_batch* q,
+                      ii2_terms_out* out);
+void ii2_terms_out_free(ii2_terms_out* out);
+
 /* ---- cross-shard exchange: one process per GPU, contiguous shard-key ranges per
  *      rank (shardKey, shard.go:362-378), NCCL over NVLink --------------------
  * Compaction needs no exchange (shards never interact, shard.go:19-20).  Reads

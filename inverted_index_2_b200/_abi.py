@@ -151,6 +151,20 @@ class PatternBatch(C.Structure):
     ]
 
 
+class TermsOut(C.Structure):
+    _fields_ = [
+        ("n_patterns", C.c_uint64),
+        ("n_terms", C.c_uint64),
+        ("pattern_term_off", u64p),
+        ("term_bytes", u8p),
+        ("term_off", u64p),
+        ("segments", u32p),
+        ("postings", u64p),
+        ("distance", u8p),
+        ("_owner", C.c_void_p),
+    ]
+
+
 class FstTerms(C.Structure):
     _fields_ = [
         ("n_terms", C.c_uint64),
@@ -249,6 +263,11 @@ PROTOTYPES = {
                                          C.POINTER(PrefixOut)]),
     "ii2_pattern_search": (C.c_int, [C.POINTER(SegView), C.c_int, C.POINTER(PatternBatch),
                                      C.POINTER(PrefixOut)]),
+    "ii2_pattern_terms_dev": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.POINTER(PatternBatch),
+                                        C.POINTER(TermsOut)]),
+    "ii2_pattern_terms": (C.c_int, [C.POINTER(SegView), C.c_int, C.POINTER(PatternBatch),
+                                    C.POINTER(TermsOut)]),
+    "ii2_terms_out_free": (None, [C.POINTER(TermsOut)]),
     "ii2_comm_unique_id": (C.c_int, [u8p]),
     "ii2_comm_init": (C.c_int, [u8p, C.c_int, C.c_int]),
     "ii2_comm_info": (C.c_int, [C.POINTER(C.c_int), C.POINTER(C.c_int)]),

@@ -1339,10 +1339,16 @@ static int pattern_compile(uint32_t i, const uint8_t* p, uint32_t n, uint8_t kin
   return II2_OK;
 }
 
-static int pattern_search_impl(ii2_seg* const* segs, int nseg, const ii2_pattern_batch* q,
-                               ii2_prefix_out* o, cudaStream_t s) {
-  ProfScope pipe_scope("pattern_total", s);
+// The host half both pattern calls share: checks the batch (every error before any launch),
+// compiles the distinct patterns, groups them and stages the segment table, the tables, the groups,
+// the output map and the prefix bytes on the device (d points into d_stage).  npat == 0 or
+// nseg == 0 leaves d without patterns (d.nu == d.ng == 0).
+static int pattern_prepare(ii2_seg* const* segs, int nseg, const ii2_pattern_batch* q,
+                           PatternDev& d, DevBuf<uint8_t>& d_stage, cudaStream_t s) {
   const uint32_t npat = q->npat;
+  d = PatternDev{};
+  d.k = nseg;
+  d.npat = npat;
   if (!q->pat_off || (npat && !q->pat_kind)) {
     set_last_error("pattern search: NULL batch array");
     return II2_ERR_INVALID;
@@ -1406,14 +1412,7 @@ static int pattern_search_impl(ii2_seg* const* segs, int nseg, const ii2_pattern
     set_last_error("pattern search: %u patterns x %d segments exceed 2^32 pairs", npat, nseg);
     return II2_ERR_UNSUPPORTED;
   }
-  if (npat == 0 || nseg == 0) {  // nothing can match
-    PatternDev d = {};
-    d.k = nseg;
-    d.npat = npat;
-    PrefixOut po;
-    II2_TRY(k10_pattern_search(d, po, s));
-    return prefix_out_download(po, npat, o, s);
-  }
+  if (npat == 0 || nseg == 0) return II2_OK;  // nothing can match
   // internal order: every anchored pattern (one with a search prefix) is a group of its own, the
   // unanchored ones share groups of kPatGroup (one scan of the dictionary per group)
   const uint32_t nu = (uint32_t)tabs.size();
@@ -1459,23 +1458,28 @@ static int pattern_search_impl(ii2_seg* const* segs, int nseg, const ii2_pattern
     const std::string& pr = pres[order[r]];
     memcpy(hb + o_pre + groups[r].pre_off, pr.data(), pr.size());
   }
-  DevBuf<uint8_t> d_stage;
   II2_TRY(d_stage.alloc_scratch(cur, s, 32));
   II2_CUDA_TRY(cudaMemcpyAsync(d_stage.p, stage.p, cur, cudaMemcpyHostToDevice, s));
   uint8_t* db = d_stage.p;
-  PatternDev d;
   d.segs = reinterpret_cast<const SegDesc*>(db + o_segs);
-  d.k = nseg;
   d.tabs = reinterpret_cast<const PatTab*>(db + o_tabs);
   d.nu = nu;
   d.groups = reinterpret_cast<const PatGroup*>(db + o_groups);
   d.ng = ng;
   d.pre = db + o_pre;
   d.uid = reinterpret_cast<const uint32_t*>(db + o_uid);
-  d.npat = npat;
+  return II2_OK;
+}
+
+static int pattern_search_impl(ii2_seg* const* segs, int nseg, const ii2_pattern_batch* q,
+                               ii2_prefix_out* o, cudaStream_t s) {
+  ProfScope pipe_scope("pattern_total", s);
+  PatternDev d;
+  DevBuf<uint8_t> d_stage;
+  II2_TRY(pattern_prepare(segs, nseg, q, d, d_stage, s));
   PrefixOut po;
   II2_TRY(k10_pattern_search(d, po, s));
-  return prefix_out_download(po, npat, o, s);
+  return prefix_out_download(po, q->npat, o, s);
 }
 
 int ii2_pattern_search_dev(ii2_seg* const* segs, int nseg, const ii2_pattern_batch* q,
@@ -1488,6 +1492,43 @@ int ii2_pattern_search_dev(ii2_seg* const* segs, int nseg, const ii2_pattern_bat
   II2_TRY(ctx_require_device(dev));
   return run_on_stream(out, [&](cudaStream_t s) { return pattern_search_impl(segs, nseg, q, out, s); });
 }
+
+static int pattern_terms_impl(ii2_seg* const* segs, int nseg, const ii2_pattern_batch* q,
+                              ii2_terms_out* o, cudaStream_t s) {
+  ProfScope pipe_scope("pattern_terms_total", s);
+  PatternDev d;
+  DevBuf<uint8_t> d_stage;
+  II2_TRY(pattern_prepare(segs, nseg, q, d, d_stage, s));
+  TermsOut to;
+  II2_TRY(k10_pattern_terms(d, to, s));
+  const uint32_t npat = q->npat;
+  const size_t n = (size_t)to.n_terms;
+  std::unique_ptr<HostOwner> own(new HostOwner());
+  II2_TRY(d2h(&o->pattern_term_off, to.pattern_term_off.p, (size_t)npat + 1, *own, s));
+  II2_TRY(d2h(&o->term_bytes, to.tb.p, (size_t)to.n_bytes, *own, s));
+  II2_TRY(d2h(&o->term_off, to.toff.p, n + 1, *own, s));
+  II2_TRY(d2h(&o->segments, to.segments.p, n, *own, s));
+  II2_TRY(d2h(&o->postings, to.postings.p, n, *own, s));
+  II2_TRY(d2h(&o->distance, to.distance.p, n, *own, s));
+  II2_CUDA_TRY(cudaStreamSynchronize(s));
+  o->n_patterns = npat;
+  o->n_terms = n;
+  o->_owner = own.release();
+  return II2_OK;
+}
+
+int ii2_pattern_terms_dev(ii2_seg* const* segs, int nseg, const ii2_pattern_batch* q,
+                          ii2_terms_out* out) {
+  if (!out) return II2_ERR_INVALID;
+  memset(out, 0, sizeof(*out));
+  if (!q || nseg < 0 || (nseg && !segs)) return II2_ERR_INVALID;
+  int dev = -1;
+  II2_TRY(handles_device(segs, nseg, nullptr, &dev));
+  II2_TRY(ctx_require_device(dev));
+  return run_on_stream(out, [&](cudaStream_t s) { return pattern_terms_impl(segs, nseg, q, out, s); });
+}
+
+void ii2_terms_out_free(ii2_terms_out* o) { host_out_free(o); }
 
 // ------------------------------------------------------------------ ingest batching
 static int ingest_impl(const ii2_doc_view* docs, int ndocs, const uint32_t* removed_sorted,
@@ -2289,6 +2330,21 @@ int ii2_pattern_search(const ii2_seg_view* segs, int nseg, const ii2_pattern_bat
     list.v.push_back(g);
   }
   return ii2_pattern_search_dev(list.v.data(), nseg, q, out);
+}
+
+int ii2_pattern_terms(const ii2_seg_view* segs, int nseg, const ii2_pattern_batch* q,
+                      ii2_terms_out* out) {
+  if (!out) return II2_ERR_INVALID;
+  memset(out, 0, sizeof(*out));
+  if (!q || nseg < 0 || (nseg && !segs)) return II2_ERR_INVALID;
+  II2_TRY(ctx_require());
+  SegList list;
+  for (int i = 0; i < nseg; i++) {
+    ii2_seg* g = nullptr;
+    II2_TRY(ii2_seg_upload(&segs[i], &g));
+    list.v.push_back(g);
+  }
+  return ii2_pattern_terms_dev(list.v.data(), nseg, q, out);
 }
 
 }  // extern "C"

@@ -23,4 +23,13 @@ int k7_ingest_sort(const uint8_t* d_tb, const uint32_t* d_toff, const uint64_t* 
                    const uint64_t* h_doff, const uint32_t* d_vals, int D, uint64_t N, uint64_t TB,
                    IngestOut& out, cudaStream_t s);
 
+// K7's segmented sort on its own: the N terms d_tb / d_toff[N+1] of D documents (d_doff[D+1] on
+// the device, maxL = the longest document) ordered by bytes.Compare inside every document.
+// idx[N] receives the term indices in sorted order; keep[N+1] / klen[N+1] = 1 / the term's byte
+// length for the first record of every distinct term of a document, 0 elsewhere (unscanned).
+// Queues the work on s; temporaries come from the calling thread's scratch arena.
+int k7_sort_distinct(const uint8_t* d_tb, const uint32_t* d_toff, const uint64_t* d_doff, int D,
+                     uint64_t N, uint64_t maxL, uint32_t* idx, uint64_t* keep, uint64_t* klen,
+                     cudaStream_t s);
+
 }  // namespace ii2

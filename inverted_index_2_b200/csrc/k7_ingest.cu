@@ -237,6 +237,36 @@ __global__ void __launch_bounds__(256) k7_emit(const K7Args a, const K7Emit e) {
   }
 }
 
+// sort every document's records by bytes.Compare of their terms: a.hi / a.lo / a.idx hold the
+// sorted records afterwards (maxL = the longest document)
+int k7_sort(const K7Args& a, uint64_t maxL, cudaStream_t s) {
+  if (!a.n) return II2_OK;
+  ProfScope scope("k7_sort", s);
+  k7_keys<<<div_up(a.n, 256), 256, 0, s>>>(a);
+  II2_LAUNCHED();
+  for (int y0 = 0; y0 < a.d; y0 += 32768) {  // grid.y limit
+    const int ny = std::min(32768, a.d - y0);
+    K7Args b = a;
+    b.doff += y0;
+    const unsigned gx = (unsigned)std::max<uint64_t>(
+        1, std::min<uint64_t>((maxL + K7_TILE - 1) / K7_TILE, 2048));
+    const dim3 grid(gx, ny);
+    k7_tile_sort<<<grid, K7_THREADS, 0, s>>>(b);
+    II2_LAUNCHED();
+    for (uint64_t kk = 2ull * K7_TILE; (kk >> 1) < maxL; kk <<= 1) {
+      k7_stage<<<grid, 256, 0, s>>>(b, kk, 0);
+      II2_LAUNCHED();
+      for (uint64_t j = kk >> 2; j >= K7_TILE; j >>= 1) {
+        k7_stage<<<grid, 256, 0, s>>>(b, kk, j);
+        II2_LAUNCHED();
+      }
+      k7_tile_merge<<<grid, K7_THREADS, 0, s>>>(b, kk);
+      II2_LAUNCHED();
+    }
+  }
+  return II2_OK;
+}
+
 }  // namespace
 
 int k7_ingest_sort(const uint8_t* d_tb, const uint32_t* d_toff, const uint64_t* d_doff,
@@ -266,31 +296,7 @@ int k7_ingest_sort(const uint8_t* d_tb, const uint32_t* d_toff, const uint64_t* 
   a.d = D;
   uint64_t maxL = 0;
   for (int d = 0; d < D; d++) maxL = std::max(maxL, h_doff[d + 1] - h_doff[d]);
-  if (N) {
-    ProfScope scope("k7_sort", s);
-    k7_keys<<<div_up(N, 256), 256, 0, s>>>(a);
-    II2_LAUNCHED();
-    for (int y0 = 0; y0 < D; y0 += 32768) {  // grid.y limit (D <= 1024 today)
-      const int ny = std::min(32768, D - y0);
-      K7Args b = a;
-      b.doff += y0;
-      const unsigned gx = (unsigned)std::max<uint64_t>(
-          1, std::min<uint64_t>((maxL + K7_TILE - 1) / K7_TILE, 2048));
-      const dim3 grid(gx, ny);
-      k7_tile_sort<<<grid, K7_THREADS, 0, s>>>(b);
-      II2_LAUNCHED();
-      for (uint64_t kk = 2ull * K7_TILE; (kk >> 1) < maxL; kk <<= 1) {
-        k7_stage<<<grid, 256, 0, s>>>(b, kk, 0);
-        II2_LAUNCHED();
-        for (uint64_t j = kk >> 2; j >= K7_TILE; j >>= 1) {
-          k7_stage<<<grid, 256, 0, s>>>(b, kk, j);
-          II2_LAUNCHED();
-        }
-        k7_tile_merge<<<grid, K7_THREADS, 0, s>>>(b, kk);
-        II2_LAUNCHED();
-      }
-    }
-  }
+  II2_TRY(k7_sort(a, maxL, s));
   ProfScope scope("k7_build", s);
   k7_mark<<<div_up(N + 1, 256), 256, 0, s>>>(a, keep.p, klen.p);
   II2_LAUNCHED();
@@ -316,6 +322,27 @@ int k7_ingest_sort(const uint8_t* d_tb, const uint32_t* d_toff, const uint64_t* 
   II2_CUDA_TRY(cudaStreamSynchronize(s));
   out.n_terms = h_tot[0];
   out.n_bytes = h_tot[1];
+  return II2_OK;
+}
+
+int k7_sort_distinct(const uint8_t* d_tb, const uint32_t* d_toff, const uint64_t* d_doff, int D,
+                     uint64_t N, uint64_t maxL, uint32_t* idx, uint64_t* keep, uint64_t* klen,
+                     cudaStream_t s) {
+  DevBuf<uint64_t> hi, lo;
+  II2_TRY(hi.alloc_scratch((size_t)N, s));
+  II2_TRY(lo.alloc_scratch((size_t)N, s));
+  K7Args a;
+  a.tb = d_tb;
+  a.toff = d_toff;
+  a.doff = d_doff;
+  a.hi = hi.p;
+  a.lo = lo.p;
+  a.idx = idx;
+  a.n = N;
+  a.d = D;
+  II2_TRY(k7_sort(a, maxL, s));
+  k7_mark<<<div_up(N + 1, 256), 256, 0, s>>>(a, keep, klen);
+  II2_LAUNCHED();
   return II2_OK;
 }
 

@@ -54,6 +54,24 @@ struct PatternDev {
 // from the calling thread's scratch arena.
 int k10_pattern_search(const PatternDev& d, PrefixOut& out, cudaStream_t s);
 
+// Device outputs of k10_pattern_terms: output pattern i's terms are [pattern_term_off[i],
+// pattern_term_off[i + 1]), ascending by bytes.Compare; term j = tb[toff[j] .. toff[j + 1]).
+struct TermsOut {
+  DevBuf<uint64_t> pattern_term_off;  // [npat + 1]
+  DevBuf<uint8_t> tb;
+  DevBuf<uint64_t> toff;              // [n_terms + 1]
+  DevBuf<uint32_t> segments;          // [n_terms] term instances over the call's segments
+  DevBuf<uint64_t> postings;          // [n_terms] sum of their stored list lengths
+  DevBuf<uint8_t> distance;           // [n_terms] FUZZY: edit distance, GLOB: 0
+  uint64_t n_terms = 0, n_bytes = 0;
+};
+
+// The distinct matching terms of every pattern over all segments, with their instance and
+// posting counts.  II2_ERR_UNSUPPORTED when the matched term instances or their bytes reach 2^32.
+// Synchronises the stream; every buffer (outputs too) comes from the calling thread's scratch
+// arena.
+int k10_pattern_terms(const PatternDev& d, TermsOut& out, cudaStream_t s);
+
 // One byte of a glob, and of a fuzzy pattern (hb = bit m - 1; global distance, Hyyrö: row 0
 // grows by one per byte, hence the 1 shifted into ph).  Host-callable so the compiler's tables
 // can be checked on the CPU.

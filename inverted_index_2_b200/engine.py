@@ -591,6 +591,45 @@ class Engine:
         matches."""
         return self._pattern_result(self.pattern_search_dev_out(segs, patterns))
 
+    def _terms_result(self, out: A.TermsOut) -> list[list[tuple[bytes, int, int, int]]]:
+        try:
+            n, nt = int(out.n_patterns), int(out.n_terms)
+            poff = A.from_ptr(out.pattern_term_off, n + 1, np.uint64)
+            toff = A.from_ptr(out.term_off, nt + 1, np.uint64)
+            tb = A.from_ptr(out.term_bytes, int(toff[-1]) if nt else 0, np.uint8).tobytes()
+            seg = A.from_ptr(out.segments, nt, np.uint32).tolist()
+            post = A.from_ptr(out.postings, nt, np.uint64).tolist()
+            dist = A.from_ptr(out.distance, nt, np.uint8).tolist()
+            toff = toff.tolist()
+            poff = poff.tolist()
+        finally:
+            self.lib.ii2_terms_out_free(C.byref(out))
+        terms = [(tb[toff[j]:toff[j + 1]], seg[j], post[j], dist[j]) for j in range(nt)]
+        return [terms[poff[i]:poff[i + 1]] for i in range(n)]
+
+    def pattern_terms(self, segs: list[FlatSegment], patterns: list
+                      ) -> list[list[tuple[bytes, int, int, int]]]:
+        """pattern_terms_dev over host views (uploaded for the call)."""
+        arr = views_array(segs)
+        batch, keep = self._pattern_args(patterns)
+        out = A.TermsOut()
+        self._check(self.lib.ii2_pattern_terms(arr, len(segs), C.byref(batch), C.byref(out)),
+                    "pattern_terms")
+        return self._terms_result(out)
+
+    def pattern_terms_dev(self, segs: list[DeviceSegment], patterns: list
+                          ) -> list[list[tuple[bytes, int, int, int]]]:
+        """The terms each pattern matches over resident segments, in one call on their device.
+        Patterns as in pattern_search_dev.  Aligned with `patterns`: the distinct matching terms
+        in bytes order, each as (term, segments, postings, distance): the term's instances over
+        `segs`, the sum of their stored list lengths, and for a fuzzy pattern its edit distance
+        (0 for a glob)."""
+        batch, keep = self._pattern_args(patterns)
+        out = A.TermsOut()
+        self._check(self.lib.ii2_pattern_terms_dev(self._handles(segs), len(segs), C.byref(batch),
+                                                   C.byref(out)), "pattern_terms_dev")
+        return self._terms_result(out)
+
     # ---- codec -----------------------------------------------------------------------
     def intcomp_encode_batch(self, post: np.ndarray, post_off: np.ndarray):
         post = np.ascontiguousarray(post, dtype=np.uint32)
